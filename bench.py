@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W [--config {1,2,3,4,5}]      (N>1: launched under torch.distributed.run)
   python bench.py --impl reference --gpus N --steps K --warmup W [--config ..]
+  python bench.py ... --dump-outputs DIR       (configs 1-4: also write what the last timed step computed as DIR/<name>.npy)
 
 A "step" is one generation of the rank's population shard: the fused evaluation (emulator + observation + both players'
 MLP + episode control for every game), the per-generation exchange (one record all-gather, issued asynchronously and
@@ -49,7 +50,14 @@ def parse():
     ap.add_argument("--cpu-seconds", type=float, default=12.0, help="budget of each cpu_baseline sample")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the saturated-GPU context run and the other configs' short runs")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the arrays the last timed generation returned (rank 0's shard) as "
+                    "DIR/<name>.npy, at most 64 MB in all, to compare two builds output for output")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and (args.impl == "reference" or args.config == 5):
+        ap.error("--dump-outputs needs the generation loop of configs 1-4 on the GPU")
+    return args
 
 
 def workload(config: int, world: int, population: int):
@@ -259,6 +267,7 @@ class Generation:
         nxt = eng.ga_step(g, fitness, seed=SEED_RUN, generation=gen)
         self.genomes = nxt["genomes"]
         self.fitness = fitness
+        self.last = (out, nxt)
         self.gen += 1
         return out["frames"]
 
@@ -296,6 +305,43 @@ def timed_generations(gen: Generation, steps: int, warmup: int, dist, sampler=No
     rollout_ms, _ = gen.eng.profile_read()                           # CUDA-event time of the dominant kernel inside the timed region
     gen.eng.profile_enable(False)
     return ms, frames, rollout_ms, launches
+
+
+DUMP_POPULATION_BYTES, DUMP_HOF_BYTES = 40 << 20, 16 << 20          # with the .npy headers well under 64 MB in all
+
+
+def _dump_rows(n: int, row_bytes: int, budget: int):
+    """All n rows, or a fixed seeded sample of them (ascending) when they do not fit in `budget` bytes."""
+    import numpy as np
+    k = min(n, max(1, budget // row_bytes))
+    return np.arange(n) if k == n else np.sort(np.random.RandomState(0).choice(n, k, replace=False))
+
+
+def dump_outputs(gen: Generation, directory: str):
+    """What the last generation handed back -- evaluate (fitness, per-game rewards and frame counts), the GA step (next
+    genomes, parents, invalid flags, fitness statistics) and the hall of fame it updated -- as DIR/<name>.npy: genomes in
+    float32, everything else in float64 (integers exactly).  Per-genome arrays keep the rows in population_rows.npy (all of
+    them unless a wide net's genomes would pass the size budget), hall-of-fame arrays those in hof_rows.npy."""
+    import numpy as np
+    torch = gen.torch
+    out, nxt = gen.last
+    groups = [("population", DUMP_POPULATION_BYTES, {"fitness": out["fitness"], "rewards": out["rewards"], "frames": out["frames"],
+                                                     "genomes": nxt["genomes"], "parent_idx": nxt["parent_idx"], "invalid": nxt["invalid"]})]
+    hg, hf = gen.hof.tensors()
+    if hf is not None:
+        groups.append(("hof", DUMP_HOF_BYTES, {"hof_fitness": hf, "hof_genomes": hg}))
+    arrays = {"ga_stats": nxt["stats"]}
+    for name, budget, group in groups:
+        n = next(iter(group.values())).shape[0]
+        row_bytes = 8 + sum((4 if t.dtype == torch.float32 else 8) * (t.numel() // n) for t in group.values())
+        rows = _dump_rows(n, row_bytes, budget)
+        idx = torch.from_numpy(rows).to(gen.eng.device)
+        arrays[name + "_rows"] = rows
+        arrays.update({k: t.index_select(0, idx) for k, t in group.items()})
+    os.makedirs(directory, exist_ok=True)
+    for k, a in arrays.items():
+        a = a.cpu().numpy() if isinstance(a, torch.Tensor) else a
+        np.save(os.path.join(directory, k + ".npy"), a.astype(np.float32 if a.dtype == np.float32 else np.float64))
 
 
 def e2e_generations(gen: Generation, steps: int, warmup: int, dist):
@@ -347,7 +393,7 @@ def reduce_ranks(torch, dist, world, maxed, summed):
 # ---------------------------------------------------------------------------------------------------
 # config 5: NN forward + GA only
 # ---------------------------------------------------------------------------------------------------
-def config5_sweep(ngp, local, world, dist, sizes=None, envs=6, reps=5):
+def config5_sweep(ngp, local, world, dist, sizes=None, envs=6, reps=5, warmup=2):
     """Policy forward on synthetic obs.npy-shaped inputs (6 observation values per environment, `envs` environments per
     genome) + one GA step (fitness statistics, tournament selection, blend crossover, Gaussian mutation), per population
     size; the population is sharded over the ranks like every other config.  Device-timed (CUDA events), max over ranks."""
@@ -363,14 +409,14 @@ def config5_sweep(ngp, local, world, dist, sizes=None, envs=6, reps=5):
         fitness = torch.rand(n, dtype=torch.float64, device=eng.device)
         ev = [torch.cuda.Event(enable_timing=True) for _ in range(3)]
         t_f = t_g = 0.0
-        for r in range(reps + 2):
+        for r in range(reps + warmup):
             ev[0].record()
             eng.mlp_forward(genomes, x, want_out=False)
             ev[1].record()
             nxt = eng.ga_step(genomes, fitness, seed=7, generation=r)
             ev[2].record()
             torch.cuda.synchronize()
-            if r >= 2:
+            if r >= warmup:
                 t_f += ev[0].elapsed_time(ev[1]); t_g += ev[1].elapsed_time(ev[2])
             genomes = nxt["genomes"]
         (mf, mg), _ = reduce_ranks(torch, dist, world, [t_f / reps, t_g / reps], [0.0])
@@ -409,11 +455,11 @@ def main():
         pass
 
     if args.config == 5:
-        rows = config5_sweep(ngp, local, world, D)
+        rows = config5_sweep(ngp, local, world, D, reps=args.steps, warmup=args.warmup)
         if rank == 0:
             top = rows[-1]
             print(json.dumps({"metric": "policy_forwards_per_sec_plus_ga", "value": top["policy_forwards_per_s"], "unit": "forwards/s", "n_gpus": world,
-                              "steps": 5, "warmup": 2, "ms_per_step": top["forward_ms"] + top["ga_step_ms"], "higher_is_better": True, "scaling": "strong",
+                              "steps": args.steps, "warmup": args.warmup, "ms_per_step": top["forward_ms"] + top["ga_step_ms"], "higher_is_better": True, "scaling": "strong",
                               "vs_baseline": None, "dtype": "f32 (hidden layers) + f64 (action layer)", "data": "synthetic",
                               "config": {"workload": "config 5: NN forward + GA only on synthetic obs.npy-shaped inputs, population sweep"}, "sweep": rows}), flush=True)
         if world > 1:
@@ -426,6 +472,8 @@ def main():
     sampler = ClockSampler(local) if rank == 0 else None
     ms, frames, rollout_ms, launches = timed_generations(gen, args.steps, args.warmup, D, sampler)
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(gen, args.dump_outputs)
     (ms, rollout_ms), (frames,) = reduce_ranks(torch, dist, world, [ms, rollout_ms], [float(frames)])
     e2e_s, e2e_frames, h2d, d2h = e2e_generations(gen, args.steps, args.warmup, D)
     (e2e_s,), (e2e_frames,) = reduce_ranks(torch, dist, world, [e2e_s], [float(e2e_frames)])
