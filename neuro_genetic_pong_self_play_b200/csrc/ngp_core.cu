@@ -11,6 +11,7 @@
 #include <string.h>
 
 #include <map>
+#include <memory>
 #include <mutex>
 #include <vector>
 
@@ -282,8 +283,7 @@ extern "C" int ngp_create(const ngp_config *cfg, const uint8_t *rom, int32_t dev
     NGP_CUDA(cudaGetDeviceCount(&count));
     NGP_REQUIRE(device >= 0 && device < count, "ngp_create: no such CUDA device");
     NGP_CUDA(cudaSetDevice(device));
-    ngp_handle *h = new ngp_handle();
-    memset(h, 0, sizeof(*h));
+    auto h = std::make_unique<ngp_handle>();     // freed with everything it holds on an early return
     h->cfg = *cfg;
     h->device = device;
     h->gene_size = gene_size_of(*cfg);
@@ -297,16 +297,16 @@ extern "C" int ngp_create(const ngp_config *cfg, const uint8_t *rom, int32_t dev
     ngp_host::build_tables(tables, rom, cfg->ball_colour, cfg->left_colour, cfg->right_colour, ngp_ntsc_palette);
     std::vector<uint32_t> needed(a26::TRIGMAX + 1);
     ngp_host::build_paddle_table(needed.data());
-    NGP_CUDA(cudaMalloc(&h->d_tables, sizeof(Tables)));
-    NGP_CUDA(cudaMemcpy(h->d_tables, &tables, sizeof(Tables), cudaMemcpyHostToDevice));
-    NGP_CUDA(cudaMalloc(&h->d_needed, needed.size() * 4));
-    NGP_CUDA(cudaMemcpy(h->d_needed, needed.data(), needed.size() * 4, cudaMemcpyHostToDevice));
-    NGP_CUDA(cudaMalloc(&h->d_palette, sizeof(ngp_ntsc_palette)));
-    NGP_CUDA(cudaMemcpy(h->d_palette, ngp_ntsc_palette, sizeof(ngp_ntsc_palette), cudaMemcpyHostToDevice));
-    NGP_CUDA(cudaMalloc(&h->d_start, 2 * sizeof(Snapshot)));
-    NGP_CUDA(cudaMalloc(&h->d_counters, 8 * sizeof(unsigned long long)));
-    NGP_CUDA(cudaMemset(h->d_counters, 0, 8 * sizeof(unsigned long long)));
-    NGP_CUDA(cudaMallocHost(&h->h_counters, 8 * sizeof(unsigned long long)));
+    NGP_CUDA(h->d_tables.ensure(1));
+    NGP_CUDA(cudaMemcpy(h->d_tables.p, &tables, sizeof(Tables), cudaMemcpyHostToDevice));
+    NGP_CUDA(h->d_needed.ensure(needed.size()));
+    NGP_CUDA(cudaMemcpy(h->d_needed.p, needed.data(), needed.size() * 4, cudaMemcpyHostToDevice));
+    NGP_CUDA(h->d_palette.ensure(128));
+    NGP_CUDA(cudaMemcpy(h->d_palette.p, ngp_ntsc_palette, sizeof(ngp_ntsc_palette), cudaMemcpyHostToDevice));
+    NGP_CUDA(h->d_start.ensure(2));
+    NGP_CUDA(h->d_counters.ensure(8));
+    NGP_CUDA(cudaMemset(h->d_counters.p, 0, 8 * sizeof(unsigned long long)));
+    NGP_CUDA(h->h_counters.ensure(8));
     // The two start snapshots depend on the cartridge image only: built once per process by the CUDA core (a single warp,
     // tens of milliseconds) and kept as an immutable host copy for later handles.
     {
@@ -314,18 +314,18 @@ extern "C" int ngp_create(const ngp_config *cfg, const uint8_t *rom, int32_t dev
         const uint64_t key = fnv1a64(rom, 2048);
         auto it = g_start_cache.find(key);
         if (it == g_start_cache.end()) {
-            build_start_states_kernel<<<2, 32>>>(h->d_tables, h->d_needed, h->d_start);
+            build_start_states_kernel<<<2, 32>>>(h->d_tables.p, h->d_needed.p, h->d_start.p);
             h->launches++;
             NGP_CUDA(cudaGetLastError());
             std::vector<Snapshot> snap(2);
-            NGP_CUDA(cudaMemcpy(snap.data(), h->d_start, 2 * sizeof(Snapshot), cudaMemcpyDeviceToHost));
+            NGP_CUDA(cudaMemcpy(snap.data(), h->d_start.p, 2 * sizeof(Snapshot), cudaMemcpyDeviceToHost));
             g_start_cache.emplace(key, std::move(snap));
         } else {
-            NGP_CUDA(cudaMemcpy(h->d_start, it->second.data(), 2 * sizeof(Snapshot), cudaMemcpyHostToDevice));
+            NGP_CUDA(cudaMemcpy(h->d_start.p, it->second.data(), 2 * sizeof(Snapshot), cudaMemcpyHostToDevice));
         }
     }
     NGP_CUDA(cudaDeviceSynchronize());
-    *out = h;
+    *out = h.release();
     return NGP_OK;
 }
 
@@ -333,15 +333,6 @@ extern "C" int ngp_destroy(ngp_handle *h)
 {
     if (!h) return NGP_OK;
     cudaSetDevice(h->device);
-    cudaFree(h->d_tables); cudaFree(h->d_needed); cudaFree(h->d_palette); cudaFree(h->d_start);
-    cudaFree(h->d_envs); cudaFree(h->d_fb); cudaFree(h->d_rewards); cudaFree(h->d_frames); cudaFree(h->d_counters);
-    cudaFree(h->d_genomes_stage); cudaFree(h->d_fitness_stage); cudaFree(h->d_hof_stage); cudaFree(h->d_hof_fit_stage);
-    cudaFree(h->mlp_a); cudaFree(h->mlp_b); cudaFree(h->mlp_z); cudaFree(h->d_parent);
-    cudaFree(h->rank_keys); cudaFree(h->rank_idx); cudaFree(h->prep_packed);
-    cudaFree(h->step_envs); cudaFree(h->step_x); cudaFree(h->step_act); cudaFree(h->step_opp);
-    cudaFree(h->hof_hash_old); cudaFree(h->hof_hash_new); cudaFree(h->hof_order); cudaFree(h->hof_tmp_genomes); cudaFree(h->hof_tmp_fitness);
-    cudaFreeHost(h->h_genomes); cudaFreeHost(h->h_fitness); cudaFreeHost(h->h_counters);
-    if (h->prof_events) { for (auto &e : *h->prof_events) { cudaEventDestroy(e.first); cudaEventDestroy(e.second); } delete h->prof_events; }
     delete h;
     return NGP_OK;
 }
@@ -352,16 +343,11 @@ extern "C" int ngp_env_reset(ngp_handle *h, int32_t n_envs, int32_t state_id, vo
     NGP_REQUIRE(state_id == NGP_STATE_START_1P || state_id == NGP_STATE_START_2P, "ngp_env_reset: unknown state");
     NGP_CUDA(cudaSetDevice(h->device));
     cudaStream_t st = (cudaStream_t)stream;
-    if (n_envs > h->cap_envs) {
-        cudaFree(h->d_envs); cudaFree(h->d_fb);
-        h->d_envs = nullptr; h->d_fb = nullptr; h->cap_envs = 0;
-        NGP_CUDA(cudaMalloc(&h->d_envs, (size_t)n_envs * sizeof(Snapshot)));
-        NGP_CUDA(cudaMalloc(&h->d_fb, (size_t)n_envs * a26::FB_ROWS * a26::FB_COLS));
-        h->cap_envs = n_envs;
-    }
+    NGP_CUDA(h->d_envs.ensure(n_envs));
+    NGP_CUDA(h->d_fb.ensure((size_t)n_envs * a26::FB_ROWS * a26::FB_COLS));
     h->n_envs = n_envs;
     h->env_players = state_id == NGP_STATE_START_1P ? 1 : 2;     // main.py:40 makes the robot game with players=1
-    env_reset_kernel<<<(n_envs + 127) / 128, 128, 0, st>>>(h->d_start + state_id, h->d_envs, n_envs);
+    env_reset_kernel<<<(n_envs + 127) / 128, 128, 0, st>>>(h->d_start.p + state_id, h->d_envs.p, n_envs);
     h->launches++;
     NGP_CUDA(cudaGetLastError());
     return NGP_OK;
@@ -389,21 +375,21 @@ extern "C" int ngp_env_step_core(ngp_handle *h, int32_t core, const uint8_t *act
     const size_t px = (size_t)n * a26::FB_ROWS * a26::FB_COLS;
     ButtonMap bmap;
     memcpy(bmap.m, h->cfg.button_map, 16);
-    if (frames) NGP_CUDA(cudaMemsetAsync(h->d_fb, 0, px, st));
+    if (frames) NGP_CUDA(cudaMemsetAsync(h->d_fb.p, 0, px, st));
     // with a frame requested every pixel is rendered (verify mode); without, the fused no-framebuffer flavour runs
     int lanes = (n + 4 * h->sm_count - 1) / (4 * h->sm_count);           // one warp per scheduler before the warps are filled
     lanes = lanes < 1 ? 1 : (lanes > 32 ? 32 : lanes);
     const unsigned grid = (unsigned)((n + lanes - 1) / lanes);
     if (frames)
-        env_step_kernel<true><<<grid, 32, 0, st>>>(h->d_tables, h->d_needed, h->d_envs, n, lanes, core ? 1 : 0, h->env_players, bmap, actions, h->d_fb, ram,
-                                                   loc, valid, regs, h->d_counters);
+        env_step_kernel<true><<<grid, 32, 0, st>>>(h->d_tables.p, h->d_needed.p, h->d_envs.p, n, lanes, core ? 1 : 0, h->env_players, bmap, actions, h->d_fb.p,
+                                                   ram, loc, valid, regs, h->d_counters.p);
     else
-        env_step_kernel<false><<<grid, 32, 0, st>>>(h->d_tables, h->d_needed, h->d_envs, n, lanes, core ? 1 : 0, h->env_players, bmap, actions, nullptr, ram,
-                                                    loc, valid, regs, h->d_counters);
+        env_step_kernel<false><<<grid, 32, 0, st>>>(h->d_tables.p, h->d_needed.p, h->d_envs.p, n, lanes, core ? 1 : 0, h->env_players, bmap, actions, nullptr,
+                                                    ram, loc, valid, regs, h->d_counters.p);
     h->launches++;
     NGP_CUDA(cudaGetLastError());
     if (frames) {
-        palette_to_rgb_kernel<<<(unsigned)((px + 255) / 256), 256, 0, st>>>(h->d_fb, h->d_palette, frames, px);
+        palette_to_rgb_kernel<<<(unsigned)((px + 255) / 256), 256, 0, st>>>(h->d_fb.p, h->d_palette.p, frames, px);
         h->launches++;
         NGP_CUDA(cudaGetLastError());
     }
@@ -414,7 +400,7 @@ extern "C" int ngp_env_digest(ngp_handle *h, uint32_t *digest, void *stream)
 {
     NGP_REQUIRE(h && digest && h->n_envs > 0, "ngp_env_digest: bad arguments");
     NGP_CUDA(cudaSetDevice(h->device));
-    env_digest_kernel<<<(h->n_envs + 127) / 128, 128, 0, (cudaStream_t)stream>>>(h->d_envs, h->n_envs, digest);
+    env_digest_kernel<<<(h->n_envs + 127) / 128, 128, 0, (cudaStream_t)stream>>>(h->d_envs.p, h->n_envs, digest);
     h->launches++;
     NGP_CUDA(cudaGetLastError());
     return NGP_OK;
@@ -437,16 +423,11 @@ extern "C" int ngp_evaluate(ngp_handle *h, const float *genomes, int32_t n, cons
     const int games = h->cfg.games_to_play;
     const long long total = (long long)n * games;
     NGP_REQUIRE(total < (1ll << 31), "ngp_evaluate: too many environments");
-    if (total > h->cap_eval) {
-        cudaFree(h->d_rewards); cudaFree(h->d_frames);
-        h->d_rewards = nullptr; h->d_frames = nullptr; h->cap_eval = 0;
-        NGP_CUDA(cudaMalloc(&h->d_rewards, (size_t)total * sizeof(double)));
-        NGP_CUDA(cudaMalloc(&h->d_frames, (size_t)total * sizeof(int32_t)));
-        h->cap_eval = (int)total;
-    }
-    NGP_CUDA(cudaMemsetAsync(h->d_counters, 0, 8 * sizeof(unsigned long long), st));
+    NGP_CUDA(h->d_rewards.ensure(total));
+    NGP_CUDA(h->d_frames.ensure(total));
+    NGP_CUDA(cudaMemsetAsync(h->d_counters.p, 0, 8 * sizeof(unsigned long long), st));
     RolloutParams p;
-    p.tables = h->d_tables; p.needed = h->d_needed; p.start = h->d_start;
+    p.tables = h->d_tables.p; p.needed = h->d_needed.p; p.start = h->d_start.p;
     p.genomes = genomes; p.hof_genomes = hof_genomes; p.hof_fitness = hof_fitness; p.hof_pick = hof_pick;
     p.n = n; p.n_hof = n_hof; p.G = h->gene_size; p.games = games; p.schedule = h->cfg.schedule;
     p.core = h->cfg.core ? 1 : 0;
@@ -466,16 +447,16 @@ extern "C" int ngp_evaluate(ngp_handle *h, const float *genomes, int32_t n, cons
                 a[6] = la == pol::ACT_UP; a[7] = la == pol::ACT_DOWN;         // action[6:8] = left (main.py:92)
                 p.input_table[players - 1][la * 3 + ra] = roll::action_to_input(a, players, h->cfg.button_map);
             }
-    p.rewards = rewards ? rewards : h->d_rewards; p.frames = frames ? frames : h->d_frames; p.counters = h->d_counters;
+    p.rewards = rewards ? rewards : h->d_rewards.p; p.frames = frames ? frames : h->d_frames.p; p.counters = h->d_counters.p;
     if (wide) {
         const int rc = ngp_evaluate_stepwise(h, p, st);
         if (rc != NGP_OK) return rc;
         fitness_reduce_kernel<<<(n + 127) / 128, 128, 0, st>>>(p.rewards, n, games, fitness);
         h->launches++;
         NGP_CUDA(cudaGetLastError());
-        if (frames_total) *frames_total = h->h_counters[1];
-        if (h->h_counters[2]) {
-            ngp_set_error("ngp_evaluate: %llu environments stopped on an emulator error", h->h_counters[2]);
+        if (frames_total) *frames_total = h->h_counters.p[1];
+        if (h->h_counters.p[2]) {
+            ngp_set_error("ngp_evaluate: %llu environments stopped on an emulator error", h->h_counters.p[2]);
             return NGP_ERR_EMULATOR;
         }
         return NGP_OK;
@@ -520,13 +501,12 @@ extern "C" int ngp_evaluate(ngp_handle *h, const float *genomes, int32_t n, cons
     if (blocks > resident) blocks = resident;            // persistent lanes pull the rest from the queue
     cudaEvent_t ev0 = nullptr, ev1 = nullptr;
     if (h->profile_on) {
-        if (!h->prof_events) h->prof_events = new std::vector<std::pair<cudaEvent_t, cudaEvent_t>>();
-        if (h->prof_used == (int)h->prof_events->size()) {
+        if (h->prof_used == (int)h->prof_events.size()) {
             cudaEvent_t a, b;
             NGP_CUDA(cudaEventCreate(&a)); NGP_CUDA(cudaEventCreate(&b));
-            h->prof_events->push_back({a, b});
+            h->prof_events.push_back({a, b});
         }
-        ev0 = (*h->prof_events)[h->prof_used].first; ev1 = (*h->prof_events)[h->prof_used].second;
+        ev0 = h->prof_events[h->prof_used].first; ev1 = h->prof_events[h->prof_used].second;
         h->prof_used++;
         NGP_CUDA(cudaEventRecord(ev0, st));
     }
@@ -538,11 +518,11 @@ extern "C" int ngp_evaluate(ngp_handle *h, const float *genomes, int32_t n, cons
     h->launches++;
     NGP_CUDA(cudaGetLastError());
     if (frames_total) {
-        NGP_CUDA(cudaMemcpyAsync(h->h_counters, h->d_counters, 4 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+        NGP_CUDA(cudaMemcpyAsync(h->h_counters.p, h->d_counters.p, 4 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
         NGP_CUDA(cudaStreamSynchronize(st));
-        *frames_total = h->h_counters[1];
-        if (h->h_counters[2]) {
-            ngp_set_error("ngp_evaluate: %llu environments stopped on an emulator error", h->h_counters[2]);
+        *frames_total = h->h_counters.p[1];
+        if (h->h_counters.p[2]) {
+            ngp_set_error("ngp_evaluate: %llu environments stopped on an emulator error", h->h_counters.p[2]);
             return NGP_ERR_EMULATOR;
         }
     }
@@ -563,8 +543,8 @@ extern "C" int ngp_profile_read(ngp_handle *h, double *rollout_ms, int32_t *roll
     double total = 0.0;
     for (int i = 0; i < h->prof_used; ++i) {
         float ms = 0.f;
-        NGP_CUDA(cudaEventSynchronize((*h->prof_events)[i].second));
-        NGP_CUDA(cudaEventElapsedTime(&ms, (*h->prof_events)[i].first, (*h->prof_events)[i].second));
+        NGP_CUDA(cudaEventSynchronize(h->prof_events[i].second));
+        NGP_CUDA(cudaEventElapsedTime(&ms, h->prof_events[i].first, h->prof_events[i].second));
         total += ms;
     }
     *rollout_ms = total;
@@ -578,39 +558,27 @@ extern "C" int ngp_evaluate_host(ngp_handle *h, const float *genomes, int32_t n,
 {
     NGP_REQUIRE(h && genomes && fitness && n > 0, "ngp_evaluate_host: bad arguments");
     NGP_CUDA(cudaSetDevice(h->device));
-    const size_t gbytes = (size_t)n * h->gene_size * sizeof(float), fbytes = (size_t)n * sizeof(double);
-    if (gbytes > h->stage_genomes) {
-        cudaFreeHost(h->h_genomes); cudaFree(h->d_genomes_stage); h->stage_genomes = 0;
-        NGP_CUDA(cudaMallocHost(&h->h_genomes, gbytes));
-        NGP_CUDA(cudaMalloc(&h->d_genomes_stage, gbytes));
-        h->stage_genomes = gbytes;
-    }
-    if (fbytes > h->stage_fitness) {
-        cudaFreeHost(h->h_fitness); cudaFree(h->d_fitness_stage); h->stage_fitness = 0;
-        NGP_CUDA(cudaMallocHost(&h->h_fitness, fbytes));
-        NGP_CUDA(cudaMalloc(&h->d_fitness_stage, fbytes));
-        h->stage_fitness = fbytes;
-    }
-    const size_t hbytes = (size_t)n_hof * h->gene_size * sizeof(float);
-    if (n_hof > 0 && hbytes > h->stage_hof) {
-        cudaFree(h->d_hof_stage); cudaFree(h->d_hof_fit_stage); h->stage_hof = 0;
-        NGP_CUDA(cudaMalloc(&h->d_hof_stage, hbytes));
-        NGP_CUDA(cudaMalloc(&h->d_hof_fit_stage, (size_t)n_hof * sizeof(double)));
-        h->stage_hof = hbytes;
-    }
-    memcpy(h->h_genomes, genomes, gbytes);
-    NGP_CUDA(cudaMemcpyAsync(h->d_genomes_stage, h->h_genomes, gbytes, cudaMemcpyHostToDevice, 0));
+    const size_t genes = (size_t)n * h->gene_size, gbytes = genes * sizeof(float), fbytes = (size_t)n * sizeof(double);
+    NGP_CUDA(h->h_genomes.ensure(genes));
+    NGP_CUDA(h->d_genomes_stage.ensure(genes));
+    NGP_CUDA(h->h_fitness.ensure(n));
+    NGP_CUDA(h->d_fitness_stage.ensure(n));
+    memcpy(h->h_genomes.p, genomes, gbytes);
+    NGP_CUDA(cudaMemcpyAsync(h->d_genomes_stage.p, h->h_genomes.p, gbytes, cudaMemcpyHostToDevice, 0));
     if (n_hof > 0) {
-        NGP_CUDA(cudaMemcpyAsync(h->d_hof_stage, hof_genomes, hbytes, cudaMemcpyHostToDevice, 0));
-        NGP_CUDA(cudaMemcpyAsync(h->d_hof_fit_stage, hof_fitness, (size_t)n_hof * sizeof(double), cudaMemcpyHostToDevice, 0));
+        const size_t hof_genes = (size_t)n_hof * h->gene_size;
+        NGP_CUDA(h->d_hof_stage.ensure(hof_genes));
+        NGP_CUDA(h->d_hof_fit_stage.ensure(n_hof));
+        NGP_CUDA(cudaMemcpyAsync(h->d_hof_stage.p, hof_genomes, hof_genes * sizeof(float), cudaMemcpyHostToDevice, 0));
+        NGP_CUDA(cudaMemcpyAsync(h->d_hof_fit_stage.p, hof_fitness, (size_t)n_hof * sizeof(double), cudaMemcpyHostToDevice, 0));
     }
     uint64_t ft = 0;
-    int rc = ngp_evaluate(h, h->d_genomes_stage, n, n_hof ? h->d_hof_stage : nullptr, n_hof ? h->d_hof_fit_stage : nullptr, n_hof,
-                          nullptr, seed, generation, h->d_fitness_stage, nullptr, nullptr, &ft, 0);
+    int rc = ngp_evaluate(h, h->d_genomes_stage.p, n, n_hof ? h->d_hof_stage.p : nullptr, n_hof ? h->d_hof_fit_stage.p : nullptr, n_hof,
+                          nullptr, seed, generation, h->d_fitness_stage.p, nullptr, nullptr, &ft, 0);
     if (rc != NGP_OK) return rc;
-    NGP_CUDA(cudaMemcpyAsync(h->h_fitness, h->d_fitness_stage, fbytes, cudaMemcpyDeviceToHost, 0));
+    NGP_CUDA(cudaMemcpyAsync(h->h_fitness.p, h->d_fitness_stage.p, fbytes, cudaMemcpyDeviceToHost, 0));
     NGP_CUDA(cudaStreamSynchronize(0));
-    memcpy(fitness, h->h_fitness, fbytes);
+    memcpy(fitness, h->h_fitness.p, fbytes);
     if (frames_total) *frames_total = ft;
     return NGP_OK;
 }

@@ -398,18 +398,13 @@ extern "C" int ngp_mlp_prepare(ngp_handle *h, const float *genomes, int32_t n_ge
         if (layer_is_packed(sh, l)) per_genome += tmm::packed_floats(sh.nodes[l], sh.nodes[l + 1]);
     h->prep_n = 0; h->prep_src = nullptr; h->prep_per_genome = per_genome;
     if (per_genome == 0) { h->prep_n = n_genomes; h->prep_src = genomes; return NGP_OK; }      // nothing to pack for this network
-    const size_t need = per_genome * (size_t)n_genomes * sizeof(float);
-    if (need > h->prep_cap) {
-        cudaFree(h->prep_packed); h->prep_packed = nullptr; h->prep_cap = 0;
-        NGP_CUDA(cudaMalloc(&h->prep_packed, need));
-        h->prep_cap = need;
-    }
+    NGP_CUDA(h->prep_packed.ensure(per_genome * (size_t)n_genomes));
     size_t w_off = 0, layer_off = 0;
     for (int l = 0; l < L; ++l) {
         const int ni = sh.nodes[l], no = sh.nodes[l + 1];
         if (layer_is_packed(sh, l)) {
             dim3 grid(128, n_genomes);
-            tmm::mlp_pack_layer_kernel<<<grid, 256, 0, st>>>(genomes, w_off, h->gene_size, ni, no, bias, h->prep_packed, per_genome, layer_off);
+            tmm::mlp_pack_layer_kernel<<<grid, 256, 0, st>>>(genomes, w_off, h->gene_size, ni, no, bias, h->prep_packed.p, per_genome, layer_off);
             h->launches++;
             NGP_CUDA(cudaGetLastError());
             layer_off += tmm::packed_floats(ni, no);
@@ -424,7 +419,7 @@ extern "C" int ngp_mlp_prepare(ngp_handle *h, const float *genomes, int32_t n_ge
 int ngp_mlp_layer_tmem(ngp_handle *h, int l, const float *in, int n_genomes, int envs, float *out, cudaStream_t st)
 {
     const pol::Shape &sh = h->shape;
-    if (!layer_is_packed(sh, l) || envs < 16 || !h->prep_packed) return NGP_ERR_UNSUPPORTED;
+    if (!layer_is_packed(sh, l) || envs < 16 || !h->prep_packed.p) return NGP_ERR_UNSUPPORTED;
     size_t layer_off = 0;
     for (int i = 0; i < l; ++i)
         if (layer_is_packed(sh, i)) layer_off += tmm::packed_floats(sh.nodes[i], sh.nodes[i + 1]);
@@ -436,10 +431,10 @@ int ngp_mlp_layer_tmem(ngp_handle *h, int l, const float *in, int n_genomes, int
     }
     if (envs > 64) {
         dim3 grid((no + tmm::TM - 1) / tmm::TM, (envs + 127) / 128, n_genomes);
-        tmm::mlp_layer_tmem_kernel<128><<<grid, tmm::threads(128), tmm::smem_bytes(128), st>>>(h->prep_packed, h->prep_per_genome, layer_off, in, envs, ni, no, out);
+        tmm::mlp_layer_tmem_kernel<128><<<grid, tmm::threads(128), tmm::smem_bytes(128), st>>>(h->prep_packed.p, h->prep_per_genome, layer_off, in, envs, ni, no, out);
     } else {
         dim3 grid((no + tmm::TM - 1) / tmm::TM, 1, n_genomes);
-        tmm::mlp_layer_tmem_kernel<64><<<grid, tmm::threads(64), tmm::smem_bytes(64), st>>>(h->prep_packed, h->prep_per_genome, layer_off, in, envs, ni, no, out);
+        tmm::mlp_layer_tmem_kernel<64><<<grid, tmm::threads(64), tmm::smem_bytes(64), st>>>(h->prep_packed.p, h->prep_per_genome, layer_off, in, envs, ni, no, out);
     }
     h->launches++;
     NGP_CUDA(cudaGetLastError());

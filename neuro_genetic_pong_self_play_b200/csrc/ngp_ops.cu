@@ -465,8 +465,6 @@ __global__ void mlp_decide_kernel(const double *__restrict__ z, long long rows, 
 int ngp_mlp_layer_tf32(ngp_handle *h, const float *genomes, size_t w_off, const float *in, int n_genomes, int envs, int ni, int no, int bias,
                        float *out, cudaStream_t st);   // ngp_mlp_tf32.cu
 
-struct MlpScratch { float *&a, *&b; double *&z; size_t &cap_ab, &cap_z; };     // view of the handle's scratch
-
 int ngp_mlp_layer_tmem(ngp_handle *h, int l, const float *in, int n_genomes, int envs, float *out, cudaStream_t st);    // ngp_mlp_tmem.cu
 
 static int mlp_forward_impl(ngp_handle *h, const float *genomes, const float *x, int32_t n_genomes, int32_t envs, uint8_t *act, float *out,
@@ -502,21 +500,11 @@ static int mlp_forward_impl(ngp_handle *h, const float *genomes, const float *x,
         NGP_CUDA(cudaGetLastError());
         return NGP_OK;
     }
-    MlpScratch sc{h->mlp_a, h->mlp_b, h->mlp_z, h->mlp_cap_ab, h->mlp_cap_z};
-    const size_t need_ab = (size_t)rows * widest, need_z = (size_t)rows * sh.nodes[sh.n_layers - 1];
-    if (need_ab > sc.cap_ab) {
-        cudaFree(sc.a); cudaFree(sc.b); sc.cap_ab = 0;
-        NGP_CUDA(cudaMalloc(&sc.a, need_ab * sizeof(float)));
-        NGP_CUDA(cudaMalloc(&sc.b, need_ab * sizeof(float)));
-        sc.cap_ab = need_ab;
-    }
-    if (need_z > sc.cap_z) {
-        cudaFree(sc.z); sc.cap_z = 0;
-        NGP_CUDA(cudaMalloc(&sc.z, need_z * sizeof(double)));
-        sc.cap_z = need_z;
-    }
+    NGP_CUDA(h->mlp_a.ensure((size_t)rows * widest));
+    NGP_CUDA(h->mlp_b.ensure((size_t)rows * widest));
+    NGP_CUDA(h->mlp_z.ensure((size_t)rows * sh.nodes[sh.n_layers - 1]));
     const float *in = x;
-    float *bufs[2] = {sc.a, sc.b};
+    float *bufs[2] = {h->mlp_a.p, h->mlp_b.p};
     size_t w_off = 0;
     const int bias = sh.bias ? 1 : 0, L = sh.n_layers - 1;
     for (int l = 0; l < L; ++l) {
@@ -559,7 +547,7 @@ static int mlp_forward_impl(ngp_handle *h, const float *genomes, const float *x,
             else if (rc != NGP_ERR_UNSUPPORTED) return rc;
         }
         if (!launched) {
-            if (l == L - 1) mlp_layer_kernel<true><<<grid, 256, 0, st>>>(genomes, w_off, h->gene_size, in, envs, ni, no, bias, nullptr, sc.z);
+            if (l == L - 1) mlp_layer_kernel<true><<<grid, 256, 0, st>>>(genomes, w_off, h->gene_size, in, envs, ni, no, bias, nullptr, h->mlp_z.p);
             else mlp_layer_kernel<false><<<grid, 256, 0, st>>>(genomes, w_off, h->gene_size, in, envs, ni, no, bias, bufs[l & 1], nullptr);
             h->launches++;
             NGP_CUDA(cudaGetLastError());
@@ -567,7 +555,7 @@ static int mlp_forward_impl(ngp_handle *h, const float *genomes, const float *x,
         in = bufs[l & 1];
         w_off += (size_t)(ni + bias) * no;
     }
-    mlp_decide_kernel<<<(unsigned)((rows + 255) / 256), 256, 0, st>>>(sc.z, rows, sh.nodes[L], act, out);
+    mlp_decide_kernel<<<(unsigned)((rows + 255) / 256), 256, 0, st>>>(h->mlp_z.p, rows, sh.nodes[L], act, out);
     h->launches++;
     NGP_CUDA(cudaGetLastError());
     return NGP_OK;
@@ -763,25 +751,22 @@ static int select_dispatch(ngp_handle *h, const double *fitness, int n, int k, i
     }
     int n_pow2 = RANK_TILE;
     while (n_pow2 < n) n_pow2 <<= 1;
-    if ((size_t)n_pow2 > h->cap_rank) {
-        cudaFree(h->rank_keys); cudaFree(h->rank_idx); h->rank_keys = nullptr; h->rank_idx = nullptr; h->cap_rank = 0;
-        NGP_CUDA(cudaMalloc(&h->rank_keys, (size_t)n_pow2 * sizeof(unsigned long long)));
-        NGP_CUDA(cudaMalloc(&h->rank_idx, (size_t)n_pow2 * sizeof(int32_t)));
-        h->cap_rank = n_pow2;
-    }
-    unsigned long long *keys = (unsigned long long *)h->rank_keys;
-    rank_init_kernel<<<(n_pow2 + 255) / 256, 256, 0, st>>>(fitness, n, n_pow2, keys, h->rank_idx);
-    rank_sort_tile_kernel<<<n_pow2 / RANK_TILE, RANK_TILE / 2, 0, st>>>(keys, h->rank_idx, 2, RANK_TILE);     // sorted tiles, alternating direction
+    NGP_CUDA(h->rank_keys.ensure(n_pow2));
+    NGP_CUDA(h->rank_idx.ensure(n_pow2));
+    unsigned long long *keys = h->rank_keys.p;
+    int32_t *idx = h->rank_idx.p;
+    rank_init_kernel<<<(n_pow2 + 255) / 256, 256, 0, st>>>(fitness, n, n_pow2, keys, idx);
+    rank_sort_tile_kernel<<<n_pow2 / RANK_TILE, RANK_TILE / 2, 0, st>>>(keys, idx, 2, RANK_TILE);     // sorted tiles, alternating direction
     h->launches += 2;
     for (int kk = RANK_TILE * 2; kk <= n_pow2; kk <<= 1) {
         for (int j = kk >> 1; j >= RANK_TILE; j >>= 1) {
-            rank_sort_global_kernel<<<(n_pow2 / 2 + 255) / 256, 256, 0, st>>>(keys, h->rank_idx, n_pow2, kk, j);
+            rank_sort_global_kernel<<<(n_pow2 / 2 + 255) / 256, 256, 0, st>>>(keys, idx, n_pow2, kk, j);
             h->launches++;
         }
-        rank_sort_tile_kernel<<<n_pow2 / RANK_TILE, RANK_TILE / 2, 0, st>>>(keys, h->rank_idx, kk, kk);        // distances below the tile size
+        rank_sort_tile_kernel<<<n_pow2 / RANK_TILE, RANK_TILE / 2, 0, st>>>(keys, idx, kk, kk);        // distances below the tile size
         h->launches++;
     }
-    select_order_stat_kernel<<<(k + 255) / 256, 256, 0, st>>>(keys, h->rank_idx, n, k, T, seed, generation, parent_idx);
+    select_order_stat_kernel<<<(k + 255) / 256, 256, 0, st>>>(keys, idx, n, k, T, seed, generation, parent_idx);
     h->launches++;
     NGP_CUDA(cudaGetLastError());
     return NGP_OK;
@@ -856,12 +841,8 @@ extern "C" int ngp_ga_step(ngp_handle *h, const float *genomes, const double *fi
     int T = h->cfg.tournament_size;
     if (T < 1) T = 1;
     if (!parent_idx) {
-        if ((size_t)n > h->cap_parent) {
-            cudaFree(h->d_parent); h->d_parent = nullptr; h->cap_parent = 0;
-            NGP_CUDA(cudaMalloc(&h->d_parent, (size_t)n * sizeof(int32_t)));
-            h->cap_parent = n;
-        }
-        parent_idx = h->d_parent;
+        NGP_CUDA(h->d_parent.ensure(n));
+        parent_idx = h->d_parent.p;
     }
     if (stats) {
         fitness_stats_kernel<<<1, 1024, 0, st>>>(fitness, n, stats);

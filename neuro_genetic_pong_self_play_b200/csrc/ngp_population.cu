@@ -107,15 +107,6 @@ __global__ void hof_gather_kernel(HofArgs a, const int32_t *__restrict__ count, 
     if (threadIdx.x == 0) { out_fitness[m] = hof_fit(a, v); out_hash[m] = hof_hash_of(a, v); }
 }
 
-static int ensure(void **p, size_t *cap, size_t bytes)
-{
-    if (bytes <= *cap) return NGP_OK;
-    cudaFree(*p); *p = nullptr; *cap = 0;
-    NGP_CUDA(cudaMalloc(p, bytes));
-    *cap = bytes;
-    return NGP_OK;
-}
-
 extern "C" int ngp_hof_update(ngp_handle *h, float *hof_genomes, double *hof_fitness, int32_t *n_hof, int32_t maxsize,
                               const float *genomes, const double *fitness, int32_t n, void *stream)
 {
@@ -126,36 +117,35 @@ extern "C" int ngp_hof_update(ngp_handle *h, float *hof_genomes, double *hof_fit
     NGP_CUDA(cudaSetDevice(h->device));
     cudaStream_t st = (cudaStream_t)stream;
     const int G = h->gene_size;
-    int rc;
-    if ((rc = ensure((void **)&h->hof_hash_old, &h->hof_cap_hash_old, (size_t)maxsize * 8))) return rc;
-    if ((rc = ensure((void **)&h->hof_hash_new, &h->hof_cap_hash_new, (size_t)n * 8))) return rc;
-    if ((rc = ensure((void **)&h->hof_order, &h->hof_cap_order, ((size_t)maxsize + 2) * 4))) return rc;
-    if ((rc = ensure((void **)&h->hof_tmp_genomes, &h->hof_cap_tmp_genomes, (size_t)maxsize * G * 4))) return rc;
-    if ((rc = ensure((void **)&h->hof_tmp_fitness, &h->hof_cap_tmp_fitness, (size_t)maxsize * 16))) return rc;
+    NGP_CUDA(h->hof_hash_old.ensure(maxsize));
+    NGP_CUDA(h->hof_hash_new.ensure(n));
+    NGP_CUDA(h->hof_order.ensure((size_t)maxsize + 2));
+    NGP_CUDA(h->hof_tmp_genomes.ensure((size_t)maxsize * G));
+    NGP_CUDA(h->hof_tmp_fitness.ensure((size_t)maxsize * 2));          // fitness, then the hashes as 64-bit words
     if (*n_hof > 0) {
-        genome_hash_kernel<<<(unsigned)(((long long)*n_hof * 32 + 255) / 256), 256, 0, st>>>(hof_genomes, *n_hof, G, h->hof_hash_old);
+        genome_hash_kernel<<<(unsigned)(((long long)*n_hof * 32 + 255) / 256), 256, 0, st>>>(hof_genomes, *n_hof, G, h->hof_hash_old.p);
         h->launches++;
     }
-    genome_hash_kernel<<<(unsigned)(((long long)n * 32 + 255) / 256), 256, 0, st>>>(genomes, n, G, h->hof_hash_new);
+    genome_hash_kernel<<<(unsigned)(((long long)n * 32 + 255) / 256), 256, 0, st>>>(genomes, n, G, h->hof_hash_new.p);
     h->launches++;
     NGP_CUDA(cudaGetLastError());
     HofArgs a;
-    a.hof_genomes = hof_genomes; a.hof_fitness = hof_fitness; a.hof_hash = h->hof_hash_old;
-    a.genomes = genomes; a.fitness = fitness; a.hash = h->hof_hash_new;
+    a.hof_genomes = hof_genomes; a.hof_fitness = hof_fitness; a.hof_hash = h->hof_hash_old.p;
+    a.genomes = genomes; a.fitness = fitness; a.hash = h->hof_hash_new.p;
     a.n_hof = *n_hof; a.maxsize = maxsize; a.n = n; a.G = G;
-    a.order = h->hof_order; a.out_count = h->hof_order + maxsize + 1;
+    a.order = h->hof_order.p; a.out_count = h->hof_order.p + maxsize + 1;
     hof_update_kernel<<<1, 1024, 0, st>>>(a);
     h->launches++;
     NGP_CUDA(cudaGetLastError());
-    double *tmp_fit = h->hof_tmp_fitness;
-    uint64_t *tmp_hash = reinterpret_cast<uint64_t *>(h->hof_tmp_fitness + maxsize);
-    hof_gather_kernel<<<maxsize, 128, 0, st>>>(a, a.out_count, h->hof_tmp_genomes, tmp_fit, tmp_hash);
+    double *tmp_fit = h->hof_tmp_fitness.p;
+    uint64_t *tmp_hash = reinterpret_cast<uint64_t *>(tmp_fit + maxsize);
+    hof_gather_kernel<<<maxsize, 128, 0, st>>>(a, a.out_count, h->hof_tmp_genomes.p, tmp_fit, tmp_hash);
     h->launches++;
     NGP_CUDA(cudaGetLastError());
-    NGP_CUDA(cudaMemcpyAsync(h->h_counters + 3, a.out_count, 4, cudaMemcpyDeviceToHost, st));
+    NGP_CUDA(cudaMemcpyAsync(h->h_counters.p + 3, a.out_count, 4, cudaMemcpyDeviceToHost, st));
     NGP_CUDA(cudaStreamSynchronize(st));
-    const int count = (int)(h->h_counters[3] & 0xFFFFFFFFull);
-    NGP_CUDA(cudaMemcpyAsync(hof_genomes, h->hof_tmp_genomes, (size_t)count * G * 4, cudaMemcpyDeviceToDevice, st));
+    const int count = (int)(h->h_counters.p[3] & 0xFFFFFFFFull);
+    NGP_CUDA(cudaMemcpyAsync(hof_genomes, h->hof_tmp_genomes.p, (size_t)count * G * 4, cudaMemcpyDeviceToDevice, st));
     NGP_CUDA(cudaMemcpyAsync(hof_fitness, tmp_fit, (size_t)count * 8, cudaMemcpyDeviceToDevice, st));
     NGP_CUDA(cudaStreamSynchronize(st));
     *n_hof = count;

@@ -195,32 +195,24 @@ int ngp_evaluate_stepwise(ngp_handle *h, const RolloutParams &p, cudaStream_t st
     const bool rr = p.schedule == NGP_SCHEDULE_ROUND_ROBIN;
     const bool hof = !rr && p.n_hof > 0 && p.games > 3;
     const long long rows = rr ? 2ll * total : total, rows_hof = hof ? 3ll * p.n : 0;
-    const size_t need_env = (size_t)total * sizeof(StepEnv), need_x = (size_t)(rows + rows_hof) * 6 * sizeof(float), need_act = (size_t)(rows + rows_hof);
-    const size_t need_opp = (size_t)rows_hof * p.G * sizeof(float);
-    if (need_opp > (size_t)32 << 30) {
+    const size_t n_x = (size_t)(rows + rows_hof) * 6, n_act = (size_t)(rows + rows_hof), n_opp = (size_t)rows_hof * p.G;
+    if (n_opp * sizeof(float) > (size_t)32 << 30) {
         ngp_set_error("ngp_evaluate: %lld hall-of-fame opponents of %d genes need more than 32 GiB of gathered weights", rows_hof, p.G);
         return NGP_ERR_UNSUPPORTED;
     }
-    auto grow = [](void **ptr, size_t &cap, size_t need) -> cudaError_t {
-        if (need <= cap) return cudaSuccess;
-        cudaFree(*ptr); *ptr = nullptr; cap = 0;
-        cudaError_t e = cudaMalloc(ptr, need);
-        if (e == cudaSuccess) cap = need;
-        return e;
-    };
-    NGP_CUDA(grow(&h->step_envs, h->step_cap_envs, need_env));
-    NGP_CUDA(grow((void **)&h->step_x, h->step_cap_x, need_x));
-    NGP_CUDA(grow((void **)&h->step_act, h->step_cap_act, need_act));
-    if (hof) NGP_CUDA(grow((void **)&h->step_opp, h->step_cap_opp, need_opp));
-    StepEnv *envs = (StepEnv *)h->step_envs;
-    float *x = h->step_x, *x_hof = h->step_x + rows * 6;
-    uint8_t *act = h->step_act, *act_hof = h->step_act + rows;
-    NGP_CUDA(cudaMemsetAsync(x, 0, need_x, st));                 // rows of frames without a model call are never read, but keep them finite
-    NGP_CUDA(cudaMemsetAsync(act, 0, need_act, st));
+    NGP_CUDA(h->step_envs.ensure((size_t)total * sizeof(StepEnv)));
+    NGP_CUDA(h->step_x.ensure(n_x));
+    NGP_CUDA(h->step_act.ensure(n_act));
+    if (hof) NGP_CUDA(h->step_opp.ensure(n_opp));
+    StepEnv *envs = reinterpret_cast<StepEnv *>(h->step_envs.p);
+    float *x = h->step_x.p, *x_hof = x + rows * 6;
+    uint8_t *act = h->step_act.p, *act_hof = act + rows;
+    NGP_CUDA(cudaMemsetAsync(x, 0, n_x * sizeof(float), st));    // rows of frames without a model call are never read, but keep them finite
+    NGP_CUDA(cudaMemsetAsync(act, 0, n_act, st));
     step_begin_kernel<<<(total + 127) / 128, 128, 0, st>>>(p, envs, total);
     h->launches++;
     if (hof) {
-        step_gather_opponents_kernel<<<(unsigned)rows_hof, 256, 0, st>>>(p, h->step_opp);
+        step_gather_opponents_kernel<<<(unsigned)rows_hof, 256, 0, st>>>(p, h->step_opp.p);
         h->launches++;
     }
     NGP_CUDA(cudaGetLastError());
@@ -237,16 +229,16 @@ int ngp_evaluate_stepwise(ngp_handle *h, const RolloutParams &p, cudaStream_t st
         int rc = ngp_mlp_forward_prepared(h, p.genomes, x, p.n, per_genome, act, nullptr, st);
         if (rc != NGP_OK) return rc;
         if (hof) {
-            rc = ngp_mlp_forward(h, h->step_opp, x_hof, (int32_t)rows_hof, 1, act_hof, nullptr, st);
+            rc = ngp_mlp_forward(h, h->step_opp.p, x_hof, (int32_t)rows_hof, 1, act_hof, nullptr, st);
             if (rc != NGP_OK) return rc;
         }
         step_decide_kernel<<<(total + 127) / 128, 128, 0, st>>>(p, envs, total, act, act_hof);
         h->launches++;
         NGP_CUDA(cudaGetLastError());
         if (frame % CHECK_EVERY == 0) {
-            NGP_CUDA(cudaMemcpyAsync(h->h_counters, h->d_counters, 4 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+            NGP_CUDA(cudaMemcpyAsync(h->h_counters.p, h->d_counters.p, 4 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
             NGP_CUDA(cudaStreamSynchronize(st));
-            if (h->h_counters[3] >= (unsigned long long)total) break;
+            if (h->h_counters.p[3] >= (unsigned long long)total) break;
         }
     }
     return NGP_OK;
