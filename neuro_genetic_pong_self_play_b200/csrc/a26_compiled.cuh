@@ -17,8 +17,12 @@ enum : int { ERR_UNTRANSLATED = 4 };
 
 // hooks emitted by the generator at the head of dispatch entries $F621, $F58D and $F5CC (pong_superblocks.cuh)
 #ifndef A26_NO_SUPERBLOCKS
+// the display-loop block's queue placement follows the flavour (superblock_f621); tests/host_sim builds can force either one
+#ifndef A26_SB_REPLAY_AT_TOP
+#define A26_SB_REPLAY_AT_TOP SYNC
+#endif
 #define A26_SUPERBLOCK_F621 \
-    if (superblock_f621<VERIFY>(s, T, ram, fb, a, x, y, sp, pc, fc, fv, nv, zv, fid, cyc, cpu_ls, sb_iters)) { A26_STAT(6); goto a26_next_; }
+    if (superblock_f621<VERIFY, A26_SB_REPLAY_AT_TOP>(s, T, ram, fb, a, x, y, sp, pc, fc, fv, nv, zv, fid, cyc, cpu_ls, sb_iters)) { A26_STAT(6); goto a26_next_; }
 #define A26_SUPERBLOCK_F58D \
     if (superblock_f58d<VERIFY>(s, T, ram, fb, a, x, y, pc, fc, nv, zv, cyc, cpu_ls, sb_iters)) { A26_STAT(7); goto a26_next_; }
 #define A26_SUPERBLOCK_F5CC \

@@ -571,6 +571,18 @@ __device__ __noinline__ void render_span(Chip &s_, const Tables &T_, int x0, int
     }
 }
 
+// black VBLANK pixels x0..x1 of a crop row (only reached when a target colour has a 0 channel: out of line, so that the
+// copies of render_to() do not carry it)
+static __device__ __noinline__ void render_black_span(Chip &s_, const Tables &T_, int x0, int x1, int row)
+{
+    Chip &s = chip_local(s_);
+    const Tables &T = tables_shared(T_);
+    Masks R;
+#pragma unroll
+    for (int i = 0; i < 5; ++i) R.w[i] = range_word(i, x0, x1);
+    accumulate_class(s, T, 0, R, row - CROP_TOP);
+}
+
 // advance the renderer to pixel x of the current scanline
 template <bool VERIFY>
 __device__ __forceinline__ void render_to(Chip &s, const Tables &T, int x, uint8_t *fb)
@@ -584,12 +596,7 @@ __device__ __forceinline__ void render_to(Chip &s, const Tables &T, int x, uint8
         }
         // VBLANK: black; the framebuffer is pre-cleared to 0 and black matches no target channel
         // unless a target colour has a 0 channel, which accumulate_class would need to see:
-        else if (row >= CROP_TOP && row < CROP_BOTTOM && T.weight[0]) {
-            Masks R;
-#pragma unroll
-            for (int i = 0; i < 5; ++i) R.w[i] = range_word(i, s.rx, x);
-            accumulate_class(s, T, 0, R, row - CROP_TOP);
-        }
+        else if (row >= CROP_TOP && row < CROP_BOTTOM && T.weight[0]) render_black_span(s, T, s.rx, x, row);
     }
     s.rx = x;
 }
@@ -616,10 +623,14 @@ __device__ __forceinline__ void render_full_lines(Chip &s, const Tables &T, int 
     for (int i = 0; i < k; ++i) { render_to<VERIFY>(s, T, FB_COLS, fb); tia_newline(s, 1); }
 }
 
-// bring the TIA up to colour clock h, measured from the start of its current scanline
+// bring the TIA up to colour clock h, measured from the start of its current scanline.  Out of line: one copy of the renderer's
+// catch-up serves register writes, collision reads and the end of a frame (inlined, each of them carried its own ~12 KB of SASS,
+// all of it fetched every frame).
 template <bool VERIFY>
-__device__ __forceinline__ void tia_catchup(Chip &s, const Tables &T, int h, uint8_t *fb)
+__device__ __noinline__ void tia_catchup(Chip &s_, const Tables &T_, int h, uint8_t *fb)
 {
+    Chip &s = chip_local(s_);
+    const Tables &T = tables_shared(T_);
     if (!VERIFY && h > LINE_CLOCKS && !(s.hmove_blank | s.suppress) && !(s.vblank & 2)) {
         // several lines with one register state: one classification of the objects for all of them
         const int hh = h - LINE_CLOCKS, full = (hh - 1) / LINE_CLOCKS;

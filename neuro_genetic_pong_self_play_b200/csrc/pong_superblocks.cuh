@@ -54,7 +54,8 @@ __device__ __forceinline__ uint32_t sb_php(uint32_t r, uint32_t c, uint32_t v, u
 //   $F5E0-$F61F  first line of the next pair: ENAM0, GRP1, PF0-2, GRP0 value, ENABL, STX WSYNC
 // Up to max_iters iterations run back to back, until the loop test ends the loop.
 // Returns false (nothing touched) when a guard fails; otherwise pc is $F63E (loop ended) or $F621.
-template <bool VERIFY>
+// REPLAY_AT_TOP: where the queue of deferred writes is made room for (see the loop).
+template <bool VERIFY, bool REPLAY_AT_TOP>
 __device__ __forceinline__ bool superblock_f621(Chip &s, const Tables &T, Ram ram, uint8_t *fb, uint32_t &a, uint32_t &x, uint32_t &y,
                                                 uint32_t &sp, uint32_t &pc, uint32_t &fc, uint32_t &fv, uint32_t &nv, uint32_t &zv,
                                                 uint32_t fid, uint32_t &cyc, uint32_t cpu_ls, int max_iters)
@@ -115,8 +116,16 @@ __device__ __forceinline__ bool superblock_f621(Chip &s, const Tables &T, Ram ra
         }                                                                                                      \
     } while (0)
     uint32_t rel = (cyc - cpu_ls) % LINE_CYCLES;                        // see sb_wsync
-    // bounded by the caller (at most one trip of X through its 8-bit range), then back through the dispatcher
+    pc = 0xF621u;
+    // bounded by the caller (at most one trip of X through its 8-bit range), then back through the dispatcher.
+    // Every copy of replay() is a loop around a call of tia_poke_changed().  REPLAY_AT_TOP makes room at the top of every
+    // iteration (an iteration queues at most eight writes) and so needs one copy besides the one after the loop: ~20
+    // registers and a sixth of the spills fewer in the CTA-synchronous flavours, whose register budgets are capped (config 3:
+    // 4-6 % faster, measured).  The one-warp flavour has registers to spare and keeps the test off the iteration's path: room
+    // is made only where writes are queued (config 2: 2 % faster that way; profiles/r03a_rollout_ab.txt).
+    // Replaying earlier or later changes nothing: the renderer reads no RAM, and every event carries its latch block.
     for (int iter = 0; iter < max_iters; ++iter) {
+        if (REPLAY_AT_TOP && n_ev > MAX_EVENTS - 8) replay();
         const uint32_t x1 = (x + 1u) & 0xFFu, x2 = (x + 2u) & 0xFFu;
         const uint32_t row = x1 >> 3;                                   // TXA, LSR x3, TAY
         const uint32_t t0 = cyc;
@@ -136,13 +145,12 @@ __device__ __forceinline__ bool superblock_f621(Chip &s, const Tables &T, Ram ra
         if (in1) k += 3u; else { ram.wr(0x85u, x); k += 5u; }
         // ---- CPX #$DC ; BNE $F5E0 ----
         if (x == 0xDCu) {
-            if (n_ev > MAX_EVENTS - 2) replay();
+            if (!REPLAY_AT_TOP && n_ev > MAX_EVENTS - 2) replay();
             A26_SB_WRITE(0x1B, v_grp0, t0 + 3u);
             A26_SB_WRITE(0x1E, v_enam1, t0 + 16u);
-            replay();
             a = in1; y = sel; sp = 0x1Du; fc = 1u; fv = v; nv = zv = 0u;
             cyc = t0 + k + 4u; pc = 0xF63Eu;
-            return true;
+            break;
         }
         k += 6u;                                                        // CPX 2 + taken branch across a page 4
         // ---- $F5E0 TXA ; LDY #$F0 ; SEC ; SBC $B3 ; AND $A6 ; BEQ ; LDY #$00 ----
@@ -181,7 +189,7 @@ __device__ __forceinline__ bool superblock_f621(Chip &s, const Tables &T, Ram ra
         prev_a = pack_a; prev_b = pack_b;
         if (steady < 2) {
             if (!hot_display_writes(hot, v_grp0, v_enam1, v_enam0, g1, v_pf0, v_pf1, v_pf2, v_enabl)) {
-                if (n_ev > MAX_EVENTS - 8) replay();
+                if (!REPLAY_AT_TOP && n_ev > MAX_EVENTS - 8) replay();
                 A26_SB_WRITE(0x1B, v_grp0, t0 + 3u);
                 A26_SB_WRITE(0x1E, v_enam1, t0 + 16u);
                 A26_SB_WRITE(0x1D, v_enam0, t0 + t_enam0);
@@ -196,7 +204,6 @@ __device__ __forceinline__ bool superblock_f621(Chip &s, const Tables &T, Ram ra
         cyc = t0 + k + sb_wsync(rel, k);                                // k <= 153: within three lines of the iteration's line start
     }
     replay();
-    pc = 0xF621u;
     return true;
 #undef A26_SB_WRITE
 }
