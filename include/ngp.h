@@ -149,6 +149,34 @@ int ngp_evaluate_host(ngp_handle *h, const float *genomes, int32_t n, const floa
                       const double *hof_fitness, int32_t n_hof, uint64_t seed, uint64_t generation,
                       double *fitness, uint64_t *frames_total);
 
+/* left-player codes of ngp_play_matches that are not genome rows */
+enum { NGP_OPP_HARDCODED = -1,         /* dumb_ais.HardcodedAi: game 0 of main.evaluate */
+       NGP_OPP_SCORE_HARDCODED = -2,   /* dumb_ais.ScoreHardcodedAi: game 2 */
+       NGP_OPP_ROBOT = -3 };           /* the cartridge robot game: game 1 ('Start', players=1, HardcodedAi on action[6:8]) */
+
+/* ---- an explicit match list in one fused launch.  Generalises main.evaluate's schedule (main.py:28-66): cross tables
+ * between generations, every genome against the scripted opponents, custom tournaments.
+ * genomes: device f32[n_genomes][G]; right, left: device i32[n_matches].  Match m is one perform_episode
+ * (main.py:69-112): genome row right[m] plays on the right; left[m] is a genome row, which plays on the left with the
+ * x-mirrored inputs as in self-play, or an NGP_OPP_* code.  mult: optional device f64[n_matches], the hall-of-fame
+ * multiplier on the right player's score bonus (calculate_reward, utils.py:104-109); NULL = 1.0.
+ * Outputs (device): rewards f64[n_matches], the right player's reward by ngp_evaluate's formula; frames i32[n_matches]
+ * (env.step calls, may be NULL); scores i32[n_matches][2] = (score1, score2) as the cartridge keeps them (RAM $8D, $8E),
+ * i.e. the left and the right player's points (may be NULL).  The fall-back random actions of get_actions are keyed by
+ * Philox(seed, generation, m, frame, player): ngp_evaluate's key with environment index = match index.  win_score,
+ * timeout_thresh, max_frames, time_scaler, paddle height, colours, button map and core come from the handle's config;
+ * schedule, games_to_play and the hall of fame play no part.  *frames_total (host, may be NULL) and the emulator-error
+ * report behave as in ngp_evaluate.
+ * A right[m] outside [0, n_genomes), a left[m] that is neither a row nor an NGP_OPP_* code, or n_matches < 1 return
+ * NGP_ERR_INVALID and nothing is played: the lists are checked on the device and the count of bad entries is read back,
+ * so the call synchronises its stream once before the rollout is launched.  Networks wider than the fused rollout
+ * takes (any layer > 32 units) return NGP_ERR_UNSUPPORTED. */
+int ngp_play_matches(ngp_handle *h, const float *genomes, int32_t n_genomes,
+                     const int32_t *right, const int32_t *left, const double *mult, int32_t n_matches,
+                     uint64_t seed, uint64_t generation,
+                     double *rewards, int32_t *frames, int32_t *scores,
+                     uint64_t *frames_total, void *stream);
+
 /* ---- K4: GA step.  Replaces toolbox.select / varAnd(mate, mutate) inside eaSimple
  * (ga.py:89-94, main.py:165-170; DEAP selTournament, cxBlend, mutGaussian).
  * Injected noise (all device, all optional = NULL -> Philox(seed, generation)). */

@@ -10,6 +10,7 @@
 #include <stdlib.h>
 #include <string.h>
 
+#include <algorithm>
 #include <map>
 #include <memory>
 #include <mutex>
@@ -212,6 +213,7 @@ __global__ void __launch_bounds__(MAXT, 1) rollout_kernel(RolloutParams p)
             if (done) {
                 p.rewards[ep.env] = reward;
                 p.frames[ep.env] = ep.frame;
+                if (p.scores) { p.scores[2 * ep.env] = ep.last_s1; p.scores[2 * ep.env + 1] = ep.last_s2; }
                 if (s.error) atomicAdd(&p.counters[2], 1ull);
                 ep.env = -1;
             }
@@ -232,6 +234,19 @@ __global__ void fitness_reduce_kernel(const double *__restrict__ rewards, int n,
     double sum = 0.0;
     for (int k = 0; k < games; ++k) sum = __dadd_rn(sum, rewards[(size_t)g * games + k]);
     fitness[g] = __ddiv_rn(sum, (double)games);
+}
+
+// ngp_play_matches' argument check: counts the match entries that name no genome row (right) or neither a row nor an
+// NGP_OPP_* code (left)
+__global__ void match_check_kernel(const int32_t *__restrict__ right, const int32_t *__restrict__ left, int n, int n_genomes,
+                                   unsigned long long *bad)
+{
+    unsigned long long c = 0;
+    for (int m = blockIdx.x * blockDim.x + threadIdx.x; m < n; m += gridDim.x * blockDim.x) {
+        const int r = right[m], l = left[m];
+        c += (r < 0 || r >= n_genomes) + (l < NGP_OPP_ROBOT || l >= n_genomes);
+    }
+    if (c) atomicAdd(bad, c);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -406,35 +421,13 @@ extern "C" int ngp_env_digest(ngp_handle *h, uint32_t *digest, void *stream)
     return NGP_OK;
 }
 
-extern "C" int ngp_evaluate(ngp_handle *h, const float *genomes, int32_t n, const float *hof_genomes, const double *hof_fitness,
-                            int32_t n_hof, const int32_t *hof_pick, uint64_t seed, uint64_t generation, double *fitness,
-                            double *rewards, int32_t *frames, uint64_t *frames_total, void *stream)
+// The RolloutParams fields both fused entry points fill the same way; everything else starts zero (no match list).
+static RolloutParams rollout_params(const ngp_handle *h, const float *genomes, uint64_t seed, uint64_t generation)
 {
-    NGP_REQUIRE(h && genomes && fitness && n > 0, "ngp_evaluate: bad arguments");
-    NGP_REQUIRE(n_hof == 0 || (hof_genomes && hof_fitness), "ngp_evaluate: hall of fame pointers missing");
-    bool wide = false;            // a layer too wide for the fused thread-per-environment MLP: per-frame stepwise driver (ngp_stepwise.cu)
-    for (int i = 0; i < h->cfg.n_layers; ++i) wide |= h->cfg.nodes[i] > pol::FUSED_MAX_WIDTH;
-    NGP_REQUIRE(!wide || (h->cfg.nodes[0] == 6 && h->cfg.nodes[h->cfg.n_layers - 1] <= 8),
-                "ngp_evaluate: wide networks need 6 inputs and at most 8 outputs");
-    if (h->cfg.schedule == NGP_SCHEDULE_REFERENCE)
-        NGP_REQUIRE(h->cfg.games_to_play <= NGP_GAMES_TO_PLAY, "ngp_evaluate: the reference schedule has at most 6 games");
-    NGP_CUDA(cudaSetDevice(h->device));
-    cudaStream_t st = (cudaStream_t)stream;
-    const int games = h->cfg.games_to_play;
-    const long long total = (long long)n * games;
-    NGP_REQUIRE(total < (1ll << 31), "ngp_evaluate: too many environments");
-    NGP_CUDA(h->d_rewards.ensure(total));
-    NGP_CUDA(h->d_frames.ensure(total));
-    NGP_CUDA(cudaMemsetAsync(h->d_counters.p, 0, 8 * sizeof(unsigned long long), st));
-    RolloutParams p;
+    RolloutParams p = {};
     p.tables = h->d_tables.p; p.needed = h->d_needed.p; p.start = h->d_start.p;
-    p.genomes = genomes; p.hof_genomes = hof_genomes; p.hof_fitness = hof_fitness; p.hof_pick = hof_pick;
-    p.n = n; p.n_hof = n_hof; p.G = h->gene_size; p.games = games; p.schedule = h->cfg.schedule;
+    p.genomes = genomes; p.G = h->gene_size; p.schedule = h->cfg.schedule;
     p.core = h->cfg.core ? 1 : 0;
-    if (p.core && !h->rom_translated) {
-        ngp_set_error("ngp_evaluate: the statically translated core was generated from a different cartridge; use NGP_CORE_INTERPRETER");
-        return NGP_ERR_UNSUPPORTED;
-    }
     p.win_score = h->cfg.win_score; p.timeout_thresh = h->cfg.timeout_thresh; p.max_frames = h->cfg.max_frames;
     p.time_scaler = (double)h->cfg.time_scaler; p.paddle_height = (double)h->cfg.scaled_paddle_height;
     p.seed = seed; p.generation = generation; p.shape = h->shape;
@@ -447,20 +440,13 @@ extern "C" int ngp_evaluate(ngp_handle *h, const float *genomes, int32_t n, cons
                 a[6] = la == pol::ACT_UP; a[7] = la == pol::ACT_DOWN;         // action[6:8] = left (main.py:92)
                 p.input_table[players - 1][la * 3 + ra] = roll::action_to_input(a, players, h->cfg.button_map);
             }
-    p.rewards = rewards ? rewards : h->d_rewards.p; p.frames = frames ? frames : h->d_frames.p; p.counters = h->d_counters.p;
-    if (wide) {
-        const int rc = ngp_evaluate_stepwise(h, p, st);
-        if (rc != NGP_OK) return rc;
-        fitness_reduce_kernel<<<(n + 127) / 128, 128, 0, st>>>(p.rewards, n, games, fitness);
-        h->launches++;
-        NGP_CUDA(cudaGetLastError());
-        if (frames_total) *frames_total = h->h_counters.p[1];
-        if (h->h_counters.p[2]) {
-            ngp_set_error("ngp_evaluate: %llu environments stopped on an emulator error", h->h_counters.p[2]);
-            return NGP_ERR_EMULATOR;
-        }
-        return NGP_OK;
-    }
+    p.counters = h->d_counters.p;
+    return p;
+}
+
+// Launches rollout_kernel over `total` environments, between the profiling events when profiling is on.
+static int launch_rollout(ngp_handle *h, const RolloutParams &p, long long total, cudaStream_t st, const char *who)
+{
     // Launch geometry (measured, profiles/README.md).  Small launches: one-warp CTAs spread over all SMs.  From ~2 warps per
     // SM upwards the CTA-synchronous flavour wins: all warps of a CTA walk through the frame together and share their
     // instruction fetches; the CTA grows with the launch until one 16-warp CTA per SM (128 registers/thread) is reached.
@@ -487,7 +473,10 @@ extern "C" int ngp_evaluate(ngp_handle *h, const float *genomes, int32_t n, cons
     if (h->opt_rollout_lean) lean = h->opt_rollout_lean - 1;       // option value 1..3 = flavour 0 (256), 1 (512), 2 (384)
     if (!sync) lean = 0;
     if (sync && block > (lean == 0 ? 256 : lean == 2 ? 384 : 512)) lean = block > 384 ? 1 : 2;   // the flavour's launch bound must hold the CTA
-    NGP_REQUIRE(block <= (sync ? 512 : p.core ? 256 : 384), "ngp_evaluate: rollout_block exceeds the kernel flavour's launch bound");
+    if (block > (sync ? 512 : p.core ? 256 : 384)) {
+        ngp_set_error("%s: rollout_block exceeds the kernel flavour's launch bound", who);
+        return NGP_ERR_INVALID;
+    }
     auto kernel = !p.core ? rollout_kernel<0, false, 384>
                           : (!sync ? rollout_kernel<1, false, 256>
                                    : (lean == 2 ? rollout_kernel<1, true, 384> : lean == 1 ? rollout_kernel<1, true, 512> : rollout_kernel<1, true, 256>));
@@ -514,19 +503,110 @@ extern "C" int ngp_evaluate(ngp_handle *h, const float *genomes, int32_t n, cons
     h->launches++;
     NGP_CUDA(cudaGetLastError());
     if (ev1) NGP_CUDA(cudaEventRecord(ev1, st));
-    fitness_reduce_kernel<<<(n + 127) / 128, 128, 0, st>>>(p.rewards, n, games, fitness);
-    h->launches++;
-    NGP_CUDA(cudaGetLastError());
-    if (frames_total) {
-        NGP_CUDA(cudaMemcpyAsync(h->h_counters.p, h->d_counters.p, 4 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
-        NGP_CUDA(cudaStreamSynchronize(st));
-        *frames_total = h->h_counters.p[1];
+    return NGP_OK;
+}
+
+// Copies the frame and error counters back (synchronises the stream); the emulator-error report of both fused entry points.
+static int read_rollout_counters(ngp_handle *h, cudaStream_t st, uint64_t *frames_total, const char *who)
+{
+    NGP_CUDA(cudaMemcpyAsync(h->h_counters.p, h->d_counters.p, 4 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+    NGP_CUDA(cudaStreamSynchronize(st));
+    *frames_total = h->h_counters.p[1];
+    if (h->h_counters.p[2]) {
+        ngp_set_error("%s: %llu environments stopped on an emulator error", who, h->h_counters.p[2]);
+        return NGP_ERR_EMULATOR;
+    }
+    return NGP_OK;
+}
+
+extern "C" int ngp_evaluate(ngp_handle *h, const float *genomes, int32_t n, const float *hof_genomes, const double *hof_fitness,
+                            int32_t n_hof, const int32_t *hof_pick, uint64_t seed, uint64_t generation, double *fitness,
+                            double *rewards, int32_t *frames, uint64_t *frames_total, void *stream)
+{
+    NGP_REQUIRE(h && genomes && fitness && n > 0, "ngp_evaluate: bad arguments");
+    NGP_REQUIRE(n_hof == 0 || (hof_genomes && hof_fitness), "ngp_evaluate: hall of fame pointers missing");
+    bool wide = false;            // a layer too wide for the fused thread-per-environment MLP: per-frame stepwise driver (ngp_stepwise.cu)
+    for (int i = 0; i < h->cfg.n_layers; ++i) wide |= h->cfg.nodes[i] > pol::FUSED_MAX_WIDTH;
+    NGP_REQUIRE(!wide || (h->cfg.nodes[0] == 6 && h->cfg.nodes[h->cfg.n_layers - 1] <= 8),
+                "ngp_evaluate: wide networks need 6 inputs and at most 8 outputs");
+    if (h->cfg.schedule == NGP_SCHEDULE_REFERENCE)
+        NGP_REQUIRE(h->cfg.games_to_play <= NGP_GAMES_TO_PLAY, "ngp_evaluate: the reference schedule has at most 6 games");
+    NGP_CUDA(cudaSetDevice(h->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    const int games = h->cfg.games_to_play;
+    const long long total = (long long)n * games;
+    NGP_REQUIRE(total < (1ll << 31), "ngp_evaluate: too many environments");
+    NGP_CUDA(h->d_rewards.ensure(total));
+    NGP_CUDA(h->d_frames.ensure(total));
+    NGP_CUDA(cudaMemsetAsync(h->d_counters.p, 0, 8 * sizeof(unsigned long long), st));
+    RolloutParams p = rollout_params(h, genomes, seed, generation);
+    p.hof_genomes = hof_genomes; p.hof_fitness = hof_fitness; p.hof_pick = hof_pick;
+    p.n = n; p.n_hof = n_hof; p.games = games;
+    if (p.core && !h->rom_translated) {
+        ngp_set_error("ngp_evaluate: the statically translated core was generated from a different cartridge; use NGP_CORE_INTERPRETER");
+        return NGP_ERR_UNSUPPORTED;
+    }
+    p.rewards = rewards ? rewards : h->d_rewards.p; p.frames = frames ? frames : h->d_frames.p;
+    if (wide) {
+        const int rc = ngp_evaluate_stepwise(h, p, st);
+        if (rc != NGP_OK) return rc;
+        fitness_reduce_kernel<<<(n + 127) / 128, 128, 0, st>>>(p.rewards, n, games, fitness);
+        h->launches++;
+        NGP_CUDA(cudaGetLastError());
+        if (frames_total) *frames_total = h->h_counters.p[1];
         if (h->h_counters.p[2]) {
             ngp_set_error("ngp_evaluate: %llu environments stopped on an emulator error", h->h_counters.p[2]);
             return NGP_ERR_EMULATOR;
         }
+        return NGP_OK;
     }
-    return NGP_OK;
+    const int rc = launch_rollout(h, p, total, st, "ngp_evaluate");
+    if (rc != NGP_OK) return rc;
+    fitness_reduce_kernel<<<(n + 127) / 128, 128, 0, st>>>(p.rewards, n, games, fitness);
+    h->launches++;
+    NGP_CUDA(cudaGetLastError());
+    return frames_total ? read_rollout_counters(h, st, frames_total, "ngp_evaluate") : NGP_OK;
+}
+
+extern "C" int ngp_play_matches(ngp_handle *h, const float *genomes, int32_t n_genomes, const int32_t *right, const int32_t *left,
+                                const double *mult, int32_t n_matches, uint64_t seed, uint64_t generation, double *rewards,
+                                int32_t *frames, int32_t *scores, uint64_t *frames_total, void *stream)
+{
+    NGP_REQUIRE(h && genomes && right && left && rewards && n_genomes > 0 && n_matches > 0, "ngp_play_matches: bad arguments");
+    for (int i = 0; i < h->cfg.n_layers; ++i)
+        if (h->cfg.nodes[i] > pol::FUSED_MAX_WIDTH) {
+            // the stepwise driver batches the MLP by genome with a fixed number of rows per genome; a match list has none
+            ngp_set_error("ngp_play_matches: networks with a layer wider than %d units are not supported (the fused rollout only)",
+                          pol::FUSED_MAX_WIDTH);
+            return NGP_ERR_UNSUPPORTED;
+        }
+    if (h->cfg.core && !h->rom_translated) {
+        ngp_set_error("ngp_play_matches: the statically translated core was generated from a different cartridge; use NGP_CORE_INTERPRETER");
+        return NGP_ERR_UNSUPPORTED;
+    }
+    NGP_CUDA(cudaSetDevice(h->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    if (!frames) NGP_CUDA(h->d_frames.ensure(n_matches));
+    NGP_CUDA(cudaMemsetAsync(h->d_counters.p, 0, 8 * sizeof(unsigned long long), st));
+    // the lists live on the device: count their bad entries there and refuse before anything is played
+    const int check_blocks = (int)std::min<long long>(((long long)n_matches + 255) / 256, 4ll * h->sm_count);
+    match_check_kernel<<<check_blocks, 256, 0, st>>>(right, left, n_matches, n_genomes, h->d_counters.p + 3);
+    h->launches++;
+    NGP_CUDA(cudaGetLastError());
+    NGP_CUDA(cudaMemcpyAsync(h->h_counters.p + 3, h->d_counters.p + 3, sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+    NGP_CUDA(cudaStreamSynchronize(st));
+    if (h->h_counters.p[3]) {
+        ngp_set_error("ngp_play_matches: %llu match entries name no genome row (right) or no genome row or NGP_OPP_* code (left)",
+                      h->h_counters.p[3]);
+        return NGP_ERR_INVALID;
+    }
+    RolloutParams p = rollout_params(h, genomes, seed, generation);
+    p.n = n_matches; p.games = 1;
+    p.match_right = right; p.match_left = left; p.match_mult = mult;
+    p.rewards = rewards; p.frames = frames ? frames : h->d_frames.p; p.scores = scores;
+    const int rc = launch_rollout(h, p, n_matches, st, "ngp_play_matches");
+    if (rc != NGP_OK) return rc;
+    return frames_total ? read_rollout_counters(h, st, frames_total, "ngp_play_matches") : NGP_OK;
 }
 
 extern "C" int ngp_profile_enable(ngp_handle *h, int32_t on)

@@ -86,6 +86,11 @@ struct RolloutParams {
     double *rewards;                // [n*games]
     int32_t *frames;                // [n*games]
     unsigned long long *counters;   // [0] next env, [1] frames, [2] errors
+    // ngp_play_matches (null for ngp_evaluate): environment e is match e of an explicit list, played with games = 1
+    const int32_t *match_right;     // [n] genome rows
+    const int32_t *match_left;      // [n] genome rows or NGP_OPP_*
+    const double *match_mult;       // [n] or null (1.0)
+    int32_t *scores;                // [n][2] (score1, score2) at the end of the episode, or null
 };
 
 struct EnvPlan {
@@ -99,6 +104,15 @@ struct EnvPlan {
 __device__ __forceinline__ EnvPlan plan_env(const RolloutParams &p, int e)
 {
     EnvPlan pl;
+    if (p.match_right) {                                   // an explicit match list (ngp_play_matches)
+        const int l = p.match_left[e];
+        pl.right_genome = p.genomes + (size_t)p.match_right[e] * p.G;
+        pl.state = l == NGP_OPP_ROBOT ? NGP_STATE_START_1P : NGP_STATE_START_2P;
+        pl.left_kind = l >= 0 ? pol::KIND_MLP : l == NGP_OPP_SCORE_HARDCODED ? pol::KIND_SCORE_HARDCODED : pol::KIND_HARDCODED;
+        pl.left_genome = l >= 0 ? p.genomes + (size_t)l * p.G : nullptr;
+        pl.mult = p.match_mult ? p.match_mult[e] : 1.0;
+        return pl;
+    }
     const int g = e / p.games, k = e % p.games;
     pl.right_genome = p.genomes + (size_t)g * p.G;
     pl.state = NGP_STATE_START_2P;

@@ -172,6 +172,31 @@ class Engine:
                                         ctypes.byref(total) if sync else None, _stream(self.device)), "ngp_evaluate")
         return {"fitness": fitness, "rewards": rewards, "frames": frames, "frames_total": int(total.value) if sync else None}
 
+    def play_matches(self, genomes: torch.Tensor, right: torch.Tensor, left: torch.Tensor, mult: torch.Tensor | None = None,
+                     seed: int = 0, generation: int = 0, sync: bool = True):
+        """An explicit match list in one fused launch (ngp_play_matches): match m puts genome row right[m] on the right against
+        genome row left[m] (x-mirrored, as in self-play) or an OPP_* code; mult[m] is the hall-of-fame multiplier of the right
+        player's score bonus (None = 1.0).  Returns dict(rewards f64[M] of the right player, frames i32[M], scores i32[M, 2]
+        = (left, right) points, frames_total).  The lists are checked on the device; a bad entry raises NgpError and nothing
+        is played."""
+        self._check_tensor(genomes, torch.float32, "genomes")
+        self._check_tensor(right, torch.int32, "right")
+        self._check_tensor(left, torch.int32, "left")
+        assert genomes.dim() == 2 and genomes.shape[1] == self.gene_size
+        m = right.shape[0]
+        assert right.dim() == 1 and tuple(left.shape) == (m,)
+        if mult is not None:
+            self._check_tensor(mult, torch.float64, "mult")
+            assert tuple(mult.shape) == (m,)
+        rewards = torch.empty(m, dtype=torch.float64, device=self.device)
+        frames = torch.empty(m, dtype=torch.int32, device=self.device)
+        scores = torch.empty((m, 2), dtype=torch.int32, device=self.device)
+        total = ctypes.c_uint64(0)
+        _lib.check(self._L.ngp_play_matches(self._h, _p(genomes), genomes.shape[0], _p(right), _p(left), _p(mult), m, seed, generation,
+                                            _p(rewards), _p(frames), _p(scores), ctypes.byref(total) if sync else None,
+                                            _stream(self.device)), "ngp_play_matches")
+        return {"rewards": rewards, "frames": frames, "scores": scores, "frames_total": int(total.value) if sync else None}
+
     def evaluate_host(self, genomes: np.ndarray, hof_genomes: np.ndarray | None = None, hof_fitness: np.ndarray | None = None,
                       seed: int = 0, generation: int = 0):
         """Same, through host buffers (H2D of genomes and D2H of fitness inside the call)."""

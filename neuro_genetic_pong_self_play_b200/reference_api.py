@@ -9,6 +9,7 @@ Names and argument meaning follow the reference so its call sites read the same:
   run_generations(...)  (eaSimple-shaped loop + logbook)       main.py:157-173
   save_checkpoint / load_latest_population                     utils.py:116-125, ga.py:13-53
   replay(individual) / repeat_upsample                         pickle_inspector.py:1-12, main.py:115-125, utils.py:156-168
+  cross_play(toolbox, a, b)                                    no counterpart: main.evaluate's schedule as any match list
 Every call lands in libngp.so's CUDA kernels through Engine; nothing here computes on the CPU except argument
 marshalling (individuals are rows of device tensors instead of Python lists)."""
 from __future__ import annotations
@@ -188,6 +189,21 @@ class Toolbox:
     def vary(self, genomes: torch.Tensor, fitness: torch.Tensor, noise: dict | None = None):
         """toolbox.select + varAnd(mate, mutate) as one fused GA step."""
         return self.engine.ga_step(genomes, fitness, seed=self.seed, generation=self.generation, noise=noise)
+
+
+def cross_play(toolbox: Toolbox, a: torch.Tensor, b: torch.Tensor):
+    """Every row of `a` on the right against every row of `b` on the left, one fused launch (ngp_play_matches over
+    cat([a, b]), the toolbox's seed and generation): a cross table such as this generation's champions against earlier
+    generations' champions.  Returns dict(reward f64[A][B] of the right player, score i32[A][B][2] = (left, right) points,
+    frames i32[A][B]); match (i, j) is list entry i * B + j."""
+    eng = toolbox.engine
+    genomes = torch.cat([a, b]).to(eng.device, torch.float32).contiguous()
+    A, B = a.shape[0], b.shape[0]
+    rows = torch.arange(A + B, dtype=torch.int32, device=eng.device)
+    right = rows[:A].repeat_interleave(B)
+    left = rows[A:].repeat(A)
+    out = eng.play_matches(genomes, right, left, seed=toolbox.seed, generation=toolbox.generation)
+    return {"reward": out["rewards"].view(A, B), "score": out["scores"].view(A, B, 2), "frames": out["frames"].view(A, B)}
 
 
 def _stats_row(gen, nevals, fit, frames, t0):
