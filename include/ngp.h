@@ -177,6 +177,36 @@ int ngp_play_matches(ngp_handle *h, const float *genomes, int32_t n_genomes,
                      double *rewards, int32_t *frames, int32_t *scores,
                      uint64_t *frames_total, void *stream);
 
+/* One frame of a recorded match (ngp_record_matches): what perform_episode saw and decided on env.step t
+ * (main.py:76-107).  Enough to re-render the game pixel for pixel through ngp_env_step, and the raw material of
+ * behaviour statistics (paddle-ball distance, action mix, fall-back frames, rally lengths). */
+typedef struct {
+    float   loc[3][2];   /* find_stuff after env.step t: (row, col) of ball, left, right in cropped coordinates; 0 when not
+                          * found.  The rollout's FP64 centroid rounded to float, exactly as ngp_env_step rounds its loc */
+    uint8_t valid;       /* bit 0 ball, bit 1 left paddle, bit 2 right paddle found */
+    uint8_t score[2];    /* RAM $8D, $8E after env.step t (score1 = left, score2 = right) */
+    uint8_t act;         /* the decisions taken on frame t, after the bounds clamp: left | right << 2 (NGP_ACT_*); they
+                          * drive env.step t+1 */
+    int32_t timeout;     /* calculate_timeout_and_frames' counter after frame t (main.py:128-135) */
+} ngp_frame_record;      /* 32 bytes */
+
+/* ---- ngp_play_matches with a per-frame trace of every match, recorded inside the same fused launch.
+ * Every argument of ngp_play_matches means what it means there, and with key == NULL rewards, frames, scores and
+ * *frames_total are bit-identical to ngp_play_matches on the same arguments.
+ * record: device ngp_frame_record[n_matches][max_record], 16-byte aligned.  For t < min(frames[m], max_record) entry
+ * m * max_record + t describes env.step t of match m; entries past that are left untouched.  frames[m] always holds the
+ * full length, so a truncated record can be recognised.
+ * key: optional device i32[n_matches], the environment index of the fall-back key Philox(seed, generation, key[m], frame,
+ * player); NULL = m.  With it one match reproduces one game of an ngp_evaluate call exactly: round-robin game k of genome
+ * g has key g * games + k.
+ * Refusals (NGP_ERR_INVALID, nothing written): those of ngp_play_matches, max_record < 1, a NULL or misaligned record, and
+ * any key[m] < 0 (counted on the device with the list check, no further synchronisation).  Networks wider than 32 units
+ * return NGP_ERR_UNSUPPORTED. */
+int ngp_record_matches(ngp_handle *h, const float *genomes, int32_t n_genomes,
+                       const int32_t *right, const int32_t *left, const double *mult, const int32_t *key, int32_t n_matches,
+                       uint64_t seed, uint64_t generation, int32_t max_record, ngp_frame_record *record,
+                       double *rewards, int32_t *frames, int32_t *scores, uint64_t *frames_total, void *stream);
+
 /* ---- K4: GA step.  Replaces toolbox.select / varAnd(mate, mutate) inside eaSimple
  * (ga.py:89-94, main.py:165-170; DEAP selTournament, cxBlend, mutGaussian).
  * Injected noise (all device, all optional = NULL -> Philox(seed, generation)). */

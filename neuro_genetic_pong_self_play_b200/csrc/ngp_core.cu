@@ -17,7 +17,7 @@
 #include <vector>
 
 #include "ngp_internal.h"
-#include "rollout.cuh"
+#include "rollout_kernel.cuh"
 #include "host_tables.h"
 
 // ------------------------------------------------------------------------------------------------
@@ -82,14 +82,6 @@ extern "C" void ngp_default_config(ngp_config *cfg, int32_t population)
 using a26::Chip; using a26::CpuRegs; using a26::Ram; using a26::Snapshot; using a26::Tables;
 using roll::RolloutParams; using roll::load_snapshot; using roll::store_snapshot; using roll::action_to_input;
 using pol::ACT_UP; using pol::ACT_DOWN;
-
-__device__ __forceinline__ void load_tables(Tables &dst, const Tables *__restrict__ src)
-{
-    const uint32_t *s = reinterpret_cast<const uint32_t *>(src);
-    uint32_t *d = reinterpret_cast<uint32_t *>(&dst);
-    for (unsigned i = threadIdx.x; i < sizeof(Tables) / 4; i += blockDim.x) d[i] = s[i];
-    __syncthreads();
-}
 
 // ------------------------------------------------------------------------------------------------
 // start-state construction: power-on + scripted console switches (DESIGN.md "start states")
@@ -179,51 +171,6 @@ __global__ void env_digest_kernel(const Snapshot *envs, int n, uint32_t *out)
     o[7] = s.dump_enabled;
 }
 
-// Fused rollout: one environment (= one game of one genome) per thread.  Lanes are persistent and
-// pull the next environment from a global counter at frame boundaries, so a warp stays in
-// scanline lock-step whatever episode each of its lanes is in.
-template <int CORE, bool SYNC, int MAXT>
-__global__ void __launch_bounds__(MAXT, 1) rollout_kernel(RolloutParams p)
-{
-    __shared__ Tables T;
-    extern __shared__ uint32_t ram_smem[];
-    load_tables(T, p.tables);
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    Ram ram{&ram_smem[warp * 1024 + lane]};
-    const int total = p.n * p.games;
-    Chip s; CpuRegs r;
-    roll::Episode ep;
-    ep.env = -1;
-    bool exhausted = false;
-    unsigned long long my_frames = 0;
-    for (;;) {
-        if (ep.env < 0 && !exhausted) {
-            int e = (int)atomicAdd(&p.counters[0], 1ull);
-            if (e < total) roll::episode_begin(ep, p, e, s, r, ram);
-            else exhausted = true;
-        }
-        const bool active = ep.env >= 0;
-        // SYNC: the CTA walks through frames together (CTA-wide barriers inside the frame), so it also stops together
-        if (SYNC) { if (!__syncthreads_or(active)) break; }
-        else if (__all_sync(0xFFFFFFFFu, !active)) break;
-        if (SYNC || active) {
-            double reward;
-            const bool done = roll::episode_frame<CORE, SYNC>(ep, p, s, r, T, ram, &reward, active);
-            if (active) my_frames++;
-            if (done) {
-                p.rewards[ep.env] = reward;
-                p.frames[ep.env] = ep.frame;
-                if (p.scores) { p.scores[2 * ep.env] = ep.last_s1; p.scores[2 * ep.env + 1] = ep.last_s2; }
-                if (s.error) atomicAdd(&p.counters[2], 1ull);
-                ep.env = -1;
-            }
-        }
-    }
-    // one atomic per warp for the frame counter
-    for (int off = 16; off; off >>= 1) my_frames += __shfl_down_sync(0xFFFFFFFFu, my_frames, off);
-    if (lane == 0 && my_frames) atomicAdd(&p.counters[1], my_frames);
-}
-
 int ngp_evaluate_stepwise(ngp_handle *h, const RolloutParams &p, cudaStream_t st);     // ngp_stepwise.cu
 
 // fitness[g] = sum(rewards[g][:]) / games, summed in game order (main.py:65)
@@ -236,15 +183,15 @@ __global__ void fitness_reduce_kernel(const double *__restrict__ rewards, int n,
     fitness[g] = __ddiv_rn(sum, (double)games);
 }
 
-// ngp_play_matches' argument check: counts the match entries that name no genome row (right) or neither a row nor an
-// NGP_OPP_* code (left)
-__global__ void match_check_kernel(const int32_t *__restrict__ right, const int32_t *__restrict__ left, int n, int n_genomes,
-                                   unsigned long long *bad)
+// the argument check of ngp_play_matches / ngp_record_matches: counts the match entries that name no genome row (right),
+// neither a row nor an NGP_OPP_* code (left), or a negative fall-back key (key, may be null)
+__global__ void match_check_kernel(const int32_t *__restrict__ right, const int32_t *__restrict__ left, const int32_t *__restrict__ key,
+                                   int n, int n_genomes, unsigned long long *bad)
 {
     unsigned long long c = 0;
     for (int m = blockIdx.x * blockDim.x + threadIdx.x; m < n; m += gridDim.x * blockDim.x) {
         const int r = right[m], l = left[m];
-        c += (r < 0 || r >= n_genomes) + (l < NGP_OPP_ROBOT || l >= n_genomes);
+        c += (r < 0 || r >= n_genomes) + (l < NGP_OPP_ROBOT || l >= n_genomes) + (key && key[m] < 0);
     }
     if (c) atomicAdd(bad, c);
 }
@@ -444,8 +391,10 @@ static RolloutParams rollout_params(const ngp_handle *h, const float *genomes, u
     return p;
 }
 
-// Launches rollout_kernel over `total` environments, between the profiling events when profiling is on.
-static int launch_rollout(ngp_handle *h, const RolloutParams &p, long long total, cudaStream_t st, const char *who)
+// Launches rollout_kernel over `total` environments, between the profiling events when profiling is on.  With `rec`
+// (ngp_record_matches) the recording twin of the flavour these rules pick is launched instead.
+static int launch_rollout(ngp_handle *h, const RolloutParams &p, long long total, cudaStream_t st, const char *who,
+                          const roll::RecordArgs *rec = nullptr)
 {
     // Launch geometry (measured, profiles/README.md).  Small launches: one-warp CTAs spread over all SMs.  From ~2 warps per
     // SM upwards the CTA-synchronous flavour wins: all warps of a CTA walk through the frame together and share their
@@ -477,9 +426,10 @@ static int launch_rollout(ngp_handle *h, const RolloutParams &p, long long total
         ngp_set_error("%s: rollout_block exceeds the kernel flavour's launch bound", who);
         return NGP_ERR_INVALID;
     }
-    auto kernel = !p.core ? rollout_kernel<0, false, 384>
-                          : (!sync ? rollout_kernel<1, false, 256>
-                                   : (lean == 2 ? rollout_kernel<1, true, 384> : lean == 1 ? rollout_kernel<1, true, 512> : rollout_kernel<1, true, 256>));
+    const int flavour = !p.core ? 0 : !sync ? 1 : lean == 2 ? 3 : lean == 1 ? 4 : 2;      // rollout_record_kernel's numbering
+    static const RolloutKernel flavours[5] = {rollout_kernel<0, false, 384>, rollout_kernel<1, false, 256>, rollout_kernel<1, true, 256>,
+                                              rollout_kernel<1, true, 384>, rollout_kernel<1, true, 512>};
+    const RolloutKernel kernel = rec ? rollout_record_kernel(flavour) : flavours[flavour];
     const size_t smem = (size_t)block * 32 * 4;
     int per_sm = 0;
     if (smem + sizeof(Tables) > 48 * 1024) NGP_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -499,7 +449,7 @@ static int launch_rollout(ngp_handle *h, const RolloutParams &p, long long total
         h->prof_used++;
         NGP_CUDA(cudaEventRecord(ev0, st));
     }
-    kernel<<<(unsigned)blocks, block, smem, st>>>(p);
+    kernel<<<(unsigned)blocks, block, smem, st>>>(p, rec ? *rec : roll::RecordArgs{});
     h->launches++;
     NGP_CUDA(cudaGetLastError());
     if (ev1) NGP_CUDA(cudaEventRecord(ev1, st));
@@ -568,45 +518,71 @@ extern "C" int ngp_evaluate(ngp_handle *h, const float *genomes, int32_t n, cons
     return frames_total ? read_rollout_counters(h, st, frames_total, "ngp_evaluate") : NGP_OK;
 }
 
-extern "C" int ngp_play_matches(ngp_handle *h, const float *genomes, int32_t n_genomes, const int32_t *right, const int32_t *left,
-                                const double *mult, int32_t n_matches, uint64_t seed, uint64_t generation, double *rewards,
-                                int32_t *frames, int32_t *scores, uint64_t *frames_total, void *stream)
+// ngp_play_matches, and ngp_record_matches when `rec` is set (its record pointer and length already checked)
+static int play_match_list(ngp_handle *h, const float *genomes, int32_t n_genomes, const int32_t *right, const int32_t *left,
+                           const double *mult, const int32_t *key, int32_t n_matches, uint64_t seed, uint64_t generation,
+                           double *rewards, int32_t *frames, int32_t *scores, uint64_t *frames_total, cudaStream_t st,
+                           const roll::RecordArgs *rec, const char *who)
 {
-    NGP_REQUIRE(h && genomes && right && left && rewards && n_genomes > 0 && n_matches > 0, "ngp_play_matches: bad arguments");
+    if (!(h && genomes && right && left && rewards && n_genomes > 0 && n_matches > 0)) {
+        ngp_set_error("%s: bad arguments", who);
+        return NGP_ERR_INVALID;
+    }
     for (int i = 0; i < h->cfg.n_layers; ++i)
         if (h->cfg.nodes[i] > pol::FUSED_MAX_WIDTH) {
             // the stepwise driver batches the MLP by genome with a fixed number of rows per genome; a match list has none
-            ngp_set_error("ngp_play_matches: networks with a layer wider than %d units are not supported (the fused rollout only)",
+            ngp_set_error("%s: networks with a layer wider than %d units are not supported (the fused rollout only)", who,
                           pol::FUSED_MAX_WIDTH);
             return NGP_ERR_UNSUPPORTED;
         }
     if (h->cfg.core && !h->rom_translated) {
-        ngp_set_error("ngp_play_matches: the statically translated core was generated from a different cartridge; use NGP_CORE_INTERPRETER");
+        ngp_set_error("%s: the statically translated core was generated from a different cartridge; use NGP_CORE_INTERPRETER", who);
         return NGP_ERR_UNSUPPORTED;
     }
     NGP_CUDA(cudaSetDevice(h->device));
-    cudaStream_t st = (cudaStream_t)stream;
     if (!frames) NGP_CUDA(h->d_frames.ensure(n_matches));
     NGP_CUDA(cudaMemsetAsync(h->d_counters.p, 0, 8 * sizeof(unsigned long long), st));
     // the lists live on the device: count their bad entries there and refuse before anything is played
     const int check_blocks = (int)std::min<long long>(((long long)n_matches + 255) / 256, 4ll * h->sm_count);
-    match_check_kernel<<<check_blocks, 256, 0, st>>>(right, left, n_matches, n_genomes, h->d_counters.p + 3);
+    match_check_kernel<<<check_blocks, 256, 0, st>>>(right, left, key, n_matches, n_genomes, h->d_counters.p + 3);
     h->launches++;
     NGP_CUDA(cudaGetLastError());
     NGP_CUDA(cudaMemcpyAsync(h->h_counters.p + 3, h->d_counters.p + 3, sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
     NGP_CUDA(cudaStreamSynchronize(st));
     if (h->h_counters.p[3]) {
-        ngp_set_error("ngp_play_matches: %llu match entries name no genome row (right) or no genome row or NGP_OPP_* code (left)",
-                      h->h_counters.p[3]);
+        ngp_set_error(key ? "%s: %llu match entries name no genome row (right), no genome row or NGP_OPP_* code (left) or a negative key"
+                          : "%s: %llu match entries name no genome row (right) or no genome row or NGP_OPP_* code (left)",
+                      who, h->h_counters.p[3]);
         return NGP_ERR_INVALID;
     }
     RolloutParams p = rollout_params(h, genomes, seed, generation);
     p.n = n_matches; p.games = 1;
     p.match_right = right; p.match_left = left; p.match_mult = mult;
     p.rewards = rewards; p.frames = frames ? frames : h->d_frames.p; p.scores = scores;
-    const int rc = launch_rollout(h, p, n_matches, st, "ngp_play_matches");
+    const int rc = launch_rollout(h, p, n_matches, st, who, rec);
     if (rc != NGP_OK) return rc;
-    return frames_total ? read_rollout_counters(h, st, frames_total, "ngp_play_matches") : NGP_OK;
+    return frames_total ? read_rollout_counters(h, st, frames_total, who) : NGP_OK;
+}
+
+extern "C" int ngp_play_matches(ngp_handle *h, const float *genomes, int32_t n_genomes, const int32_t *right, const int32_t *left,
+                                const double *mult, int32_t n_matches, uint64_t seed, uint64_t generation, double *rewards,
+                                int32_t *frames, int32_t *scores, uint64_t *frames_total, void *stream)
+{
+    return play_match_list(h, genomes, n_genomes, right, left, mult, nullptr, n_matches, seed, generation, rewards, frames, scores,
+                           frames_total, (cudaStream_t)stream, nullptr, "ngp_play_matches");
+}
+
+extern "C" int ngp_record_matches(ngp_handle *h, const float *genomes, int32_t n_genomes, const int32_t *right, const int32_t *left,
+                                  const double *mult, const int32_t *key, int32_t n_matches, uint64_t seed, uint64_t generation,
+                                  int32_t max_record, ngp_frame_record *record, double *rewards, int32_t *frames, int32_t *scores,
+                                  uint64_t *frames_total, void *stream)
+{
+    NGP_REQUIRE(max_record >= 1 && record, "ngp_record_matches: needs a record buffer and max_record >= 1");
+    NGP_REQUIRE(((uintptr_t)record & 15) == 0, "ngp_record_matches: the record buffer must be 16-byte aligned");
+    roll::RecordArgs rec;
+    rec.record = record; rec.key = key; rec.max_record = max_record;
+    return play_match_list(h, genomes, n_genomes, right, left, mult, key, n_matches, seed, generation, rewards, frames, scores,
+                           frames_total, (cudaStream_t)stream, &rec, "ngp_record_matches");
 }
 
 extern "C" int ngp_profile_enable(ngp_handle *h, int32_t on)

@@ -3,6 +3,8 @@
 // for debugging).  Reference path: main.evaluate 28-66, main.perform_episode 69-112,
 // main.get_actions 138-154, main.calculate_timeout_and_frames 128-135, utils.calculate_reward 104-109.
 #pragma once
+#include <string.h>
+
 #include "../../include/ngp.h"
 #include "a26_compiled.cuh"
 #include "policy.cuh"
@@ -93,6 +95,39 @@ struct RolloutParams {
     int32_t *scores;                // [n][2] (score1, score2) at the end of the episode, or null
 };
 
+// ngp_record_matches: a separate kernel argument that only the recording twins of rollout_kernel read, so the flavours
+// ngp_evaluate and ngp_play_matches run compile as before
+struct RecordArgs {
+    ngp_frame_record *record;       // [n][max_record], 16-byte aligned
+    const int32_t *key;             // [n] environment index of the fall-back key, or null (= match index)
+    int max_record;
+};
+
+// Half `half` (16 bytes) of record entry (env, frame): one vector store on the device.
+__device__ __forceinline__ void record_store(const RecordArgs &rec, int env, int frame, int half, uint32_t a, uint32_t b, uint32_t c,
+                                             uint32_t d)
+{
+    uint32_t *dst = reinterpret_cast<uint32_t *>(rec.record + (size_t)env * rec.max_record + frame) + 4 * half;
+#ifdef __CUDA_ARCH__
+    *reinterpret_cast<uint4 *>(dst) = make_uint4(a, b, c, d);
+#else
+    dst[0] = a; dst[1] = b; dst[2] = c; dst[3] = d;
+#endif
+}
+
+// the bits of v rounded to float (ngp_env_step's loc rounding)
+__device__ __forceinline__ uint32_t f32_bits(double v)
+{
+    const float f = (float)v;
+#ifdef __CUDA_ARCH__
+    return __float_as_uint(f);
+#else
+    uint32_t u;
+    memcpy(&u, &f, 4);
+    return u;
+#endif
+}
+
 struct EnvPlan {
     int state;
     int left_kind;
@@ -162,6 +197,26 @@ struct Episode {
     EnvPlan plan;
 };
 
+// Record entry ep.frame - 1 of match ep.env (include/ngp.h ngp_frame_record), the frame episode_frame<.., REC = true> has
+// just played, as two 16-byte stores; s1, s2 = its scores.  The centroids are recomputed from the chip's counters exactly
+// as episode_frame computes them.  Out of line on purpose: inlined (at this point or inside episode_frame, in one or two
+// halves) the stores cost the register-capped CTA-synchronous flavours 8-16 B more spill stores and 20-40 B more spill
+// loads per frame than the flavours they twin; called, they spill less than those (profiles/r03c_ptxas.txt).
+static __device__ __noinline__ void record_frame(const RecordArgs &rec, const Episode &ep, const Chip &s, int s1, int s2)
+{
+    uint32_t w[6], vb = 0;
+#pragma unroll
+    for (int t = 0; t < 3; ++t) {
+        const bool v = s.cnt[t] > 0;
+        vb |= (uint32_t)v << t;
+        w[2 * t] = f32_bits(v ? __ddiv_rn((double)s.sy[t], (double)s.cnt[t]) : 0.0);
+        w[2 * t + 1] = f32_bits(v ? __ddiv_rn((double)s.sx[t], (double)s.cnt[t]) : 0.0);
+    }
+    record_store(rec, ep.env, ep.frame - 1, 0, w[0], w[1], w[2], w[3]);
+    record_store(rec, ep.env, ep.frame - 1, 1, w[4], w[5], vb | (uint32_t)s1 << 8 | (uint32_t)s2 << 16 | (uint32_t)(ep.left_act | ep.right_act << 2) << 24,
+                 (uint32_t)ep.timeout);
+}
+
 __device__ __forceinline__ void episode_begin(Episode &ep, const RolloutParams &p, int e, Chip &s, CpuRegs &r, Ram ram)
 {
     ep.env = e;
@@ -177,9 +232,11 @@ __device__ __forceinline__ void episode_begin(Episode &ep, const RolloutParams &
 // then *reward holds main.py:109-112's value.
 // `active` = this lane owns an environment; with SYNC every thread of the CTA must come through here (the
 // frame contains CTA-wide barriers), inactive lanes only take part in the barriers.
-template <int CORE, bool SYNC = false>
+// REC (ngp_record_matches): the fall-back key is rec->key[ep.env] when given; rollout_kernel then stores the frame with
+// record_frame.
+template <int CORE, bool SYNC = false, bool REC = false>
 __device__ __forceinline__ bool episode_frame(Episode &ep, const RolloutParams &p, Chip &s, CpuRegs &r, const Tables &T, Ram ram,
-                                              double *reward, bool active = true)
+                                              double *reward, bool active = true, const RecordArgs *rec = nullptr)
 {
     if (active) {
         const uint32_t in = p.input_table[ep.plan.state == NGP_STATE_START_1P ? 0 : 1][ep.left_act * 3 + ep.right_act];
@@ -211,8 +268,9 @@ __device__ __forceinline__ bool episode_frame(Episode &ep, const RolloutParams &
             left_act = run_policy(p.shape, ep.plan.left_kind, ep.plan.left_genome, fball, flast, loc[1][0], loc[2][0], s1, s2);
             right_act = run_policy(p.shape, pol::KIND_MLP, ep.plan.right_genome, loc[0], lb, loc[2][0], loc[1][0], s1, s2);
         } else {
-            left_act = pol::random_action_bit(p.seed, p.generation, (uint32_t)ep.env, (uint32_t)ep.frame, 0) ? pol::ACT_DOWN : pol::ACT_UP;
-            right_act = pol::random_action_bit(p.seed, p.generation, (uint32_t)ep.env, (uint32_t)ep.frame, 1) ? pol::ACT_DOWN : pol::ACT_UP;
+            const uint32_t key = REC && rec->key ? (uint32_t)rec->key[ep.env] : (uint32_t)ep.env;
+            left_act = pol::random_action_bit(p.seed, p.generation, key, (uint32_t)ep.frame, 0) ? pol::ACT_DOWN : pol::ACT_UP;
+            right_act = pol::random_action_bit(p.seed, p.generation, key, (uint32_t)ep.frame, 1) ? pol::ACT_DOWN : pol::ACT_UP;
         }
     }
     ep.have_last_ball = valid[0];

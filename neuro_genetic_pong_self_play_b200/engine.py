@@ -31,6 +31,14 @@ def _stream(device) -> ctypes.c_void_p:
     return ctypes.c_void_p(torch.cuda.current_stream(device).cuda_stream)
 
 
+def record_views(raw: torch.Tensor) -> dict:
+    """Named views of an ngp_frame_record buffer u8[M, T, 32] (include/ngp.h): loc f32[M, T, 3, 2], valid u8[M, T],
+    score u8[M, T, 2], act u8[M, T], timeout i32[M, T]; `raw` is the buffer itself."""
+    m, t = raw.shape[0], raw.shape[1]
+    return {"raw": raw, "loc": raw[..., 0:24].view(torch.float32).view(m, t, 3, 2), "valid": raw[..., 24],
+            "score": raw[..., 25:27], "act": raw[..., 27], "timeout": raw[..., 28:32].view(torch.int32).view(m, t)}
+
+
 class Engine:
     def __init__(self, config: Config | None = None, device: int | None = None, rom: bytes | None = None):
         if not torch.cuda.is_available():
@@ -196,6 +204,37 @@ class Engine:
                                             _p(rewards), _p(frames), _p(scores), ctypes.byref(total) if sync else None,
                                             _stream(self.device)), "ngp_play_matches")
         return {"rewards": rewards, "frames": frames, "scores": scores, "frames_total": int(total.value) if sync else None}
+
+    def record_matches(self, genomes: torch.Tensor, right: torch.Tensor, left: torch.Tensor, mult: torch.Tensor | None = None,
+                       key: torch.Tensor | None = None, max_record: int = 2048, seed: int = 0, generation: int = 0, sync: bool = True):
+        """play_matches with a per-frame trace of every match, recorded in the same fused launch (ngp_record_matches).
+        key[m] (None = m) is the environment index of the random fall-back key, so that one match can reproduce one game of
+        an evaluate call (round-robin game k of genome g: key g * games + k).  Returns play_matches' dict plus `left` (kept
+        for rendering) and `record`: named views over one u8[M, T, 32] buffer (T = max_record; frame t of match m is valid
+        for t < min(frames[m], T)): loc f32[M, T, 3, 2], valid u8[M, T] (bit 0 ball, 1 left, 2 right), score u8[M, T, 2],
+        act u8[M, T] (left | right << 2, after the bounds clamp) and timeout i32[M, T]."""
+        self._check_tensor(genomes, torch.float32, "genomes")
+        self._check_tensor(right, torch.int32, "right")
+        self._check_tensor(left, torch.int32, "left")
+        assert genomes.dim() == 2 and genomes.shape[1] == self.gene_size
+        m = right.shape[0]
+        assert right.dim() == 1 and tuple(left.shape) == (m,)
+        if mult is not None:
+            self._check_tensor(mult, torch.float64, "mult")
+            assert tuple(mult.shape) == (m,)
+        if key is not None:
+            self._check_tensor(key, torch.int32, "key")
+            assert tuple(key.shape) == (m,)
+        raw = torch.empty((m, max(int(max_record), 0), _lib.NGP_FRAME_RECORD_BYTES), dtype=torch.uint8, device=self.device)
+        rewards = torch.empty(m, dtype=torch.float64, device=self.device)
+        frames = torch.empty(m, dtype=torch.int32, device=self.device)
+        scores = torch.empty((m, 2), dtype=torch.int32, device=self.device)
+        total = ctypes.c_uint64(0)
+        _lib.check(self._L.ngp_record_matches(self._h, _p(genomes), genomes.shape[0], _p(right), _p(left), _p(mult), _p(key), m, seed,
+                                              generation, int(max_record), _p(raw), _p(rewards), _p(frames), _p(scores),
+                                              ctypes.byref(total) if sync else None, _stream(self.device)), "ngp_record_matches")
+        return {"rewards": rewards, "frames": frames, "scores": scores, "frames_total": int(total.value) if sync else None,
+                "left": left, "record": record_views(raw)}
 
     def evaluate_host(self, genomes: np.ndarray, hof_genomes: np.ndarray | None = None, hof_fitness: np.ndarray | None = None,
                       seed: int = 0, generation: int = 0):

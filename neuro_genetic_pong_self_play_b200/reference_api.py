@@ -10,6 +10,7 @@ Names and argument meaning follow the reference so its call sites read the same:
   save_checkpoint / load_latest_population                     utils.py:116-125, ga.py:13-53
   replay(individual) / repeat_upsample                         pickle_inspector.py:1-12, main.py:115-125, utils.py:156-168
   cross_play(toolbox, a, b)                                    no counterpart: main.evaluate's schedule as any match list
+  render_recorded / replay_selfplay                            main.evaluate(render=True) for recorded fused games
 Every call lands in libngp.so's CUDA kernels through Engine; nothing here computes on the CPU except argument
 marshalling (individuals are rows of device tensors instead of Python lists)."""
 from __future__ import annotations
@@ -356,6 +357,76 @@ def replay(toolbox: Toolbox, individual, game: int = 0, upsample=(4, 4), max_fra
             break
     reward = 0.0 if s1 == s2 else ((s2 - s1) + s2 * mult) / (total / cfg.TIME_SCALER)       # utils.calculate_reward, utils.py:104-109
     return {"frames": torch.stack(frames), "reward": reward, "steps": steps, "score": (s1, s2)}
+
+
+def render_recorded(toolbox: Toolbox, rec: dict, matches, upsample=(1, 1), core: int | None = None, want_ram: bool = False):
+    """Re-renders recorded games (Engine.record_matches' result) pixel for pixel: the emulator is deterministic, so the
+    recorded decisions are all it needs.  Each match m in `matches` is played again through env_reset + env_step (verify
+    mode, every pixel), one batch per start state ('Start' with players = 1 for ROBOT matches, 'Start.2P' for the rest):
+    step 0 gets BLANK_ACTION, step t gets BLANK_ACTION with record t-1's decisions written to [4:6] (right) and [6:8] (left),
+    as perform_episode does (main.py:91-92).  Returns one u8[T_m, 210*k, 160*l, 3] device tensor per match, T_m =
+    min(frames[m], max_record); with want_ram, (frames, ram u8[T_m, 128]) pairs.  core: the 6507 core of env_step (None =
+    the toolbox config's CORE).  Resets the engine's stepwise environments (env_reset)."""
+    eng, cfg = toolbox.engine, toolbox.config
+    dev = eng.device
+    core = cfg.CORE if core is None else int(core)
+    matches = [int(m) for m in matches]
+    frames_n = rec["frames"].cpu().tolist()
+    left = rec["left"].cpu().tolist()
+    act = rec["record"]["act"]
+    T_max = act.shape[1]
+    out = {}
+    blank = torch.tensor(cfg.blank_action(), dtype=torch.uint8, device=dev)
+    for state in (_lib.STATE_START_1P, _lib.STATE_START_2P):
+        group = [m for m in dict.fromkeys(matches) if (left[m] == _lib.OPP_ROBOT) == (state == _lib.STATE_START_1P)]
+        if not group:
+            continue
+        lens = [min(frames_n[m], T_max) for m in group]
+        T = max(lens)
+        a = act[torch.tensor(group, device=dev)][:, :T].long()                       # [n, T]: decisions of frame t
+        actions = blank.repeat(T, len(group), 1)                                      # [T, n, 16]: input of env.step t
+        ra, la = (a[:, : T - 1] >> 2).t(), (a[:, : T - 1] & 3).t()
+        actions[1:, :, cfg.RIGHT_ACTION_START] = (ra == _lib.ACT_UP).to(torch.uint8)
+        actions[1:, :, cfg.RIGHT_ACTION_START + 1] = (ra == _lib.ACT_DOWN).to(torch.uint8)
+        actions[1:, :, cfg.RIGHT_ACTION_END] = (la == _lib.ACT_UP).to(torch.uint8)
+        actions[1:, :, cfg.RIGHT_ACTION_END + 1] = (la == _lib.ACT_DOWN).to(torch.uint8)
+        pix = [torch.empty((n, 210, 160, 3), dtype=torch.uint8, device=dev) for n in lens]
+        ram = [torch.empty((n, 128), dtype=torch.uint8, device=dev) for n in lens]
+        eng.env_reset(len(group), state)
+        for t in range(T):
+            step = eng.env_step(actions[t].contiguous(), want_frames=True, want_obs=False, core=core)
+            for i, n in enumerate(lens):
+                if t < n:
+                    pix[i][t] = step["frames"][i]
+                    ram[i][t] = step["ram"][i]
+        for i, m in enumerate(group):
+            out[m] = (repeat_upsample(pix[i], *upsample), ram[i])
+    return [out[m] if want_ram else out[m][0] for m in matches]
+
+
+def replay_selfplay(toolbox: Toolbox, genomes: torch.Tensor, g: int, k: int, upsample=(4, 4)):
+    """Round-robin game k of genome g, played and rendered exactly as Engine.evaluate plays it under SCHEDULE_ROUND_ROBIN
+    with the toolbox's seed and generation: one record_matches call (right = g, left = (g + k + 1) % n, key = g * games + k),
+    then render_recorded.  Returns replay's dict: frames u8[T, 210*k, 160*l, 3], reward, steps, score = (left, right)."""
+    eng, cfg = toolbox.engine, toolbox.config
+    dev = eng.device
+    n, games = genomes.shape[0], cfg.GAMES_TO_PLAY
+    genomes = genomes.to(dev, torch.float32).contiguous()
+
+    def one(v):
+        return torch.tensor([v], dtype=torch.int32, device=dev)
+
+    # an episode ends at the latest when a point has not been scored for TIMEOUT_THRESH frames after the last of the
+    # 2 * WIN_SCORE - 1 points that can be scored
+    bound = cfg.MAX_FRAMES if cfg.MAX_FRAMES > 0 else 2 * cfg.WIN_SCORE * (cfg.TIMEOUT_THRESH + 2)
+    args = (genomes, one(g), one((g + k + 1) % n))
+    rec = eng.record_matches(*args, key=one(g * games + k), max_record=bound, seed=toolbox.seed, generation=toolbox.generation)
+    steps = int(rec["frames"].item())
+    if steps > bound:                                    # never expected; the replay is deterministic, so record it again
+        rec = eng.record_matches(*args, key=one(g * games + k), max_record=steps, seed=toolbox.seed, generation=toolbox.generation)
+    frames = render_recorded(toolbox, rec, [0], upsample=upsample)[0]
+    s1, s2 = (int(v) for v in rec["scores"][0].tolist())
+    return {"frames": frames, "reward": float(rec["rewards"].item()), "steps": steps, "score": (s1, s2)}
 
 
 # ---- checkpoint / resume (utils.py:116-125, ga.py:13-53) -------------------------------------------

@@ -37,10 +37,20 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 PKG = os.path.join(ROOT, "neuro_genetic_pong_self_play_b200")
 CSRC = os.path.join(PKG, "csrc")
 INC = os.path.join(CSRC, "generated", "pong_core.inc")
-KERNELS = {"cfg2": "_Z14rollout_kernelILi1ELb0ELi256EEvN4roll13RolloutParamsE",
-           "sync256": "_Z14rollout_kernelILi1ELb1ELi256EEvN4roll13RolloutParamsE",
-           "sync384": "_Z14rollout_kernelILi1ELb1ELi384EEvN4roll13RolloutParamsE",
-           "sync512": "_Z14rollout_kernelILi1ELb1ELi512EEvN4roll13RolloutParamsE"}
+
+def _rollout(sync, maxt, rec):
+    """mangled name of rollout_kernel<1, sync, maxt, rec>(RolloutParams, RecordArgs) (csrc/rollout_kernel.cuh)"""
+    return f"_Z14rollout_kernelILi1ELb{int(sync)}ELi{maxt}ELb{int(rec)}EEvN4roll13RolloutParamsENS0_10RecordArgsE"
+
+
+# translated-core flavours (ngp_core.cu) and their recording twins (rec_*, ngp_record.cu: ngp_record_matches)
+KERNELS = {"cfg2": _rollout(0, 256, 0), "sync256": _rollout(1, 256, 0), "sync384": _rollout(1, 384, 0), "sync512": _rollout(1, 512, 0),
+           "rec_cfg2": _rollout(0, 256, 1), "rec_sync256": _rollout(1, 256, 1), "rec_sync384": _rollout(1, 384, 1),
+           "rec_sync512": _rollout(1, 512, 1)}
+
+
+def default_object(kernel_key):
+    return os.path.join(PKG, "build", ("ngp_record" if kernel_key.startswith("rec_") else "ngp_core") + ".cu.o")
 NVCC = shutil.which("nvcc") or "/usr/local/cuda/bin/nvcc"
 CUDA_BIN = os.path.dirname(NVCC)
 
@@ -87,10 +97,13 @@ INSN = re.compile(r"^\s+/\*([0-9a-f]{4,})\*/\s+(.*?)\s*;")
 
 def disassemble(obj, kernel, workdir):
     subprocess.check_call([tool("cuobjdump"), "-xelf", "all", obj], cwd=workdir, stdout=subprocess.DEVNULL)
-    cubin = [f for f in os.listdir(workdir) if f.endswith(".cubin") and "ngp_core" in f][0]
+    source = os.path.basename(obj).split(".")[0]                 # ngp_core.cu.o -> ngp_core.sm_100a.cubin
+    cubin = [f for f in os.listdir(workdir) if f.endswith(".cubin") and source in f][0]
     sass = subprocess.run([tool("nvdisasm"), "-gi", "-c", os.path.join(workdir, cubin)], check=True, capture_output=True,
                           text=True).stdout.splitlines()
-    start = next(i for i, l in enumerate(sass) if l.startswith(f".text.{kernel}:"))
+    start = next((i for i, l in enumerate(sass) if l.startswith(f".text.{kernel}:")), None)
+    if start is None:
+        raise SystemExit(f"{kernel} is not in {obj}: the kernel's signature changed, update KERNELS")
     end = next((i for i in range(start + 1, len(sass)) if sass[i].lstrip().startswith(".section")), len(sass))
     out, fn, chain, pending = [], "kernel", [], []
     for line in sass[start:end]:
@@ -270,13 +283,14 @@ def print_table(r):
 
 def main():
     ap = argparse.ArgumentParser(description=__doc__.split("\n")[0])
-    ap.add_argument("--object", default=os.path.join(PKG, "build", "ngp_core.cu.o"),
-                    help="ngp_core.cu object built with -lineinfo (default: the one build.py leaves; built if missing)")
+    ap.add_argument("--object", help="object built with -lineinfo that holds the kernel (default: the ngp_core.cu / ngp_record.cu "
+                                     "object build.py leaves; built if missing)")
     ap.add_argument("--kernel", default="cfg2", choices=sorted(KERNELS))
     ap.add_argument("--frames", type=int, default=400)
     ap.add_argument("--seed", type=int, default=7)
     ap.add_argument("--json", help="write the full report here")
     a = ap.parse_args()
+    a.object = a.object or default_object(a.kernel)
     if not os.path.exists(a.object):
         sys.path.insert(0, ROOT)
         from neuro_genetic_pong_self_play_b200 import build
