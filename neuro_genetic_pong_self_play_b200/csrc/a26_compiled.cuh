@@ -4,7 +4,8 @@
 // statements (generated/pong_core.inc).  This header provides the dispatcher around them.  TIA, RIOT,
 // paddles, rendering and observation accumulation are the same device functions the interpreter
 // (a26_core.cuh::run_frame, the verify-mode core) uses, so only instruction fetch/decode/addressing is
-// specialised.  Control transfers return to `switch (blockmap[pc])`, where diverged lanes re-converge;
+// specialised.  Control transfers that the generator cannot resolve to a known block (and WSYNC, see below) return to
+// `switch (blockmap[pc])`, where diverged lanes re-converge;
 // the loop is scanline-synchronous like the interpreter's.  A program counter outside the translated set
 // raises ERR_UNTRANSLATED (never happens for this cartridge: the traversal covers all of its code).
 #pragma once
@@ -14,6 +15,9 @@
 namespace a26 {
 
 enum : int { ERR_UNTRANSLATED = 4 };
+// A26_STATS counters (indices into a26_stats) of the arrivals at the dispatcher (a26_next_), by what sent the lane there; TRIP_ALL counts every arrival,
+// the ones not named here (super-block exits, backward JMPs, branches too far for a direct jump) are the difference
+enum : int { TRIP_WSYNC = 9, TRIP_RTS = 10, TRIP_JMP_IND = 11, TRIP_BRK_RTI = 12, TRIP_FRAME_END = 13, TRIP_CYCLE_CAP = 14, TRIP_ALL = 15 };
 
 // hooks emitted by the generator at the head of dispatch entries $F621, $F58D and $F5CC (pong_superblocks.cuh)
 #ifndef A26_NO_SUPERBLOCKS
@@ -42,6 +46,7 @@ enum : int { ERR_UNTRANSLATED = 4 };
     do {                                                                               \
         if (solo && (cyc - start_cyc) < FRAME_CYCLE_CAP) goto LABEL_;                  \
         pc = (PC_);                                                                    \
+        A26_STAT(solo ? TRIP_CYCLE_CAP : TRIP_WSYNC);                                  \
         goto a26_next_;                                                                \
     } while (0)
 
@@ -136,7 +141,8 @@ __device__ __forceinline__ void run_frame_compiled(Chip &s, CpuRegs &r, const Ta
                         done = 1;
                         break;
                     }
-                a26_next_:;
+                a26_next_:
+                    A26_STAT(TRIP_ALL);
                 }
                 cpu_ls += (cyc - cpu_ls) / LINE_CYCLES * LINE_CYCLES;
             }

@@ -9,7 +9,9 @@ where diverged lanes of a warp re-converge.  Semantics follow csrc/a26_core.cuh:
 driven interpreter, which stays as the verify-mode core) statement for statement; both are checked
 bit-for-bit against the CPU oracle.
 
-Usage: python tools/gen_rom_core.py        (rewrites the .inc next to the other CUDA sources)
+Usage: python tools/gen_rom_core.py [OUT] [--no-straight-returns]
+  (rewrites the .inc next to the other CUDA sources; --no-straight-returns sends every RTS, RTI, JMP ind and BRK through the
+  dispatcher, the translation before straight returns, which tests/test_host_sim_dispatch_trips.py compares against)
 """
 import hashlib
 import os
@@ -51,17 +53,79 @@ def rb(rom, a):
     return rom[a & 0x7FF]
 
 
+def vector_targets(rom):
+    """targets of JMP ($00A1) / JMP ($00A3): high byte forced to $F3 ($F28D-$F291), low bytes from the 9-byte game
+    records at $F659 (bytes 6 and 8 of each record); sorted"""
+    return sorted({0xF300 | rb(rom, 0xF659 + 9 * rec + k) for rec in range(7) for k in (6, 8)})
+
+
+def return_sites(instrs):
+    """RTS address -> sorted return sites it can go back to: the instruction after every JSR whose target reaches that RTS
+    without passing another RTS (a nested JSR is assumed to return to its own return site; RTI, BRK and JMP ind end the
+    walk).  Any other address an RTS pops (a manipulated stack) still goes through the dispatcher."""
+    sites = {}
+    for j in sorted(a for a, ins in instrs.items() if ins[0] == "JSR"):
+        site = j + 3
+        work, seen = [instrs[j][3] | instrs[j][4] << 8], set()
+        while work:
+            a = 0xF000 | (work.pop() & 0x7FF)
+            if a in seen or a not in instrs:
+                continue
+            seen.add(a)
+            mn, mode, _, b1, b2, n = instrs[a]
+            if mn == "RTS":
+                sites.setdefault(a, set()).add(site)
+            elif mn in ("RTI", "BRK") or (mn == "JMP" and mode == "ind"):
+                pass
+            elif mn == "JMP":
+                work.append(b1 | b2 << 8)
+            elif mn == "JSR":
+                work.append(a + 3)
+            elif mode == "rel":
+                work += [a + 2, a + 2 + (b1 - 256 if b1 > 127 else b1)]
+            else:
+                work.append(a + n)
+    return {r: sorted(v) for r, v in sites.items()}
+
+
+def acyclic_extension(edges, candidates):
+    """The direct jumps (`goto L_xxxx` between dispatch entries, and falling through into the next entry) bypass the
+    dispatcher and with it its FRAME_CYCLE_CAP check, so they must not form a cycle: a chain of them could then run for
+    ever inside one trip.  `edges` (block -> block: fall-through, JSR, forward branches and forward JMPs) must already be
+    acyclic; the in-place loops of backward branches are not in it (each is a short loop of the cartridge that ends), nor
+    is the single-lane WSYNC shortcut (it checks the cap itself).  A candidate (block, target) is accepted, in the given
+    order, only when `target` cannot reach `block` through the edges accepted so far; a refused one keeps its trip through
+    the dispatcher.  Returns the accepted candidates."""
+    succ = {}
+    for a, b in edges:
+        succ.setdefault(a, set()).add(b)
+
+    def reaches(a, b):
+        work, seen = [a], set()
+        while work:
+            x = work.pop()
+            if x == b:
+                return True
+            if x not in seen:
+                seen.add(x)
+                work += succ.get(x, ())
+        return False
+    for a in list(succ):
+        if any(reaches(b, a) for b in succ[a]):
+            raise SystemExit(f"the direct jumps form a cycle through entry {a:04X}")
+    accepted = []
+    for a, b in candidates:
+        if not reaches(b, a):
+            succ.setdefault(a, set()).add(b)
+            accepted.append((a, b))
+    return accepted
+
+
 def traverse(rom):
     """Recursive-descent discovery of instruction starts and block leaders."""
     reset = rb(rom, 0xFFFC) | rb(rom, 0xFFFD) << 8
     irq = rb(rom, 0xFFFE) | rb(rom, 0xFFFF) << 8
-    seeds = {reset, irq}
-    # JMP ($00A1) / JMP ($00A3): high byte forced to $F3 ($F28D-$F291), low bytes from the 9-byte game
-    # records at $F659 (bytes 6 and 8 of each record)
-    for rec in range(7):
-        base = 0xF659 + 9 * rec
-        seeds.add(0xF300 | rb(rom, base + 6))
-        seeds.add(0xF300 | rb(rom, base + 8))
+    seeds = {reset, irq} | set(vector_targets(rom))
     instrs, leaders = {}, set(seeds)
     fwd_branches = {}          # pc -> target, forward conditional branches (candidates for structured emission)
     work = list(seeds)
@@ -157,12 +221,33 @@ def addr_class(a):
 
 
 class Gen:
-    def __init__(self, rom):
+    def __init__(self, rom, straight_returns=True):
         self.rom = rom
         self.instrs, self.leaders, self.structured = traverse(rom)
         self.out = []
         self.goto_targets = set()
         self.inline_backward = True
+        self.return_sites = return_sites(self.instrs)
+        self.vector_targets = vector_targets(rom)
+        self.brk_returns = sorted(a + 2 for a, ins in self.instrs.items() if ins[0] == "BRK")     # where RTI goes back to
+        self.allowed = set()                  # (block, target) of RTS / RTI / JMP ind / BRK that may jump straight there
+        self.straight_returns = straight_returns
+
+    def direct(self, t):
+        """`goto` the label of dispatch entry t from the current block (an edge of the graph acyclic_extension checks)"""
+        self.goto_targets.add(t)
+        self.edges.append((self.cur_block, t))
+        return f"goto L_{t:04X};"
+
+    def known_targets(self, pc, targets, trip):
+        """after a transfer to a computed or constant pc (RTS, RTI, JMP ind, BRK): straight to each of the known targets, any
+        other pc through the dispatcher"""
+        for t in targets:
+            if t in self.leaders and t in self.instrs:
+                self.candidates.append((self.cur_block, t))
+                if (self.cur_block, t) in self.allowed:
+                    self.emit(f"if (pc == 0x{t:04X}u) {self.direct(t)}")
+        self.emit(f"A26_STAT({trip}); goto a26_next_;")
 
     def emit(self, s):
         self.out.append("    " + s)
@@ -256,7 +341,7 @@ class Gen:
         if static_ea is None:
             e(f"A26_WRITE_DYN(ea_, {val}, cyc + {cyc}u);")
             e(f"cyc += {cyc}u + stall_;")
-            e(f"if (done) {{ pc = 0x{nxt:04X}u; goto a26_next_; }}")
+            e(f"if (done) {{ pc = 0x{nxt:04X}u; A26_STAT(TRIP_FRAME_END); goto a26_next_; }}")
             return False
         cls = addr_class(static_ea)
         if cls == "ram":
@@ -273,12 +358,12 @@ class Gen:
                     self.goto_targets.add(nxt)
                     e(f"cyc += {cyc}u; cyc += wsync_stall(cyc, cpu_ls); A26_AFTER_WSYNC(0x{nxt:04X}u, L_{nxt:04X});")
                 else:
-                    e(f"cyc += {cyc}u; cyc += wsync_stall(cyc, cpu_ls); pc = 0x{nxt:04X}u; goto a26_next_;")
+                    e(f"cyc += {cyc}u; cyc += wsync_stall(cyc, cpu_ls); pc = 0x{nxt:04X}u; A26_STAT(TRIP_WSYNC); goto a26_next_;")
                 return True
             e(f"if (!poke_quick(s, 0x{reg:02X}u, {val})) tia_poke_changed<VERIFY>(s, T, 0x{reg:02X}u, {val}, cyc + {cyc}u, cpu_ls, fb);")
             e(f"cyc += {cyc}u + stall_;")
             if reg == 0x00:
-                e(f"if (s.frame_done) {{ done = 1; pc = 0x{nxt:04X}u; goto a26_next_; }}")
+                e(f"if (s.frame_done) {{ done = 1; pc = 0x{nxt:04X}u; A26_STAT(TRIP_FRAME_END); goto a26_next_; }}")
         return False
 
     def is_intim_wait(self, pc, nxt):
@@ -406,17 +491,15 @@ class Gen:
                 self.goto_targets.add(t)
                 e(f"if ({flag} == {want}u) {{ cyc += {taken}u; goto L_{t:04X}; }}")
             elif t > pc and t in self.leaders and t in self.instrs:
-                # forward branch to another block: straight there (cannot loop, so the dispatcher's cycle cap is not needed)
-                self.goto_targets.add(t)
-                e(f"if ({flag} == {want}u) {{ cyc += {taken}u; goto L_{t:04X}; }}")
+                # forward branch to another block: straight there (an edge of the graph acyclic_extension checks)
+                e(f"if ({flag} == {want}u) {{ cyc += {taken}u; {self.direct(t)} }}")
             else:
                 e(f"if ({flag} == {want}u) {{ pc = 0x{t:04X}u; cyc += {taken}u; goto a26_next_; }}")
             e("cyc += 2u;")
         elif mn == "JMP" and mode == "abs":
             t = b1 | b2 << 8
             if t > pc and t in self.leaders and t in self.instrs:
-                self.goto_targets.add(t)
-                e(f"cyc += 3u; goto L_{t:04X};")
+                e(f"cyc += 3u; {self.direct(t)}")
             else:
                 e(f"pc = 0x{t:04X}u; cyc += 3u; goto a26_next_;")
             ends = True
@@ -424,32 +507,34 @@ class Gen:
             p = b1 | b2 << 8
             p2 = (p & 0xFF00) | ((p + 1) & 0xFF)
             e(f"const uint32_t lo_ = bus_read<VERIFY>(s, T, ram, 0x{p & 0x1FFF:04X}u, cyc, 0x{b2:02X}u, fb), hi_ = bus_read<VERIFY>(s, T, ram, 0x{p2 & 0x1FFF:04X}u, cyc, lo_, fb);")
-            e("pc = lo_ | (hi_ << 8); cyc += 5u; goto a26_next_;")
+            e("pc = lo_ | (hi_ << 8); cyc += 5u;")
+            self.known_targets(pc, self.vector_targets, "TRIP_JMP_IND")
             ends = True
         elif mn == "JSR":
             ret = (pc + 2) & 0xFFFF
             e("uint32_t stall_ = 0;")
             e(f"A26_WRITE_DYN(0x100u | sp, 0x{ret >> 8:02X}u, cyc + 4u); sp = (sp - 1) & 0xFFu;")
             e(f"A26_WRITE_DYN(0x100u | sp, 0x{ret & 0xFF:02X}u, cyc + 5u); sp = (sp - 1) & 0xFFu;")
-            # straight to the subroutine's block (no trip through the dispatcher; the matching RTS goes through it)
+            # straight to the subroutine's block (no trip through the dispatcher; the matching RTS returns straight too)
             t = b1 | b2 << 8
             if t in self.leaders and t in self.instrs:
-                self.goto_targets.add(t)
-                e(f"cyc += 6u + stall_; if (done) {{ pc = 0x{t:04X}u; goto a26_next_; }} goto L_{t:04X};")
+                e(f"cyc += 6u + stall_; if (done) {{ pc = 0x{t:04X}u; A26_STAT(TRIP_FRAME_END); goto a26_next_; }} {self.direct(t)}")
             else:
                 e(f"pc = 0x{t:04X}u; cyc += 6u + stall_; goto a26_next_;")
             ends = True
         elif mn == "RTS":
             e("sp = (sp + 1) & 0xFFu; const uint32_t lo_ = bus_read<VERIFY>(s, T, ram, 0x100u | sp, cyc, 0u, fb);")
             e("sp = (sp + 1) & 0xFFu; const uint32_t hi_ = bus_read<VERIFY>(s, T, ram, 0x100u | sp, cyc, lo_, fb);")
-            e("pc = ((lo_ | (hi_ << 8)) + 1) & 0xFFFFu; cyc += 6u; goto a26_next_;")
+            e("pc = ((lo_ | (hi_ << 8)) + 1) & 0xFFFFu; cyc += 6u;")
+            self.known_targets(pc, self.return_sites.get(pc, []), "TRIP_RTS")
             ends = True
         elif mn == "RTI":
             e("sp = (sp + 1) & 0xFFu; const uint32_t p_ = bus_read<VERIFY>(s, T, ram, 0x100u | sp, cyc, 0u, fb);")
             e("A26_UNPACK_P(p_);")
             e("sp = (sp + 1) & 0xFFu; const uint32_t lo_ = bus_read<VERIFY>(s, T, ram, 0x100u | sp, cyc, p_, fb);")
             e("sp = (sp + 1) & 0xFFu; const uint32_t hi_ = bus_read<VERIFY>(s, T, ram, 0x100u | sp, cyc, lo_, fb);")
-            e("pc = lo_ | (hi_ << 8); cyc += 6u; goto a26_next_;")
+            e("pc = lo_ | (hi_ << 8); cyc += 6u;")
+            self.known_targets(pc, self.brk_returns, "TRIP_BRK_RTI")
             ends = True
         elif mn == "BRK":
             ret = (pc + 2) & 0xFFFF
@@ -458,14 +543,15 @@ class Gen:
             e(f"A26_WRITE_DYN(0x100u | sp, 0x{ret >> 8:02X}u, cyc + 3u); sp = (sp - 1) & 0xFFu;")
             e(f"A26_WRITE_DYN(0x100u | sp, 0x{ret & 0xFF:02X}u, cyc + 4u); sp = (sp - 1) & 0xFFu;")
             e("A26_WRITE_DYN(0x100u | sp, p_, cyc + 5u); sp = (sp - 1) & 0xFFu;")
-            e(f"fid |= 4u; pc = 0x{vec:04X}u; cyc += 7u + stall_; goto a26_next_;")
+            e(f"fid |= 4u; pc = 0x{vec:04X}u; cyc += 7u + stall_; if (done) {{ A26_STAT(TRIP_FRAME_END); goto a26_next_; }}")
+            self.known_targets(pc, [vec], "TRIP_BRK_RTI")
             ends = True
         elif mn in ("PHA", "PHP"):
             val = "a" if mn == "PHA" else "(A26_PACK_P() | 0x30u)"
             e(f"uint32_t stall_ = 0; const uint32_t v_ = {val};")
             e("A26_WRITE_DYN(0x100u | sp, v_, cyc + 3u); sp = (sp - 1) & 0xFFu;")
             e("cyc += 3u + stall_;")
-            e(f"if (done) {{ pc = 0x{nxt:04X}u; goto a26_next_; }}")
+            e(f"if (done) {{ pc = 0x{nxt:04X}u; A26_STAT(TRIP_FRAME_END); goto a26_next_; }}")
         elif mn == "PLA":
             e("sp = (sp + 1) & 0xFFu; a = bus_read<VERIFY>(s, T, ram, 0x100u | sp, cyc + 4u, 0u, fb); nv = zv = a; cyc += 4u;")
         elif mn == "PLP":
@@ -503,6 +589,30 @@ class Gen:
             fnv = ((fnv ^ b) * 0x01000193) & 0xFFFFFFFF
         self.out.append(f"static const uint32_t kCompiledRomFnv1a = 0x{fnv:08X}u;   // FNV-1a of the 2 KiB image this file was generated from")
         self.out.append("#else")
+        head = self.out
+        # pass 1 without the straight RTS / RTI / JMP ind / BRK jumps finds the other direct jumps and the candidates; pass 2 emits the
+        # candidates that leave the direct jumps acyclic
+        self.allowed = set()
+        self.code(order, ids)
+        self.allowed = set(acyclic_extension(self.edges, self.candidates if self.straight_returns else []))
+        self.refused = sorted({c for c in self.candidates if c not in self.allowed}) if self.straight_returns else []
+        self.out = head + self.code(order, ids)
+        self.out.append("#endif")
+        os.makedirs(os.path.dirname(OUT_PATH), exist_ok=True)
+        hot = [a for a in HOT_ENTRIES if a in ids]
+        self.goto_targets.update(hot)
+        chain = " ".join(f"if (pc == 0x{a:04X}u) goto L_{a:04X};" for a in hot)
+        self.out.insert(2, f"#define A26_HOT_DISPATCH {chain}")
+        text = "\n".join(self.out) + "\n"
+        text = re.sub(r"@LABEL_([0-9A-F]{4})@", lambda m: f"L_{m.group(1)}:" if int(m.group(1), 16) in self.goto_targets else "", text)
+        with open(OUT_PATH, "w") as f:
+            f.write(text)
+        return len(order), len(leaders)
+
+    def code(self, order, ids):
+        """the case entries of the dispatcher switch; records the direct jumps in self.edges"""
+        self.out, self.goto_targets, self.edges, self.candidates = [], set(), [], []
+        self.cur_block = None
         prev_fell_through = False
         self.open_regions = []
         self.skip = set()
@@ -517,6 +627,9 @@ class Gen:
             if pc in ids:
                 if self.open_regions:
                     raise SystemExit(f"leader {pc:04X} inside a structured region")
+                if prev_fell_through:
+                    self.edges.append((self.cur_block, pc))
+                self.cur_block = pc
                 self.out.append(f"case {ids[pc]}: @LABEL_{pc:04X}@ /* ---- {pc:04X} ---- */")
                 if pc in SUPERBLOCKS:
                     lo, hi, want = SUPERBLOCKS[pc]
@@ -539,22 +652,14 @@ class Gen:
             prev_fell_through = not ends
         if self.open_regions:
             raise SystemExit("unterminated structured region")
-        self.out.append("#endif")
-        os.makedirs(os.path.dirname(OUT_PATH), exist_ok=True)
-        hot = [a for a in HOT_ENTRIES if a in ids]
-        self.goto_targets.update(hot)
-        chain = " ".join(f"if (pc == 0x{a:04X}u) goto L_{a:04X};" for a in hot)
-        self.out.insert(2, f"#define A26_HOT_DISPATCH {chain}")
-        text = "\n".join(self.out) + "\n"
-        text = re.sub(r"@LABEL_([0-9A-F]{4})@", lambda m: f"L_{m.group(1)}:" if int(m.group(1), 16) in self.goto_targets else "", text)
-        with open(OUT_PATH, "w") as f:
-            f.write(text)
-        return len(order), len(leaders)
+        return self.out
 
 
 if __name__ == "__main__":
-    if len(sys.argv) > 1:
-        OUT_PATH = sys.argv[1]
-    g = Gen(load_rom())
+    args = [a for a in sys.argv[1:] if a != "--no-straight-returns"]
+    if args:
+        OUT_PATH = args[0]
+    g = Gen(load_rom(), straight_returns="--no-straight-returns" not in sys.argv)
     n, l = g.generate()
-    print(f"wrote {os.path.relpath(OUT_PATH, ROOT)}: {n} instructions, {l} dispatch entries, {len(g.structured)} structured branches")
+    print(f"wrote {os.path.relpath(OUT_PATH, ROOT)}: {n} instructions, {l} dispatch entries, {len(g.structured)} structured branches, "
+          f"{len(g.allowed)} straight RTS / RTI / JMP ind / BRK targets ({len(g.refused)} refused: they would close a cycle)")
