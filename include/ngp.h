@@ -207,6 +207,51 @@ int ngp_record_matches(ngp_handle *h, const float *genomes, int32_t n_genomes,
                        uint64_t seed, uint64_t generation, int32_t max_record, ngp_frame_record *record,
                        double *rewards, int32_t *frames, int32_t *scores, uint64_t *frames_total, void *stream);
 
+/* ---- save states (ALE cloneState/restoreState, gym-retro env.em.get_state()/set_state()).
+ * One game state: the console (TIA, RIOT, paddles, CPU registers, RAM) and, when it was captured inside a match, the
+ * episode (perform_episode's locals, main.py:70-75: frame counter, timeout, total_frames, last scores, last ball and the
+ * decisions that drive the next env.step).  The contents are documented (DESIGN.md section 4, "save states") but opaque to
+ * callers: state arrays are device memory, 16-byte aligned, and the library only reads states that carry the magic and
+ * version of this format, the hash of the handle's cartridge image, players 1 or 2 and a matching checksum. */
+#define NGP_GAME_STATE_BYTES 512
+typedef struct { uint8_t b[NGP_GAME_STATE_BYTES]; } ngp_game_state;
+
+/* out: device ngp_game_state[n_envs] <- the stepwise environments as ngp_env_reset / ngp_env_step left them (no episode). */
+int ngp_env_get_state(ngp_handle *h, ngp_game_state *out, void *stream);
+/* The counterpart of ngp_env_reset: the n_envs stepwise environments become the consoles of `states` (device, any episode
+ * part is ignored).  The states' players value (gym-retro `players`: 1 for the cartridge robot game) must be the same for all.
+ * The states are validated on the device and the count of bad ones is read back (the call synchronises its stream once); on
+ * any bad state the call returns NGP_ERR_INVALID and the environments are left as they were. */
+int ngp_env_set_state(ngp_handle *h, const ngp_game_state *states, int32_t n_envs, void *stream);
+
+/* ---- ngp_record_matches whose matches may start from saved states and capture their own.
+ * genomes .. key, seed, generation and the outputs mean what they mean in ngp_record_matches.
+ * start: optional device i32[n_matches]; match m starts from states[start[m]] (device ngp_game_state[n_states]); -1 or
+ *   start == NULL = the built-in start state ngp_play_matches picks.  The plan (players, multiplier) comes from the lists.
+ * A state with an episode and fresh == 0 resumes that episode: frame counter (so frames[m] is the whole episode's length and
+ *   the fall-back draws, keyed by frame, continue), timeout, total_frames, last scores, last ball and the decisions taken on
+ *   the captured frame, which drive the first resumed env.step.  Resuming a capture with the same genomes, key, seed and
+ *   generation gives the uninterrupted game's reward, frames, scores and record entries.
+ * fresh != 0, or a state without an episode: a new perform_episode from that console (frame 0, no last score or ball,
+ *   BLANK_ACTION first), as retro.make(state=...) would; points already in RAM count.
+ * capture_at: optional device i32[n_matches] with capture device ngp_game_state[n_matches]: after capture_at[m] env.steps
+ *   counted from the episode's start (0 = before the first) the state of match m, console and episode, is written to
+ *   capture[m] -- only while the episode is still running, otherwise capture[m] is left untouched (frames[m] <= capture_at[m]).
+ * record: as in ngp_record_matches (entry t = env.step t from the episode's start, so a resumed match writes entries at or
+ *   after its start frame only), or NULL for none.  *frames_total counts the env.steps emulated in this call.
+ * Refusals (NGP_ERR_INVALID, nothing written, one synchronisation as in ngp_play_matches): those of ngp_record_matches (with
+ * a non-NULL record), start[m] outside [-1, n_states), a state that fails validation, a state whose players value disagrees
+ * with left[m] (players 1 with NGP_OPP_ROBOT only), capture_at[m] < 0, capture_at without capture, misaligned state arrays.
+ * Networks wider than 32 units return NGP_ERR_UNSUPPORTED.  With start, capture_at and record all NULL the results are
+ * ngp_play_matches' bits. */
+int ngp_play_matches_states(ngp_handle *h, const float *genomes, int32_t n_genomes,
+                            const int32_t *right, const int32_t *left, const double *mult, const int32_t *key, int32_t n_matches,
+                            const ngp_game_state *states, int32_t n_states, const int32_t *start, int32_t fresh,
+                            const int32_t *capture_at, ngp_game_state *capture,
+                            int32_t max_record, ngp_frame_record *record,
+                            uint64_t seed, uint64_t generation, double *rewards, int32_t *frames, int32_t *scores,
+                            uint64_t *frames_total, void *stream);
+
 /* ---- K4: GA step.  Replaces toolbox.select / varAnd(mate, mutate) inside eaSimple
  * (ga.py:89-94, main.py:165-170; DEAP selTournament, cxBlend, mutGaussian).
  * Injected noise (all device, all optional = NULL -> Philox(seed, generation)). */

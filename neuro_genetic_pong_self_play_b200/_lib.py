@@ -16,6 +16,8 @@ CORE_INTERPRETER, CORE_TRANSLATED = 0, 1
 OPP_HARDCODED, OPP_SCORE_HARDCODED, OPP_ROBOT = -1, -2, -3
 # sizeof(ngp_frame_record) (include/ngp.h): one recorded frame of ngp_record_matches
 NGP_FRAME_RECORD_BYTES = 32
+# sizeof(ngp_game_state) (include/ngp.h): one save state of a game
+NGP_GAME_STATE_BYTES = 512
 # button map codes (include/ngp.h NGP_BTN_*): fire of paddle p = BTN_FIRE_P0 + p; paddle p up / down = BTN_UP_P0 + 2p / + 2p + 1
 BTN_NONE, BTN_FIRE_P0, BTN_UP_P0, BTN_SELECT, BTN_RESET = 0, 1, 5, 13, 14
 
@@ -25,7 +27,7 @@ EXPORTS = [
     "ngp_evaluate_host", "ngp_ga_step", "ngp_init_population", "ngp_launch_count", "ngp_profile_enable", "ngp_profile_read",
     "ngp_config_size", "ngp_set_option", "ngp_select", "ngp_mate", "ngp_mutate", "ngp_hof_update", "ngp_exchange_bytes",
     "ngp_pack_elites", "ngp_unpack_elites", "ngp_mlp_prepare", "ngp_mlp_forward_prepared",
-    "ngp_play_matches", "ngp_record_matches",
+    "ngp_play_matches", "ngp_record_matches", "ngp_env_get_state", "ngp_env_set_state", "ngp_play_matches_states",
 ]
 
 
@@ -90,6 +92,10 @@ def load(build_if_missing: bool = True):
     L.ngp_evaluate.argtypes = [vp, vp, i32, vp, vp, i32, vp, u64, u64, vp, vp, vp, ctypes.POINTER(u64), vp]
     L.ngp_play_matches.argtypes = [vp, vp, i32, vp, vp, vp, i32, u64, u64, vp, vp, vp, ctypes.POINTER(u64), vp]
     L.ngp_record_matches.argtypes = [vp, vp, i32, vp, vp, vp, vp, i32, u64, u64, i32, vp, vp, vp, vp, ctypes.POINTER(u64), vp]
+    L.ngp_env_get_state.argtypes = [vp, vp, vp]
+    L.ngp_env_set_state.argtypes = [vp, vp, i32, vp]
+    L.ngp_play_matches_states.argtypes = [vp, vp, i32, vp, vp, vp, vp, i32, vp, i32, vp, i32, vp, vp, i32, vp, u64, u64, vp, vp, vp,
+                                          ctypes.POINTER(u64), vp]
     L.ngp_evaluate_host.argtypes = [vp, vp, i32, vp, vp, i32, u64, u64, vp, ctypes.POINTER(u64)]
     L.ngp_ga_step.argtypes = [vp, vp, vp, i32, u64, u64, ctypes.POINTER(NgpNoise), vp, vp, vp, vp, vp]
     L.ngp_init_population.argtypes = [vp, vp, i32, u64, vp]

@@ -183,17 +183,38 @@ __global__ void fitness_reduce_kernel(const double *__restrict__ rewards, int n,
     fitness[g] = __ddiv_rn(sum, (double)games);
 }
 
-// the argument check of ngp_play_matches / ngp_record_matches: counts the match entries that name no genome row (right),
-// neither a row nor an NGP_OPP_* code (left), or a negative fall-back key (key, may be null)
+// the argument check of the match-list entry points: counts the faults of every match entry (gs::match_entry_faults) and the
+// start states that fail validation
 __global__ void match_check_kernel(const int32_t *__restrict__ right, const int32_t *__restrict__ left, const int32_t *__restrict__ key,
-                                   int n, int n_genomes, unsigned long long *bad)
+                                   int n, int n_genomes, const int32_t *__restrict__ capture_at, const int32_t *__restrict__ start,
+                                   const ngp_game_state *__restrict__ states, int n_states, uint64_t cart, unsigned long long *bad)
 {
     unsigned long long c = 0;
-    for (int m = blockIdx.x * blockDim.x + threadIdx.x; m < n; m += gridDim.x * blockDim.x) {
-        const int r = right[m], l = left[m];
-        c += (r < 0 || r >= n_genomes) + (l < NGP_OPP_ROBOT || l >= n_genomes) + (key && key[m] < 0);
-    }
+    for (int m = blockIdx.x * blockDim.x + threadIdx.x; m < n; m += gridDim.x * blockDim.x)
+        c += gs::match_entry_faults(m, right, left, n_genomes, key, capture_at, start, states, n_states);
+    for (int k = blockIdx.x * blockDim.x + threadIdx.x; k < n_states; k += gridDim.x * blockDim.x) c += gs::validate(states + k, cart) == 0;
     if (c) atomicAdd(bad, c);
+}
+
+// stepwise save states: pack every environment (no episode) / count the bad states of a set and, in bad[1], take the players
+// value of the first / unpack them into the environments
+__global__ void env_get_state_kernel(Snapshot *envs, int n, int players, uint64_t cart, ngp_game_state *out)
+{
+    const int e = blockIdx.x * blockDim.x + threadIdx.x;
+    if (e < n) gs::pack(out + e, cart, players, envs[e].chip, envs[e].cpu, gs::SnapRam{envs[e].ram}, nullptr);
+}
+__global__ void state_check_kernel(const ngp_game_state *states, int n, uint64_t cart, unsigned long long *bad)
+{
+    const int e = blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= n) return;
+    const int players = gs::validate(states + e, cart), first = gs::validate(states, cart);
+    if (players == 0 || players != first) atomicAdd(bad, 1ull);
+    if (e == 0) bad[1] = (unsigned long long)players;
+}
+__global__ void env_set_state_kernel(const ngp_game_state *states, Snapshot *envs, int n)
+{
+    const int e = blockIdx.x * blockDim.x + threadIdx.x;
+    if (e < n) gs::unpack(states + e, envs[e].chip, envs[e].cpu, gs::SnapRam{envs[e].ram}, nullptr);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -255,6 +276,7 @@ extern "C" int ngp_create(const ngp_config *cfg, const uint8_t *rom, int32_t dev
     NGP_CUDA(cudaDeviceGetAttribute(&h->sm_count, cudaDevAttrMultiProcessorCount, device));
 
     h->rom_translated = a26::rom_matches_translation(rom) ? 1 : 0;
+    h->cart_hash = fnv1a64(rom, 2048);
     Tables tables;
     ngp_host::build_tables(tables, rom, cfg->ball_colour, cfg->left_colour, cfg->right_colour, ngp_ntsc_palette);
     std::vector<uint32_t> needed(a26::TRIGMAX + 1);
@@ -273,7 +295,7 @@ extern "C" int ngp_create(const ngp_config *cfg, const uint8_t *rom, int32_t dev
     // tens of milliseconds) and kept as an immutable host copy for later handles.
     {
         std::lock_guard<std::mutex> lock(g_start_mutex);
-        const uint64_t key = fnv1a64(rom, 2048);
+        const uint64_t key = h->cart_hash;
         auto it = g_start_cache.find(key);
         if (it == g_start_cache.end()) {
             build_start_states_kernel<<<2, 32>>>(h->d_tables.p, h->d_needed.p, h->d_start.p);
@@ -310,6 +332,45 @@ extern "C" int ngp_env_reset(ngp_handle *h, int32_t n_envs, int32_t state_id, vo
     h->n_envs = n_envs;
     h->env_players = state_id == NGP_STATE_START_1P ? 1 : 2;     // main.py:40 makes the robot game with players=1
     env_reset_kernel<<<(n_envs + 127) / 128, 128, 0, st>>>(h->d_start.p + state_id, h->d_envs.p, n_envs);
+    h->launches++;
+    NGP_CUDA(cudaGetLastError());
+    return NGP_OK;
+}
+
+extern "C" int ngp_env_get_state(ngp_handle *h, ngp_game_state *out, void *stream)
+{
+    NGP_REQUIRE(h && out, "ngp_env_get_state: bad arguments");
+    NGP_REQUIRE(h->n_envs > 0, "ngp_env_get_state: call ngp_env_reset or ngp_env_set_state first");
+    NGP_REQUIRE(((uintptr_t)out & 15) == 0, "ngp_env_get_state: the state array must be 16-byte aligned");
+    NGP_CUDA(cudaSetDevice(h->device));
+    env_get_state_kernel<<<(h->n_envs + 127) / 128, 128, 0, (cudaStream_t)stream>>>(h->d_envs.p, h->n_envs, h->env_players, h->cart_hash, out);
+    h->launches++;
+    NGP_CUDA(cudaGetLastError());
+    return NGP_OK;
+}
+
+extern "C" int ngp_env_set_state(ngp_handle *h, const ngp_game_state *states, int32_t n_envs, void *stream)
+{
+    NGP_REQUIRE(h && states && n_envs > 0, "ngp_env_set_state: bad arguments");
+    NGP_REQUIRE(((uintptr_t)states & 15) == 0, "ngp_env_set_state: the state array must be 16-byte aligned");
+    NGP_CUDA(cudaSetDevice(h->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    // validate before anything is resized or written: a refused call leaves the environments as they were
+    NGP_CUDA(cudaMemsetAsync(h->d_counters.p + 3, 0, 2 * sizeof(unsigned long long), st));
+    state_check_kernel<<<(n_envs + 127) / 128, 128, 0, st>>>(states, n_envs, h->cart_hash, h->d_counters.p + 3);
+    h->launches++;
+    NGP_CUDA(cudaGetLastError());
+    NGP_CUDA(cudaMemcpyAsync(h->h_counters.p + 3, h->d_counters.p + 3, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+    NGP_CUDA(cudaStreamSynchronize(st));
+    if (h->h_counters.p[3]) {
+        ngp_set_error("ngp_env_set_state: %llu states fail validation or have another players value than the first", h->h_counters.p[3]);
+        return NGP_ERR_INVALID;
+    }
+    NGP_CUDA(h->d_envs.ensure(n_envs));
+    NGP_CUDA(h->d_fb.ensure((size_t)n_envs * a26::FB_ROWS * a26::FB_COLS));
+    h->n_envs = n_envs;
+    h->env_players = (int)h->h_counters.p[4];
+    env_set_state_kernel<<<(n_envs + 127) / 128, 128, 0, st>>>(states, h->d_envs.p, n_envs);
     h->launches++;
     NGP_CUDA(cudaGetLastError());
     return NGP_OK;
@@ -518,11 +579,12 @@ extern "C" int ngp_evaluate(ngp_handle *h, const float *genomes, int32_t n, cons
     return frames_total ? read_rollout_counters(h, st, frames_total, "ngp_evaluate") : NGP_OK;
 }
 
-// ngp_play_matches, and ngp_record_matches when `rec` is set (its record pointer and length already checked)
+// ngp_play_matches; ngp_record_matches and ngp_play_matches_states when `rec` is set (its pointers' alignment and the record
+// length already checked; n_states = the length of rec->states)
 static int play_match_list(ngp_handle *h, const float *genomes, int32_t n_genomes, const int32_t *right, const int32_t *left,
-                           const double *mult, const int32_t *key, int32_t n_matches, uint64_t seed, uint64_t generation,
-                           double *rewards, int32_t *frames, int32_t *scores, uint64_t *frames_total, cudaStream_t st,
-                           const roll::RecordArgs *rec, const char *who)
+                           const double *mult, int32_t n_matches, uint64_t seed, uint64_t generation, double *rewards, int32_t *frames,
+                           int32_t *scores, uint64_t *frames_total, cudaStream_t st, const roll::RecordArgs *rec, int32_t n_states,
+                           const char *who)
 {
     if (!(h && genomes && right && left && rewards && n_genomes > 0 && n_matches > 0)) {
         ngp_set_error("%s: bad arguments", who);
@@ -539,20 +601,28 @@ static int play_match_list(ngp_handle *h, const float *genomes, int32_t n_genome
         ngp_set_error("%s: the statically translated core was generated from a different cartridge; use NGP_CORE_INTERPRETER", who);
         return NGP_ERR_UNSUPPORTED;
     }
+    const roll::RecordArgs none = {};
+    const roll::RecordArgs &ra = rec ? *rec : none;
     NGP_CUDA(cudaSetDevice(h->device));
     if (!frames) NGP_CUDA(h->d_frames.ensure(n_matches));
     NGP_CUDA(cudaMemsetAsync(h->d_counters.p, 0, 8 * sizeof(unsigned long long), st));
-    // the lists live on the device: count their bad entries there and refuse before anything is played
-    const int check_blocks = (int)std::min<long long>(((long long)n_matches + 255) / 256, 4ll * h->sm_count);
-    match_check_kernel<<<check_blocks, 256, 0, st>>>(right, left, key, n_matches, n_genomes, h->d_counters.p + 3);
+    // the lists and states live on the device: count their bad entries there and refuse before anything is played
+    const long long check_items = std::max<long long>(n_matches, n_states);
+    const int check_blocks = (int)std::min<long long>((check_items + 255) / 256, 4ll * h->sm_count);
+    match_check_kernel<<<check_blocks, 256, 0, st>>>(right, left, ra.key, n_matches, n_genomes, ra.capture_at, ra.start, ra.states, n_states,
+                                                     h->cart_hash, h->d_counters.p + 3);
     h->launches++;
     NGP_CUDA(cudaGetLastError());
     NGP_CUDA(cudaMemcpyAsync(h->h_counters.p + 3, h->d_counters.p + 3, sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
     NGP_CUDA(cudaStreamSynchronize(st));
     if (h->h_counters.p[3]) {
-        ngp_set_error(key ? "%s: %llu match entries name no genome row (right), no genome row or NGP_OPP_* code (left) or a negative key"
-                          : "%s: %llu match entries name no genome row (right) or no genome row or NGP_OPP_* code (left)",
-                      who, h->h_counters.p[3]);
+        if (ra.start || ra.capture_at || n_states)
+            ngp_set_error("%s: %llu faults in the match entries (genome rows, NGP_OPP_* codes, keys, start indices, capture frames, "
+                          "players of the start states) or start states that fail validation", who, h->h_counters.p[3]);
+        else
+            ngp_set_error(ra.key ? "%s: %llu match entries name no genome row (right), no genome row or NGP_OPP_* code (left) or a negative key"
+                                 : "%s: %llu match entries name no genome row (right) or no genome row or NGP_OPP_* code (left)",
+                          who, h->h_counters.p[3]);
         return NGP_ERR_INVALID;
     }
     RolloutParams p = rollout_params(h, genomes, seed, generation);
@@ -568,8 +638,8 @@ extern "C" int ngp_play_matches(ngp_handle *h, const float *genomes, int32_t n_g
                                 const double *mult, int32_t n_matches, uint64_t seed, uint64_t generation, double *rewards,
                                 int32_t *frames, int32_t *scores, uint64_t *frames_total, void *stream)
 {
-    return play_match_list(h, genomes, n_genomes, right, left, mult, nullptr, n_matches, seed, generation, rewards, frames, scores,
-                           frames_total, (cudaStream_t)stream, nullptr, "ngp_play_matches");
+    return play_match_list(h, genomes, n_genomes, right, left, mult, n_matches, seed, generation, rewards, frames, scores,
+                           frames_total, (cudaStream_t)stream, nullptr, 0, "ngp_play_matches");
 }
 
 extern "C" int ngp_record_matches(ngp_handle *h, const float *genomes, int32_t n_genomes, const int32_t *right, const int32_t *left,
@@ -579,10 +649,31 @@ extern "C" int ngp_record_matches(ngp_handle *h, const float *genomes, int32_t n
 {
     NGP_REQUIRE(max_record >= 1 && record, "ngp_record_matches: needs a record buffer and max_record >= 1");
     NGP_REQUIRE(((uintptr_t)record & 15) == 0, "ngp_record_matches: the record buffer must be 16-byte aligned");
-    roll::RecordArgs rec;
+    roll::RecordArgs rec = {};
     rec.record = record; rec.key = key; rec.max_record = max_record;
-    return play_match_list(h, genomes, n_genomes, right, left, mult, key, n_matches, seed, generation, rewards, frames, scores,
-                           frames_total, (cudaStream_t)stream, &rec, "ngp_record_matches");
+    return play_match_list(h, genomes, n_genomes, right, left, mult, n_matches, seed, generation, rewards, frames, scores,
+                           frames_total, (cudaStream_t)stream, &rec, 0, "ngp_record_matches");
+}
+
+extern "C" int ngp_play_matches_states(ngp_handle *h, const float *genomes, int32_t n_genomes, const int32_t *right, const int32_t *left,
+                                       const double *mult, const int32_t *key, int32_t n_matches, const ngp_game_state *states,
+                                       int32_t n_states, const int32_t *start, int32_t fresh, const int32_t *capture_at,
+                                       ngp_game_state *capture, int32_t max_record, ngp_frame_record *record, uint64_t seed,
+                                       uint64_t generation, double *rewards, int32_t *frames, int32_t *scores, uint64_t *frames_total,
+                                       void *stream)
+{
+    NGP_REQUIRE(h, "ngp_play_matches_states: null handle");
+    NGP_REQUIRE(!record || max_record >= 1, "ngp_play_matches_states: a record needs max_record >= 1");
+    NGP_REQUIRE(((uintptr_t)record & 15) == 0, "ngp_play_matches_states: the record buffer must be 16-byte aligned");
+    NGP_REQUIRE(n_states >= 0 && (n_states == 0 || states), "ngp_play_matches_states: n_states states needed");
+    NGP_REQUIRE(((uintptr_t)states & 15) == 0 && ((uintptr_t)capture & 15) == 0, "ngp_play_matches_states: state arrays must be 16-byte aligned");
+    NGP_REQUIRE(!capture_at || capture, "ngp_play_matches_states: capture_at needs a capture buffer");
+    roll::RecordArgs rec = {};
+    rec.record = record; rec.key = key; rec.max_record = record ? max_record : 0;
+    rec.fresh = fresh ? 1 : 0; rec.states = states; rec.start = start; rec.capture_at = capture_at; rec.capture = capture;
+    rec.cart = h->cart_hash;
+    return play_match_list(h, genomes, n_genomes, right, left, mult, n_matches, seed, generation, rewards, frames, scores,
+                           frames_total, (cudaStream_t)stream, &rec, n_states, "ngp_play_matches_states");
 }
 
 extern "C" int ngp_profile_enable(ngp_handle *h, int32_t on)

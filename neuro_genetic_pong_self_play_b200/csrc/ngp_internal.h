@@ -51,6 +51,7 @@ struct ngp_handle {
     int gene_size;
     pol::Shape shape;
     int rom_translated;           // the ROM is the cartridge the statically translated core was generated from
+    uint64_t cart_hash;           // fnv1a64 of the cartridge image: the header of every ngp_game_state of this handle
     // device tables
     Buffer<a26::Tables> d_tables;         // rom + decode + colour-match weights
     Buffer<uint32_t> d_needed;            // paddle charge -> cycles table [4097]

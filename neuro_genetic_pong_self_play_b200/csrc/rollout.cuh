@@ -95,12 +95,19 @@ struct RolloutParams {
     int32_t *scores;                // [n][2] (score1, score2) at the end of the episode, or null
 };
 
-// ngp_record_matches: a separate kernel argument that only the recording twins of rollout_kernel read, so the flavours
-// ngp_evaluate and ngp_play_matches run compile as before
+// ngp_record_matches and ngp_play_matches_states: a separate kernel argument that only the recording twins of rollout_kernel
+// read, so the flavours ngp_evaluate and ngp_play_matches run compile as before
 struct RecordArgs {
-    ngp_frame_record *record;       // [n][max_record], 16-byte aligned
+    ngp_frame_record *record;       // [n][max_record], 16-byte aligned, or null (ngp_play_matches_states without a record)
     const int32_t *key;             // [n] environment index of the fall-back key, or null (= match index)
     int max_record;
+    // ngp_play_matches_states (all null otherwise)
+    int fresh;                      // states start new episodes from their consoles
+    const ngp_game_state *states;   // start states
+    const int32_t *start;           // [n] index into states, -1 = the built-in start state
+    const int32_t *capture_at;      // [n] env.steps after which the state of match e is written to capture[e]
+    ngp_game_state *capture;        // [n]
+    uint64_t cart;                  // the cartridge hash written into captured states
 };
 
 // Half `half` (16 bytes) of record entry (env, frame): one vector store on the device.

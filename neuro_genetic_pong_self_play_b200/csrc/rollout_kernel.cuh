@@ -2,7 +2,7 @@
 // ngp_play_matches run; ngp_record.cu instantiates their recording twins (REC = true, ngp_record_matches) in a translation
 // unit of their own, so the parallel build compiles both sets side by side.
 #pragma once
-#include "rollout.cuh"
+#include "game_state.cuh"
 
 __device__ __forceinline__ void load_tables(a26::Tables &dst, const a26::Tables *__restrict__ src)
 {
@@ -15,8 +15,9 @@ __device__ __forceinline__ void load_tables(a26::Tables &dst, const a26::Tables 
 // Fused rollout: one environment (= one game of one genome) per thread.  Lanes are persistent and
 // pull the next environment from a global counter at frame boundaries, so a warp stays in
 // scanline lock-step whatever episode each of its lanes is in.
-// `rec` is read by the REC twins only (ngp_record_matches): they store every frame below rec.max_record with
-// roll::record_frame and key the fall-back actions by rec.key.
+// `rec` is read by the REC twins only (ngp_record_matches, ngp_play_matches_states): they store every frame below
+// rec.max_record with roll::record_frame when there is a record, key the fall-back actions by rec.key, start matches from
+// rec.states with roll::resume_state and write rec.capture with roll::capture_state.
 template <int CORE, bool SYNC, int MAXT, bool REC = false>
 __global__ void __launch_bounds__(MAXT, 1) rollout_kernel(roll::RolloutParams p, roll::RecordArgs rec)
 {
@@ -31,11 +32,18 @@ __global__ void __launch_bounds__(MAXT, 1) rollout_kernel(roll::RolloutParams p,
     ep.env = -1;
     bool exhausted = false;
     unsigned long long my_frames = 0;
+    int capture_at = -1;                // REC: capture the episode after this many env.steps
     for (;;) {
         if (ep.env < 0 && !exhausted) {
             int e = (int)atomicAdd(&p.counters[0], 1ull);
-            if (e < total) roll::episode_begin(ep, p, e, s, r, ram);
-            else exhausted = true;
+            if (e < total) {
+                roll::episode_begin(ep, p, e, s, r, ram);
+                if (REC && rec.start && rec.start[e] >= 0) roll::resume_state(rec, rec.start[e], ep, s, r, ram);
+                if (REC && rec.capture_at) {
+                    capture_at = rec.capture_at[e];
+                    if (capture_at == ep.frame) roll::capture_state(rec, ep, s, r, ram);
+                }
+            } else exhausted = true;
         }
         const bool active = ep.env >= 0;
         // SYNC: the CTA walks through frames together (CTA-wide barriers inside the frame), so it also stops together
@@ -45,7 +53,8 @@ __global__ void __launch_bounds__(MAXT, 1) rollout_kernel(roll::RolloutParams p,
             double reward;
             const bool done = roll::episode_frame<CORE, SYNC, REC>(ep, p, s, r, T, ram, &reward, active, &rec);
             if (active) my_frames++;
-            if (REC && active && ep.frame <= rec.max_record) roll::record_frame(rec, ep, s, ep.last_s1, ep.last_s2);
+            if (REC && active && rec.record && ep.frame <= rec.max_record) roll::record_frame(rec, ep, s, ep.last_s1, ep.last_s2);
+            if (REC && active && !done && ep.frame == capture_at) roll::capture_state(rec, ep, s, r, ram);
             if (done) {
                 p.rewards[ep.env] = reward;
                 p.frames[ep.env] = ep.frame;

@@ -113,6 +113,22 @@ class Engine:
                                              _p(out["valid"]), _p(out["regs"]), _stream(self.device)), "ngp_env_step")
         return out
 
+    def env_get_state(self) -> torch.Tensor:
+        """Save states of the stepwise environments as env_reset / env_step / env_set_state left them (gym-retro
+        env.em.get_state()): u8[n_envs, NGP_GAME_STATE_BYTES], without an episode."""
+        out = torch.empty((self._n_envs, _lib.NGP_GAME_STATE_BYTES), dtype=torch.uint8, device=self.device)
+        _lib.check(self._L.ngp_env_get_state(self._h, _p(out), _stream(self.device)), "ngp_env_get_state")
+        return out
+
+    def env_set_state(self, states: torch.Tensor):
+        """The counterpart of env_reset (gym-retro env.em.set_state()): the stepwise environments become the consoles of
+        `states` u8[n, NGP_GAME_STATE_BYTES] (one players value for all; any episode part is ignored).  A state that fails
+        validation raises NgpError and leaves the environments as they were."""
+        self._check_tensor(states, torch.uint8, "states")
+        assert states.dim() == 2 and states.shape[1] == _lib.NGP_GAME_STATE_BYTES
+        _lib.check(self._L.ngp_env_set_state(self._h, _p(states), states.shape[0], _stream(self.device)), "ngp_env_set_state")
+        self._n_envs = states.shape[0]
+
     def env_digest(self) -> torch.Tensor:
         d = torch.empty((self._n_envs, 8), dtype=torch.int32, device=self.device)
         _lib.check(self._L.ngp_env_digest(self._h, _p(d), _stream(self.device)), "ngp_env_digest")
@@ -235,6 +251,51 @@ class Engine:
                                               ctypes.byref(total) if sync else None, _stream(self.device)), "ngp_record_matches")
         return {"rewards": rewards, "frames": frames, "scores": scores, "frames_total": int(total.value) if sync else None,
                 "left": left, "record": record_views(raw)}
+
+    def play_matches_states(self, genomes: torch.Tensor, right: torch.Tensor, left: torch.Tensor, mult: torch.Tensor | None = None,
+                            key: torch.Tensor | None = None, states: torch.Tensor | None = None, start: torch.Tensor | None = None,
+                            fresh: bool = False, capture_at: torch.Tensor | None = None, max_record: int = 0, seed: int = 0,
+                            generation: int = 0, sync: bool = True):
+        """record_matches whose matches may start from save states and capture their own (ngp_play_matches_states).
+        states: u8[S, NGP_GAME_STATE_BYTES]; start[m] (None = all -1) picks match m's start state, -1 = the built-in one.  A
+        state with an episode resumes it unless `fresh`; a fresh start plays a new episode from the state's console.
+        capture_at[m]: after that many env.steps from the episode's start the state of match m is captured (left as zeros
+        when the game ended before).  max_record > 0 records every frame as record_matches does.  Returns play_matches'
+        dict plus `left`, plus `capture` u8[M, NGP_GAME_STATE_BYTES] when capture_at is given and `record` views when
+        max_record > 0.  Bad entries or states raise NgpError and nothing is played."""
+        self._check_tensor(genomes, torch.float32, "genomes")
+        self._check_tensor(right, torch.int32, "right")
+        self._check_tensor(left, torch.int32, "left")
+        assert genomes.dim() == 2 and genomes.shape[1] == self.gene_size
+        m = right.shape[0]
+        assert right.dim() == 1 and tuple(left.shape) == (m,)
+        for t, name, dtype in ((mult, "mult", torch.float64), (key, "key", torch.int32), (start, "start", torch.int32),
+                               (capture_at, "capture_at", torch.int32)):
+            if t is not None:
+                self._check_tensor(t, dtype, name)
+                assert tuple(t.shape) == (m,), name
+        n_states = 0
+        if states is not None:
+            self._check_tensor(states, torch.uint8, "states")
+            assert states.dim() == 2 and states.shape[1] == _lib.NGP_GAME_STATE_BYTES
+            n_states = states.shape[0]
+        capture = torch.zeros((m, _lib.NGP_GAME_STATE_BYTES), dtype=torch.uint8, device=self.device) if capture_at is not None else None
+        raw = (torch.empty((m, int(max_record), _lib.NGP_FRAME_RECORD_BYTES), dtype=torch.uint8, device=self.device)
+               if max_record > 0 else None)
+        rewards = torch.empty(m, dtype=torch.float64, device=self.device)
+        frames = torch.empty(m, dtype=torch.int32, device=self.device)
+        scores = torch.empty((m, 2), dtype=torch.int32, device=self.device)
+        total = ctypes.c_uint64(0)
+        _lib.check(self._L.ngp_play_matches_states(
+            self._h, _p(genomes), genomes.shape[0], _p(right), _p(left), _p(mult), _p(key), m, _p(states) if n_states else None,
+            n_states, _p(start), 1 if fresh else 0, _p(capture_at), _p(capture), int(max_record), _p(raw), seed, generation,
+            _p(rewards), _p(frames), _p(scores), ctypes.byref(total) if sync else None, _stream(self.device)), "ngp_play_matches_states")
+        out = {"rewards": rewards, "frames": frames, "scores": scores, "frames_total": int(total.value) if sync else None, "left": left}
+        if capture is not None:
+            out["capture"] = capture
+        if raw is not None:
+            out["record"] = record_views(raw)
+        return out
 
     def evaluate_host(self, genomes: np.ndarray, hof_genomes: np.ndarray | None = None, hof_fitness: np.ndarray | None = None,
                       seed: int = 0, generation: int = 0):

@@ -359,14 +359,20 @@ def replay(toolbox: Toolbox, individual, game: int = 0, upsample=(4, 4), max_fra
     return {"frames": torch.stack(frames), "reward": reward, "steps": steps, "score": (s1, s2)}
 
 
-def render_recorded(toolbox: Toolbox, rec: dict, matches, upsample=(1, 1), core: int | None = None, want_ram: bool = False):
+def render_recorded(toolbox: Toolbox, rec: dict, matches, upsample=(1, 1), core: int | None = None, want_ram: bool = False,
+                    start_states=None):
     """Re-renders recorded games (Engine.record_matches' result) pixel for pixel: the emulator is deterministic, so the
     recorded decisions are all it needs.  Each match m in `matches` is played again through env_reset + env_step (verify
     mode, every pixel), one batch per start state ('Start' with players = 1 for ROBOT matches, 'Start.2P' for the rest):
     step 0 gets BLANK_ACTION, step t gets BLANK_ACTION with record t-1's decisions written to [4:6] (right) and [6:8] (left),
     as perform_episode does (main.py:91-92).  Returns one u8[T_m, 210*k, 160*l, 3] device tensor per match, T_m =
     min(frames[m], max_record); with want_ram, (frames, ram u8[T_m, 128]) pairs.  core: the 6507 core of env_step (None =
-    the toolbox config's CORE).  Resets the engine's stepwise environments (env_reset)."""
+    the toolbox config's CORE).  Resets the engine's stepwise environments (env_reset).
+    start_states = (states, t): renders matches that were resumed from save states (Engine.play_matches_states) from there:
+    states u8[M, NGP_GAME_STATE_BYTES] holds the state match m started from in row m, captured after t[m] env.steps (t an
+    int or a sequence per match); the environments start with env_set_state and step t[m] gets record t[m]-1's decisions, so
+    that entry must hold the captured frame's (branch() copies the entries below t from the original game).  Frames
+    t[m]..T_m-1 are returned."""
     eng, cfg = toolbox.engine, toolbox.config
     dev = eng.device
     core = cfg.CORE if core is None else int(core)
@@ -375,24 +381,35 @@ def render_recorded(toolbox: Toolbox, rec: dict, matches, upsample=(1, 1), core:
     left = rec["left"].cpu().tolist()
     act = rec["record"]["act"]
     T_max = act.shape[1]
+    if start_states is None:
+        starts = [0] * len(frames_n)
+    else:
+        states, t = start_states
+        starts = [int(t)] * len(frames_n) if np.ndim(t) == 0 else [int(v) for v in t]
     out = {}
     blank = torch.tensor(cfg.blank_action(), dtype=torch.uint8, device=dev)
     for state in (_lib.STATE_START_1P, _lib.STATE_START_2P):
         group = [m for m in dict.fromkeys(matches) if (left[m] == _lib.OPP_ROBOT) == (state == _lib.STATE_START_1P)]
         if not group:
             continue
-        lens = [min(frames_n[m], T_max) for m in group]
+        lens = [max(min(frames_n[m], T_max) - starts[m], 0) for m in group]
         T = max(lens)
-        a = act[torch.tensor(group, device=dev)][:, :T].long()                       # [n, T]: decisions of frame t
-        actions = blank.repeat(T, len(group), 1)                                      # [T, n, 16]: input of env.step t
-        ra, la = (a[:, : T - 1] >> 2).t(), (a[:, : T - 1] & 3).t()
-        actions[1:, :, cfg.RIGHT_ACTION_START] = (ra == _lib.ACT_UP).to(torch.uint8)
-        actions[1:, :, cfg.RIGHT_ACTION_START + 1] = (ra == _lib.ACT_DOWN).to(torch.uint8)
-        actions[1:, :, cfg.RIGHT_ACTION_END] = (la == _lib.ACT_UP).to(torch.uint8)
-        actions[1:, :, cfg.RIGHT_ACTION_END + 1] = (la == _lib.ACT_DOWN).to(torch.uint8)
+        # env.step k0[i] + j of match i gets the decisions of record entry k0[i] + j - 1 (BLANK_ACTION alone for step 0)
+        k = torch.tensor([starts[m] for m in group], device=dev)[:, None] + torch.arange(T, device=dev)[None, :]      # [n, T]
+        a = act[torch.tensor(group, device=dev)[:, None], (k - 1).clamp(0, T_max - 1)].long()
+        first = k == 0
+        ra, la = torch.where(first, _lib.ACT_NONE, a >> 2).t(), torch.where(first, _lib.ACT_NONE, a & 3).t()
+        actions = blank.repeat(T, len(group), 1)                                      # [T, n, 16]: input of env.step k
+        actions[:, :, cfg.RIGHT_ACTION_START] = (ra == _lib.ACT_UP).to(torch.uint8)
+        actions[:, :, cfg.RIGHT_ACTION_START + 1] = (ra == _lib.ACT_DOWN).to(torch.uint8)
+        actions[:, :, cfg.RIGHT_ACTION_END] = (la == _lib.ACT_UP).to(torch.uint8)
+        actions[:, :, cfg.RIGHT_ACTION_END + 1] = (la == _lib.ACT_DOWN).to(torch.uint8)
         pix = [torch.empty((n, 210, 160, 3), dtype=torch.uint8, device=dev) for n in lens]
         ram = [torch.empty((n, 128), dtype=torch.uint8, device=dev) for n in lens]
-        eng.env_reset(len(group), state)
+        if start_states is None:
+            eng.env_reset(len(group), state)
+        else:
+            eng.env_set_state(states[torch.tensor(group, device=dev)].contiguous())
         for t in range(T):
             step = eng.env_step(actions[t].contiguous(), want_frames=True, want_obs=False, core=core)
             for i, n in enumerate(lens):
@@ -402,6 +419,42 @@ def render_recorded(toolbox: Toolbox, rec: dict, matches, upsample=(1, 1), core:
         for i, m in enumerate(group):
             out[m] = (repeat_upsample(pix[i], *upsample), ram[i])
     return [out[m] if want_ram else out[m][0] for m in matches]
+
+
+def branch(toolbox: Toolbox, genomes: torch.Tensor, right, left, m: int, t: int, new_right: int | None = None,
+           new_left: int | None = None, key: int | None = None, mult=None, max_record: int | None = None):
+    """A counterfactual branch of list match m (right[m] vs left[m], a genome row or OPP_* code; lists as play_matches takes
+    them): the game is played to env.step t and captured there (Engine.play_matches_states), then continued from that exact
+    position with new_right / new_left (None = the same players; a robot match stays a robot match) under the same fall-back
+    key (key = None: m, the match's index in the list) and the toolbox's seed and generation.  The first resumed env.step
+    still uses the decisions the old players took on frame t.  Returns record_matches' dict for the one branched match:
+    rewards, frames, scores (the whole episode's), frames_total (the frames emulated after t), left, record (entries below
+    t are the original game's) -- plus `capture`, the state at t, and `start_states` = (capture, t) for render_recorded.
+    Raises ValueError when the game ended before env.step t."""
+    eng, cfg = toolbox.engine, toolbox.config
+    dev = eng.device
+    genomes = genomes.to(dev, torch.float32).contiguous()
+    right = [int(v) for v in (right.tolist() if torch.is_tensor(right) else right)]
+    left = [int(v) for v in (left.tolist() if torch.is_tensor(left) else left)]
+    mult_m = 1.0 if mult is None else float(mult[m])
+
+    def one(v, dtype=torch.int32):
+        return torch.tensor([v], dtype=dtype, device=dev)
+
+    bound = max_record or (cfg.MAX_FRAMES if cfg.MAX_FRAMES > 0 else 2 * cfg.WIN_SCORE * (cfg.TIMEOUT_THRESH + 2))
+    k = one(m if key is None else int(key))
+    common = dict(key=k, max_record=bound, seed=toolbox.seed, generation=toolbox.generation)
+    orig = eng.play_matches_states(genomes, one(right[m]), one(left[m]), one(mult_m, torch.float64), capture_at=one(int(t)), **common)
+    if int(orig["frames"].item()) <= t:
+        raise ValueError(f"match {m} ended after {int(orig['frames'].item())} env.steps, before env.step {t}")
+    nr = right[m] if new_right is None else int(new_right)
+    nl = left[m] if new_left is None else int(new_left)
+    out = eng.play_matches_states(genomes, one(nr), one(nl), one(mult_m, torch.float64), states=orig["capture"], start=one(0),
+                                  **common)
+    out["record"]["raw"][:, :t] = orig["record"]["raw"][:, :t]
+    out["capture"] = orig["capture"]
+    out["start_states"] = (orig["capture"], int(t))
+    return out
 
 
 def replay_selfplay(toolbox: Toolbox, genomes: torch.Tensor, g: int, k: int, upsample=(4, 4)):
