@@ -96,6 +96,10 @@ struct ngp_handle {
     }
 };
 
+// The wide MLP layer kernels take the genome from grid.y or grid.z, which CUDA caps at 65 535: ngp_mlp_forward and
+// ngp_mlp_prepare run larger genome sets in slices of at most this many genomes.
+constexpr int MLP_GENOME_SLICE = 65535;
+
 void ngp_set_error(const char *fmt, ...);
 #define NGP_CUDA(expr)                                                                           \
     do {                                                                                         \

@@ -403,10 +403,13 @@ extern "C" int ngp_mlp_prepare(ngp_handle *h, const float *genomes, int32_t n_ge
     for (int l = 0; l < L; ++l) {
         const int ni = sh.nodes[l], no = sh.nodes[l + 1];
         if (layer_is_packed(sh, l)) {
-            dim3 grid(128, n_genomes);
-            tmm::mlp_pack_layer_kernel<<<grid, 256, 0, st>>>(genomes, w_off, h->gene_size, ni, no, bias, h->prep_packed.p, per_genome, layer_off);
-            h->launches++;
-            NGP_CUDA(cudaGetLastError());
+            for (int g0 = 0; g0 < n_genomes; g0 += MLP_GENOME_SLICE) {
+                dim3 grid(128, n_genomes - g0 < MLP_GENOME_SLICE ? n_genomes - g0 : MLP_GENOME_SLICE);
+                tmm::mlp_pack_layer_kernel<<<grid, 256, 0, st>>>(genomes + (size_t)g0 * h->gene_size, w_off, h->gene_size, ni, no, bias,
+                                                                 h->prep_packed.p + (size_t)g0 * per_genome, per_genome, layer_off);
+                h->launches++;
+                NGP_CUDA(cudaGetLastError());
+            }
             layer_off += tmm::packed_floats(ni, no);
         }
         w_off += (size_t)(ni + bias) * no;
@@ -415,8 +418,9 @@ extern "C" int ngp_mlp_prepare(ngp_handle *h, const float *genomes, int32_t n_ge
     return NGP_OK;
 }
 
-// one prepared wide hidden layer (called by ngp_mlp_forward_prepared); NGP_ERR_UNSUPPORTED -> the caller uses the unprepared path
-int ngp_mlp_layer_tmem(ngp_handle *h, int l, const float *in, int n_genomes, int envs, float *out, cudaStream_t st)
+// one prepared wide hidden layer (called by ngp_mlp_forward_prepared) for the prepared genomes [g0, g0 + n_genomes);
+// NGP_ERR_UNSUPPORTED -> the caller uses the unprepared path
+int ngp_mlp_layer_tmem(ngp_handle *h, int l, size_t g0, const float *in, int n_genomes, int envs, float *out, cudaStream_t st)
 {
     const pol::Shape &sh = h->shape;
     if (!layer_is_packed(sh, l) || envs < 16 || !h->prep_packed.p) return NGP_ERR_UNSUPPORTED;
@@ -424,6 +428,7 @@ int ngp_mlp_layer_tmem(ngp_handle *h, int l, const float *in, int n_genomes, int
     for (int i = 0; i < l; ++i)
         if (layer_is_packed(sh, i)) layer_off += tmm::packed_floats(sh.nodes[i], sh.nodes[i + 1]);
     const int ni = sh.nodes[l], no = sh.nodes[l + 1];
+    const float *packed = h->prep_packed.p + g0 * h->prep_per_genome;
     if (!h->tmem_attr_set) {
         NGP_CUDA(cudaFuncSetAttribute(tmm::mlp_layer_tmem_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tmm::smem_bytes(64)));
         NGP_CUDA(cudaFuncSetAttribute(tmm::mlp_layer_tmem_kernel<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tmm::smem_bytes(128)));
@@ -431,10 +436,10 @@ int ngp_mlp_layer_tmem(ngp_handle *h, int l, const float *in, int n_genomes, int
     }
     if (envs > 64) {
         dim3 grid((no + tmm::TM - 1) / tmm::TM, (envs + 127) / 128, n_genomes);
-        tmm::mlp_layer_tmem_kernel<128><<<grid, tmm::threads(128), tmm::smem_bytes(128), st>>>(h->prep_packed.p, h->prep_per_genome, layer_off, in, envs, ni, no, out);
+        tmm::mlp_layer_tmem_kernel<128><<<grid, tmm::threads(128), tmm::smem_bytes(128), st>>>(packed, h->prep_per_genome, layer_off, in, envs, ni, no, out);
     } else {
         dim3 grid((no + tmm::TM - 1) / tmm::TM, 1, n_genomes);
-        tmm::mlp_layer_tmem_kernel<64><<<grid, tmm::threads(64), tmm::smem_bytes(64), st>>>(h->prep_packed.p, h->prep_per_genome, layer_off, in, envs, ni, no, out);
+        tmm::mlp_layer_tmem_kernel<64><<<grid, tmm::threads(64), tmm::smem_bytes(64), st>>>(packed, h->prep_per_genome, layer_off, in, envs, ni, no, out);
     }
     h->launches++;
     NGP_CUDA(cudaGetLastError());

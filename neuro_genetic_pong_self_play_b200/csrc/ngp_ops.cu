@@ -465,10 +465,12 @@ __global__ void mlp_decide_kernel(const double *__restrict__ z, long long rows, 
 int ngp_mlp_layer_tf32(ngp_handle *h, const float *genomes, size_t w_off, const float *in, int n_genomes, int envs, int ni, int no, int bias,
                        float *out, cudaStream_t st);   // ngp_mlp_tf32.cu
 
-int ngp_mlp_layer_tmem(ngp_handle *h, int l, const float *in, int n_genomes, int envs, float *out, cudaStream_t st);    // ngp_mlp_tmem.cu
+int ngp_mlp_layer_tmem(ngp_handle *h, int l, size_t g0, const float *in, int n_genomes, int envs, float *out, cudaStream_t st);  // ngp_mlp_tmem.cu
 
 static int mlp_forward_impl(ngp_handle *h, const float *genomes, const float *x, int32_t n_genomes, int32_t envs, uint8_t *act, float *out,
                             void *stream, bool prepared);
+static int mlp_forward_slice(ngp_handle *h, const float *genomes, const float *x, size_t g0, int n_genomes, int envs, uint8_t *act,
+                             float *out, cudaStream_t st, bool prepared);
 
 extern "C" int ngp_mlp_forward(ngp_handle *h, const float *genomes, const float *x, int32_t n_genomes, int32_t envs, uint8_t *act,
                                float *out, void *stream)
@@ -500,9 +502,28 @@ static int mlp_forward_impl(ngp_handle *h, const float *genomes, const float *x,
         NGP_CUDA(cudaGetLastError());
         return NGP_OK;
     }
-    NGP_CUDA(h->mlp_a.ensure((size_t)rows * widest));
-    NGP_CUDA(h->mlp_b.ensure((size_t)rows * widest));
-    NGP_CUDA(h->mlp_z.ensure((size_t)rows * sh.nodes[sh.n_layers - 1]));
+    const int n_in = sh.nodes[0], n_out = sh.nodes[sh.n_layers - 1];
+    const size_t slice_rows = (size_t)(n_genomes < MLP_GENOME_SLICE ? n_genomes : MLP_GENOME_SLICE) * envs;
+    NGP_CUDA(h->mlp_a.ensure(slice_rows * widest));
+    NGP_CUDA(h->mlp_b.ensure(slice_rows * widest));
+    NGP_CUDA(h->mlp_z.ensure(slice_rows * n_out));
+    for (int g0 = 0; g0 < n_genomes; g0 += MLP_GENOME_SLICE) {
+        const int gn = n_genomes - g0 < MLP_GENOME_SLICE ? n_genomes - g0 : MLP_GENOME_SLICE;
+        const size_t r0 = (size_t)g0 * envs;
+        const int rc = mlp_forward_slice(h, genomes + (size_t)g0 * h->gene_size, x + r0 * n_in, g0, gn, envs, act + r0,
+                                         out ? out + r0 * n_out : nullptr, st, prepared);
+        if (rc != NGP_OK) return rc;
+    }
+    return NGP_OK;
+}
+
+// the layers of the wide path for genomes [g0, g0 + n_genomes) of the call (pointers already offset to g0; g0 locates the
+// genomes in the prepared packed copy)
+static int mlp_forward_slice(ngp_handle *h, const float *genomes, const float *x, size_t g0, int n_genomes, int envs, uint8_t *act,
+                             float *out, cudaStream_t st, bool prepared)
+{
+    const pol::Shape &sh = h->shape;
+    const long long rows = (long long)n_genomes * envs;
     const float *in = x;
     float *bufs[2] = {h->mlp_a.p, h->mlp_b.p};
     size_t w_off = 0;
@@ -536,7 +557,7 @@ static int mlp_forward_impl(ngp_handle *h, const float *genomes, const float *x,
         }
         if (!launched && prepared && l != L - 1 && !h->opt_mlp_no_tf32) {
             // prepared genome set: weights stream from HBM straight into tensor memory (ngp_mlp_tmem.cu)
-            const int rc = ngp_mlp_layer_tmem(h, l, in, n_genomes, envs, bufs[l & 1], st);
+            const int rc = ngp_mlp_layer_tmem(h, l, g0, in, n_genomes, envs, bufs[l & 1], st);
             if (rc == NGP_OK) launched = true;
             else if (rc != NGP_ERR_UNSUPPORTED) return rc;
         }

@@ -53,7 +53,7 @@ double eo_det_exp(double x)
 /* ------------------------------------------------------ numpy_nn.py:35-69, 120-137 ---- */
 void eo_mlp_forward(const eo_shape *sh, const float *genome, const double *x, double *out, int *action)
 {
-    double buf_a[1024], buf_b[1024];
+    double buf_a[4097], buf_b[4097];                  /* layers up to 4096 units plus the bias input */
     double *cur = buf_a, *nxt = buf_b;
     int n_in = sh->nodes[0];
     int bias = sh->bias ? 1 : 0;
