@@ -34,21 +34,6 @@ void ngp_set_error(const char *fmt, ...)
 extern "C" const char *ngp_last_error(void) { return g_err; }
 extern "C" const char *ngp_version(void) { return "ngp 0.1 (sm_100a)"; }
 
-// Stella NTSC palette [3P-recall]; entries $0E,$22,$38,$C8 are pinned by config.py:3-6 + obs.npy
-const uint32_t ngp_ntsc_palette[128] = {
-    0x000000, 0x4a4a4a, 0x6f6f6f, 0x8e8e8e, 0xaaaaaa, 0xc0c0c0, 0xd6d6d6, 0xececec, 0x484800, 0x69690f, 0x86861d, 0xa2a22a,
-    0xbbbb35, 0xd2d240, 0xe8e84a, 0xfcfc54, 0x7c2c00, 0x904811, 0xa26221, 0xb47a30, 0xc3903d, 0xd2a44a, 0xdfb755, 0xecc860,
-    0x901c00, 0xa33915, 0xb55328, 0xc66c3a, 0xd5824a, 0xe39759, 0xf0aa67, 0xfcbc74, 0x940000, 0xa71a1a, 0xb83232, 0xc84848,
-    0xd65c5c, 0xe46f6f, 0xf08080, 0xfc9090, 0x840064, 0x97197a, 0xa8308f, 0xb846a2, 0xc659b3, 0xd46cc3, 0xe07cd2, 0xec8ce0,
-    0x500084, 0x68199a, 0x7d30ad, 0x9246c0, 0xa459d0, 0xb56ce0, 0xc57cee, 0xd48cfc, 0x140090, 0x331aa3, 0x4e32b5, 0x6848c6,
-    0x7f5cd5, 0x956fe3, 0xa980f0, 0xbc90fc, 0x000094, 0x181aa7, 0x2d32b8, 0x4248c8, 0x545cd6, 0x656fe4, 0x7580f0, 0x8490fc,
-    0x001c88, 0x183b9d, 0x2d57b0, 0x4272c2, 0x548ad2, 0x65a0e1, 0x75b5ef, 0x84c8fc, 0x003064, 0x185080, 0x2d6d98, 0x4288b0,
-    0x54a0c5, 0x65b7d9, 0x75cceb, 0x84e0fc, 0x004030, 0x18624e, 0x2d8169, 0x429e82, 0x54b899, 0x65d1ae, 0x75e7c2, 0x84fcd4,
-    0x004400, 0x1a661a, 0x328432, 0x48a048, 0x5cba5c, 0x6fd26f, 0x80e880, 0x90fc90, 0x143c00, 0x355f18, 0x527e2d, 0x6e9c42,
-    0x87b754, 0x9ed065, 0xb4e775, 0xc8fc84, 0x303800, 0x505916, 0x6d762b, 0x88923e, 0xa0ab4f, 0xb7c25f, 0xccd86e, 0xe0ec7c,
-    0x482c00, 0x694d14, 0x866a26, 0xa28638, 0xbb9f47, 0xd2b656, 0xe8cc63, 0xfce070,
-};
-
 extern "C" void ngp_default_config(ngp_config *cfg, int32_t population)
 {
     memset(cfg, 0, sizeof(*cfg));
@@ -67,13 +52,7 @@ extern "C" void ngp_default_config(ngp_config *cfg, int32_t population)
     cfg->cxpb = 0.9f; cfg->cx_alpha = 0.9f; cfg->mutpb = 0.9f; cfg->mut_mu = 0.0f; cfg->mut_sigma = 0.9f; cfg->mut_indpb = 0.9f;
     cfg->tournament_size = population / 4;
     cfg->core = NGP_CORE_TRANSLATED;
-    // button map: the reference's own naming (config.py:15-20, main.py:91-92) -- see include/ngp.h
-    cfg->button_map[0] = NGP_BTN_FIRE_P0 + 1;      // RIGHT_PLAYER_START_BUTTON = 0
-    cfg->button_map[15] = NGP_BTN_FIRE_P0 + 0;     // LEFT_PLAYER_START_BUTTON = -1
-    cfg->button_map[4] = NGP_BTN_UP_P0 + 2; cfg->button_map[5] = NGP_BTN_UP_P0 + 3;      // action[4:6]: right player = paddle 1
-    cfg->button_map[6] = NGP_BTN_UP_P0 + 0; cfg->button_map[7] = NGP_BTN_UP_P0 + 1;      // action[6:8]: left player = paddle 0
-    cfg->button_map[2] = cfg->button_map[10] = NGP_BTN_SELECT;
-    cfg->button_map[3] = cfg->button_map[11] = NGP_BTN_RESET;
+    ngp_host::default_button_map(cfg->button_map);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -220,13 +199,6 @@ __global__ void env_set_state_kernel(const ngp_game_state *states, Snapshot *env
 // ------------------------------------------------------------------------------------------------
 // host API
 // ------------------------------------------------------------------------------------------------
-static int gene_size_of(const ngp_config &c)
-{
-    int total = 0;
-    for (int i = 0; i + 1 < c.n_layers; ++i) total += (c.nodes[i] + (c.bias ? 1 : 0)) * c.nodes[i + 1];
-    return total;
-}
-
 extern "C" int32_t ngp_gene_size(const ngp_handle *h) { return h ? h->gene_size : 0; }
 extern "C" uint64_t ngp_launch_count(const ngp_handle *h) { return h ? h->launches : 0; }
 
@@ -269,16 +241,16 @@ extern "C" int ngp_create(const ngp_config *cfg, const uint8_t *rom, int32_t dev
     auto h = std::make_unique<ngp_handle>();     // freed with everything it holds on an early return
     h->cfg = *cfg;
     h->device = device;
-    h->gene_size = gene_size_of(*cfg);
     h->shape.n_layers = cfg->n_layers;
     for (int i = 0; i < 8; ++i) h->shape.nodes[i] = cfg->nodes[i];
     h->shape.bias = cfg->bias;
+    h->gene_size = pol::gene_size(h->shape);
     NGP_CUDA(cudaDeviceGetAttribute(&h->sm_count, cudaDevAttrMultiProcessorCount, device));
 
     h->rom_translated = a26::rom_matches_translation(rom) ? 1 : 0;
     h->cart_hash = fnv1a64(rom, 2048);
     Tables tables;
-    ngp_host::build_tables(tables, rom, cfg->ball_colour, cfg->left_colour, cfg->right_colour, ngp_ntsc_palette);
+    ngp_host::build_tables(tables, rom, cfg->ball_colour, cfg->left_colour, cfg->right_colour, ngp_host::ntsc_palette);
     std::vector<uint32_t> needed(a26::TRIGMAX + 1);
     ngp_host::build_paddle_table(needed.data());
     NGP_CUDA(h->d_tables.ensure(1));
@@ -286,7 +258,7 @@ extern "C" int ngp_create(const ngp_config *cfg, const uint8_t *rom, int32_t dev
     NGP_CUDA(h->d_needed.ensure(needed.size()));
     NGP_CUDA(cudaMemcpy(h->d_needed.p, needed.data(), needed.size() * 4, cudaMemcpyHostToDevice));
     NGP_CUDA(h->d_palette.ensure(128));
-    NGP_CUDA(cudaMemcpy(h->d_palette.p, ngp_ntsc_palette, sizeof(ngp_ntsc_palette), cudaMemcpyHostToDevice));
+    NGP_CUDA(cudaMemcpy(h->d_palette.p, ngp_host::ntsc_palette, sizeof(ngp_host::ntsc_palette), cudaMemcpyHostToDevice));
     NGP_CUDA(h->d_start.ensure(2));
     NGP_CUDA(h->d_counters.ensure(8));
     NGP_CUDA(cudaMemset(h->d_counters.p, 0, 8 * sizeof(unsigned long long)));
@@ -439,15 +411,7 @@ static RolloutParams rollout_params(const ngp_handle *h, const float *genomes, u
     p.win_score = h->cfg.win_score; p.timeout_thresh = h->cfg.timeout_thresh; p.max_frames = h->cfg.max_frames;
     p.time_scaler = (double)h->cfg.time_scaler; p.paddle_height = (double)h->cfg.scaled_paddle_height;
     p.seed = seed; p.generation = generation; p.shape = h->shape;
-    for (int players = 1; players <= 2; ++players)
-        for (int la = 0; la < 3; ++la)
-            for (int ra = 0; ra < 3; ++ra) {
-                uint8_t a[16] = {0};
-                a[0] = 1; a[15] = 1;                                          // BLANK_ACTION, config.py:21-23
-                a[4] = ra == pol::ACT_UP; a[5] = ra == pol::ACT_DOWN;         // action[4:6] = right (main.py:91)
-                a[6] = la == pol::ACT_UP; a[7] = la == pol::ACT_DOWN;         // action[6:8] = left (main.py:92)
-                p.input_table[players - 1][la * 3 + ra] = roll::action_to_input(a, players, h->cfg.button_map);
-            }
+    roll::fill_input_table(p, h->cfg.button_map);
     p.counters = h->d_counters.p;
     return p;
 }

@@ -114,5 +114,3 @@ void ngp_set_error(const char *fmt, ...);
     do {                                                            \
         if (!(cond)) { ngp_set_error("%s", msg); return NGP_ERR_INVALID; } \
     } while (0)
-
-extern const uint32_t ngp_ntsc_palette[128];

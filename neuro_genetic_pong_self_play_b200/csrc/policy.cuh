@@ -20,6 +20,14 @@ struct Shape {
     int bias;
 };
 
+// genes of one network: a (nodes[l] + bias) x nodes[l + 1] weight matrix per layer, in reference gene order
+inline int gene_size(const Shape &sh)
+{
+    int total = 0;
+    for (int i = 0; i + 1 < sh.n_layers; ++i) total += (sh.nodes[i] + (sh.bias ? 1 : 0)) * sh.nodes[i + 1];
+    return total;
+}
+
 #ifdef __CUDACC__
 
 __device__ __forceinline__ void philox4x32(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3, uint32_t k0, uint32_t k1, uint32_t out[4])

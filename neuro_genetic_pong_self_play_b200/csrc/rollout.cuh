@@ -95,6 +95,20 @@ struct RolloutParams {
     int32_t *scores;                // [n][2] (score1, score2) at the end of the episode, or null
 };
 
+// p.input_table through the button map `map` (ngp_config.button_map)
+__host__ inline void fill_input_table(RolloutParams &p, const uint8_t map[16])
+{
+    for (int players = 1; players <= 2; ++players)
+        for (int la = 0; la < 3; ++la)
+            for (int ra = 0; ra < 3; ++ra) {
+                uint8_t a[16] = {0};
+                a[0] = 1; a[15] = 1;                                          // BLANK_ACTION, config.py:21-23
+                a[4] = ra == pol::ACT_UP; a[5] = ra == pol::ACT_DOWN;         // action[4:6] = right (main.py:91)
+                a[6] = la == pol::ACT_UP; a[7] = la == pol::ACT_DOWN;         // action[6:8] = left (main.py:92)
+                p.input_table[players - 1][la * 3 + ra] = action_to_input(a, players, map);
+            }
+}
+
 // ngp_record_matches and ngp_play_matches_states: a separate kernel argument that only the recording twins of rollout_kernel
 // read, so the flavours ngp_evaluate and ngp_play_matches run compile as before
 struct RecordArgs {

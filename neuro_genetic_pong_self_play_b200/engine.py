@@ -196,6 +196,23 @@ class Engine:
                                         ctypes.byref(total) if sync else None, _stream(self.device)), "ngp_evaluate")
         return {"fitness": fitness, "rewards": rewards, "frames": frames, "frames_total": int(total.value) if sync else None}
 
+    def _match_list(self, genomes, right, left, **per_match):
+        """The argument check and the outputs the match-list methods share: genomes f32[N, gene_size], right and left i32[M],
+        and per_match name=(tensor or None, dtype) of shape [M].  Returns dict(rewards f64[M], frames i32[M], scores i32[M, 2])."""
+        self._check_tensor(genomes, torch.float32, "genomes")
+        self._check_tensor(right, torch.int32, "right")
+        self._check_tensor(left, torch.int32, "left")
+        assert genomes.dim() == 2 and genomes.shape[1] == self.gene_size
+        m = right.shape[0]
+        assert right.dim() == 1 and tuple(left.shape) == (m,)
+        for name, (t, dtype) in per_match.items():
+            if t is not None:
+                self._check_tensor(t, dtype, name)
+                assert tuple(t.shape) == (m,), name
+        return {"rewards": torch.empty(m, dtype=torch.float64, device=self.device),
+                "frames": torch.empty(m, dtype=torch.int32, device=self.device),
+                "scores": torch.empty((m, 2), dtype=torch.int32, device=self.device)}
+
     def play_matches(self, genomes: torch.Tensor, right: torch.Tensor, left: torch.Tensor, mult: torch.Tensor | None = None,
                      seed: int = 0, generation: int = 0, sync: bool = True):
         """An explicit match list in one fused launch (ngp_play_matches): match m puts genome row right[m] on the right against
@@ -203,23 +220,13 @@ class Engine:
         player's score bonus (None = 1.0).  Returns dict(rewards f64[M] of the right player, frames i32[M], scores i32[M, 2]
         = (left, right) points, frames_total).  The lists are checked on the device; a bad entry raises NgpError and nothing
         is played."""
-        self._check_tensor(genomes, torch.float32, "genomes")
-        self._check_tensor(right, torch.int32, "right")
-        self._check_tensor(left, torch.int32, "left")
-        assert genomes.dim() == 2 and genomes.shape[1] == self.gene_size
-        m = right.shape[0]
-        assert right.dim() == 1 and tuple(left.shape) == (m,)
-        if mult is not None:
-            self._check_tensor(mult, torch.float64, "mult")
-            assert tuple(mult.shape) == (m,)
-        rewards = torch.empty(m, dtype=torch.float64, device=self.device)
-        frames = torch.empty(m, dtype=torch.int32, device=self.device)
-        scores = torch.empty((m, 2), dtype=torch.int32, device=self.device)
+        out = self._match_list(genomes, right, left, mult=(mult, torch.float64))
         total = ctypes.c_uint64(0)
-        _lib.check(self._L.ngp_play_matches(self._h, _p(genomes), genomes.shape[0], _p(right), _p(left), _p(mult), m, seed, generation,
-                                            _p(rewards), _p(frames), _p(scores), ctypes.byref(total) if sync else None,
-                                            _stream(self.device)), "ngp_play_matches")
-        return {"rewards": rewards, "frames": frames, "scores": scores, "frames_total": int(total.value) if sync else None}
+        _lib.check(self._L.ngp_play_matches(self._h, _p(genomes), genomes.shape[0], _p(right), _p(left), _p(mult), right.shape[0], seed,
+                                            generation, _p(out["rewards"]), _p(out["frames"]), _p(out["scores"]),
+                                            ctypes.byref(total) if sync else None, _stream(self.device)), "ngp_play_matches")
+        out["frames_total"] = int(total.value) if sync else None
+        return out
 
     def record_matches(self, genomes: torch.Tensor, right: torch.Tensor, left: torch.Tensor, mult: torch.Tensor | None = None,
                        key: torch.Tensor | None = None, max_record: int = 2048, seed: int = 0, generation: int = 0, sync: bool = True):
@@ -229,28 +236,16 @@ class Engine:
         for rendering) and `record`: named views over one u8[M, T, 32] buffer (T = max_record; frame t of match m is valid
         for t < min(frames[m], T)): loc f32[M, T, 3, 2], valid u8[M, T] (bit 0 ball, 1 left, 2 right), score u8[M, T, 2],
         act u8[M, T] (left | right << 2, after the bounds clamp) and timeout i32[M, T]."""
-        self._check_tensor(genomes, torch.float32, "genomes")
-        self._check_tensor(right, torch.int32, "right")
-        self._check_tensor(left, torch.int32, "left")
-        assert genomes.dim() == 2 and genomes.shape[1] == self.gene_size
+        out = self._match_list(genomes, right, left, mult=(mult, torch.float64), key=(key, torch.int32))
         m = right.shape[0]
-        assert right.dim() == 1 and tuple(left.shape) == (m,)
-        if mult is not None:
-            self._check_tensor(mult, torch.float64, "mult")
-            assert tuple(mult.shape) == (m,)
-        if key is not None:
-            self._check_tensor(key, torch.int32, "key")
-            assert tuple(key.shape) == (m,)
         raw = torch.empty((m, max(int(max_record), 0), _lib.NGP_FRAME_RECORD_BYTES), dtype=torch.uint8, device=self.device)
-        rewards = torch.empty(m, dtype=torch.float64, device=self.device)
-        frames = torch.empty(m, dtype=torch.int32, device=self.device)
-        scores = torch.empty((m, 2), dtype=torch.int32, device=self.device)
         total = ctypes.c_uint64(0)
         _lib.check(self._L.ngp_record_matches(self._h, _p(genomes), genomes.shape[0], _p(right), _p(left), _p(mult), _p(key), m, seed,
-                                              generation, int(max_record), _p(raw), _p(rewards), _p(frames), _p(scores),
-                                              ctypes.byref(total) if sync else None, _stream(self.device)), "ngp_record_matches")
-        return {"rewards": rewards, "frames": frames, "scores": scores, "frames_total": int(total.value) if sync else None,
-                "left": left, "record": record_views(raw)}
+                                              generation, int(max_record), _p(raw), _p(out["rewards"]), _p(out["frames"]),
+                                              _p(out["scores"]), ctypes.byref(total) if sync else None, _stream(self.device)),
+                   "ngp_record_matches")
+        out.update(frames_total=int(total.value) if sync else None, left=left, record=record_views(raw))
+        return out
 
     def play_matches_states(self, genomes: torch.Tensor, right: torch.Tensor, left: torch.Tensor, mult: torch.Tensor | None = None,
                             key: torch.Tensor | None = None, states: torch.Tensor | None = None, start: torch.Tensor | None = None,
@@ -263,17 +258,9 @@ class Engine:
         when the game ended before).  max_record > 0 records every frame as record_matches does.  Returns play_matches'
         dict plus `left`, plus `capture` u8[M, NGP_GAME_STATE_BYTES] when capture_at is given and `record` views when
         max_record > 0.  Bad entries or states raise NgpError and nothing is played."""
-        self._check_tensor(genomes, torch.float32, "genomes")
-        self._check_tensor(right, torch.int32, "right")
-        self._check_tensor(left, torch.int32, "left")
-        assert genomes.dim() == 2 and genomes.shape[1] == self.gene_size
+        out = self._match_list(genomes, right, left, mult=(mult, torch.float64), key=(key, torch.int32), start=(start, torch.int32),
+                               capture_at=(capture_at, torch.int32))
         m = right.shape[0]
-        assert right.dim() == 1 and tuple(left.shape) == (m,)
-        for t, name, dtype in ((mult, "mult", torch.float64), (key, "key", torch.int32), (start, "start", torch.int32),
-                               (capture_at, "capture_at", torch.int32)):
-            if t is not None:
-                self._check_tensor(t, dtype, name)
-                assert tuple(t.shape) == (m,), name
         n_states = 0
         if states is not None:
             self._check_tensor(states, torch.uint8, "states")
@@ -282,15 +269,13 @@ class Engine:
         capture = torch.zeros((m, _lib.NGP_GAME_STATE_BYTES), dtype=torch.uint8, device=self.device) if capture_at is not None else None
         raw = (torch.empty((m, int(max_record), _lib.NGP_FRAME_RECORD_BYTES), dtype=torch.uint8, device=self.device)
                if max_record > 0 else None)
-        rewards = torch.empty(m, dtype=torch.float64, device=self.device)
-        frames = torch.empty(m, dtype=torch.int32, device=self.device)
-        scores = torch.empty((m, 2), dtype=torch.int32, device=self.device)
         total = ctypes.c_uint64(0)
         _lib.check(self._L.ngp_play_matches_states(
             self._h, _p(genomes), genomes.shape[0], _p(right), _p(left), _p(mult), _p(key), m, _p(states) if n_states else None,
             n_states, _p(start), 1 if fresh else 0, _p(capture_at), _p(capture), int(max_record), _p(raw), seed, generation,
-            _p(rewards), _p(frames), _p(scores), ctypes.byref(total) if sync else None, _stream(self.device)), "ngp_play_matches_states")
-        out = {"rewards": rewards, "frames": frames, "scores": scores, "frames_total": int(total.value) if sync else None, "left": left}
+            _p(out["rewards"]), _p(out["frames"]), _p(out["scores"]), ctypes.byref(total) if sync else None, _stream(self.device)),
+            "ngp_play_matches_states")
+        out.update(frames_total=int(total.value) if sync else None, left=left)
         if capture is not None:
             out["capture"] = capture
         if raw is not None:

@@ -41,28 +41,10 @@ static inline int __all_sync(unsigned, int v) { return v; }
 static inline unsigned __ballot_sync(unsigned, int v) { return v ? 1u : 0u; }
 static inline int __syncthreads_or(int v) { return v; }
 
-#include "../../neuro_genetic_pong_self_play_b200/csrc/rollout.cuh"
+#include "../../neuro_genetic_pong_self_play_b200/csrc/game_state.cuh"
 #include "../../neuro_genetic_pong_self_play_b200/csrc/host_tables.h"
 
 namespace {
-// ngp_default_config's button map (csrc/ngp_core.cu)
-const uint8_t kDefaultButtonMap[16] = {NGP_BTN_FIRE_P0 + 1, 0, NGP_BTN_SELECT, NGP_BTN_RESET, NGP_BTN_UP_P0 + 2, NGP_BTN_UP_P0 + 3,
-                                       NGP_BTN_UP_P0 + 0, NGP_BTN_UP_P0 + 1, 0, 0, NGP_BTN_SELECT, NGP_BTN_RESET, 0, 0, 0, NGP_BTN_FIRE_P0 + 0};
-// same palette the product uploads (csrc/ngp_core.cu: ngp_ntsc_palette)
-const uint32_t kPalette[128] = {
-    0x000000, 0x4a4a4a, 0x6f6f6f, 0x8e8e8e, 0xaaaaaa, 0xc0c0c0, 0xd6d6d6, 0xececec, 0x484800, 0x69690f, 0x86861d, 0xa2a22a,
-    0xbbbb35, 0xd2d240, 0xe8e84a, 0xfcfc54, 0x7c2c00, 0x904811, 0xa26221, 0xb47a30, 0xc3903d, 0xd2a44a, 0xdfb755, 0xecc860,
-    0x901c00, 0xa33915, 0xb55328, 0xc66c3a, 0xd5824a, 0xe39759, 0xf0aa67, 0xfcbc74, 0x940000, 0xa71a1a, 0xb83232, 0xc84848,
-    0xd65c5c, 0xe46f6f, 0xf08080, 0xfc9090, 0x840064, 0x97197a, 0xa8308f, 0xb846a2, 0xc659b3, 0xd46cc3, 0xe07cd2, 0xec8ce0,
-    0x500084, 0x68199a, 0x7d30ad, 0x9246c0, 0xa459d0, 0xb56ce0, 0xc57cee, 0xd48cfc, 0x140090, 0x331aa3, 0x4e32b5, 0x6848c6,
-    0x7f5cd5, 0x956fe3, 0xa980f0, 0xbc90fc, 0x000094, 0x181aa7, 0x2d32b8, 0x4248c8, 0x545cd6, 0x656fe4, 0x7580f0, 0x8490fc,
-    0x001c88, 0x183b9d, 0x2d57b0, 0x4272c2, 0x548ad2, 0x65a0e1, 0x75b5ef, 0x84c8fc, 0x003064, 0x185080, 0x2d6d98, 0x4288b0,
-    0x54a0c5, 0x65b7d9, 0x75cceb, 0x84e0fc, 0x004030, 0x18624e, 0x2d8169, 0x429e82, 0x54b899, 0x65d1ae, 0x75e7c2, 0x84fcd4,
-    0x004400, 0x1a661a, 0x328432, 0x48a048, 0x5cba5c, 0x6fd26f, 0x80e880, 0x90fc90, 0x143c00, 0x355f18, 0x527e2d, 0x6e9c42,
-    0x87b754, 0x9ed065, 0xb4e775, 0xc8fc84, 0x303800, 0x505916, 0x6d762b, 0x88923e, 0xa0ab4f, 0xb7c25f, 0xccd86e, 0xe0ec7c,
-    0x482c00, 0x694d14, 0x866a26, 0xa28638, 0xbb9f47, 0xd2b656, 0xe8cc63, 0xfce070,
-};
-
 struct Sim {
     a26::Tables T;
     std::vector<uint32_t> needed;
@@ -72,16 +54,19 @@ struct Sim {
     a26::CpuRegs r;
     uint32_t ram_words[32 * 32];   // lane 0 of a warp-interleaved block
     int players = 2;               // the robot game ('Start') is made with players=1 (main.py:40)
+    uint8_t button_map[16];        // ngp_default_config's
 };
 }  // namespace
 
 extern "C" {
 
-void *hs_create(const uint8_t *rom)
+// a simulator whose find_stuff looks for other target colours (ngp_config.ball_colour / left_colour / right_colour): a colour
+// that matches nothing hides that object from the observation, e.g. to force get_actions' random fall-back
+void *hs_create_colours(const uint8_t *rom, const uint8_t *ball, const uint8_t *left, const uint8_t *right)
 {
     Sim *sim = new Sim();
-    const uint8_t ball[3] = {236, 236, 236}, left[3] = {213, 130, 74}, right[3] = {92, 186, 92};
-    ngp_host::build_tables(sim->T, rom, ball, left, right, kPalette);
+    ngp_host::build_tables(sim->T, rom, ball, left, right, ngp_host::ntsc_palette);
+    ngp_host::default_button_map(sim->button_map);
     sim->needed.resize(a26::TRIGMAX + 1);
     ngp_host::build_paddle_table(sim->needed.data());
     a26::Ram ram{sim->ram_words};
@@ -90,6 +75,11 @@ void *hs_create(const uint8_t *rom)
         roll::store_snapshot(&sim->start[st], sim->s, sim->r, ram);
     }
     return sim;
+}
+void *hs_create(const uint8_t *rom)
+{
+    const uint8_t ball[3] = {236, 236, 236}, left[3] = {213, 130, 74}, right[3] = {92, 186, 92};     // ngp_default_config's
+    return hs_create_colours(rom, ball, left, right);
 }
 void hs_destroy(void *h) { delete (Sim *)h; }
 
@@ -149,7 +139,7 @@ int hs_env_step_fast(void *h, int core, const uint8_t *action16, uint8_t *ram_ou
     Sim *sim = (Sim *)h;
     a26::Ram ram{sim->ram_words};
     a26::Chip &s = sim->s;
-    const uint32_t in = roll::action_to_input(action16, sim->players, kDefaultButtonMap);
+    const uint32_t in = roll::action_to_input(action16, sim->players, sim->button_map);
     a26::apply_input(s, sim->needed.data(), in & 0xFF, (in >> 8) & 15, (in >> 12) & 15, (in >> 16) & 15);
     a26::clear_obs(s);
     if (core) a26::run_frame_compiled<false, false>(s, sim->r, sim->T, ram, nullptr);
@@ -165,47 +155,108 @@ int hs_env_step_fast(void *h, int core, const uint8_t *action16, uint8_t *ram_ou
 
 int hs_env_step(void *h, int core, const uint8_t *action16, uint8_t *ram_out, uint8_t *fb, double *loc, uint8_t *valid, uint8_t *regs, uint32_t *digest)
 {
-    const uint32_t in = roll::action_to_input(action16, ((Sim *)h)->players, kDefaultButtonMap);
+    const Sim *sim = (Sim *)h;
+    const uint32_t in = roll::action_to_input(action16, sim->players, sim->button_map);
     return hs_env_run_frame(h, core, in & 0xFF, (int)((in >> 8) & 15), (int)((in >> 12) & 15), (int)((in >> 16) & 15), ram_out, fb, loc, valid, regs, digest);
 }
 
-// fused evaluation, lanes executed one after another
+}  // extern "C"
+
+// RolloutParams as rollout_params (csrc/ngp_core.cu) fills them for ngp_default_config with this network, core and max_frames;
+// the caller adds the population or the match list and the outputs
+static roll::RolloutParams rollout_params(Sim *sim, int core, const int32_t *nodes, int n_layers, int bias, int max_frames, uint64_t seed,
+                                          uint64_t generation)
+{
+    roll::RolloutParams p = {};
+    p.tables = &sim->T; p.needed = sim->needed.data(); p.start = sim->start;
+    p.win_score = 3; p.timeout_thresh = 2000; p.max_frames = max_frames;
+    p.core = core; p.time_scaler = 100.0; p.paddle_height = 16.0; p.seed = seed; p.generation = generation;
+    p.shape.n_layers = n_layers; p.shape.bias = bias;
+    for (int i = 0; i < n_layers; ++i) p.shape.nodes[i] = nodes[i];
+    p.G = pol::gene_size(p.shape);
+    roll::fill_input_table(p, sim->button_map);
+    return p;
+}
+
+// One lane of rollout_kernel (csrc/rollout_kernel.cuh) from the start to the end of environment e's episode, in the kernel's
+// order: episode_begin; with REC the start state and the capture at frame 0; every frame episode_frame, then with REC
+// record_frame and the capture after that frame; at the end reward, frame count and scores as the kernel stores them.
+// Returns the frames played.
+template <int CORE, bool REC>
+static uint64_t play_lane(Sim *sim, const roll::RolloutParams &p, const roll::RecordArgs &rec, int e)
+{
+    a26::Ram ram{sim->ram_words};
+    a26::Chip s; a26::CpuRegs r;
+    roll::Episode ep;
+    roll::episode_begin(ep, p, e, s, r, ram);
+    if (REC && rec.start && rec.start[e] >= 0) roll::resume_state(rec, rec.start[e], ep, s, r, ram);
+    const int capture_at = REC && rec.capture_at ? rec.capture_at[e] : -1;
+    if (capture_at == ep.frame) roll::capture_state(rec, ep, s, r, ram);
+    uint64_t frames = 0;
+    double reward;
+    for (bool done = false; !done; ++frames) {
+        done = roll::episode_frame<CORE, false, REC>(ep, p, s, r, sim->T, ram, &reward, true, &rec);
+        if (REC && rec.record && ep.frame <= rec.max_record) roll::record_frame(rec, ep, s, ep.last_s1, ep.last_s2);
+        if (REC && !done && ep.frame == capture_at) roll::capture_state(rec, ep, s, r, ram);
+    }
+    p.rewards[e] = reward;
+    p.frames[e] = ep.frame;
+    if (p.scores) { p.scores[2 * e] = ep.last_s1; p.scores[2 * e + 1] = ep.last_s2; }
+    return frames;
+}
+
+// every environment of p, lanes executed one after another; returns the frames played
+template <bool REC>
+static uint64_t play_lanes(Sim *sim, const roll::RolloutParams &p, const roll::RecordArgs &rec)
+{
+    uint64_t frames = 0;
+    for (int e = 0; e < p.n * p.games; ++e) frames += p.core ? play_lane<1, REC>(sim, p, rec, e) : play_lane<0, REC>(sim, p, rec, e);
+    return frames;
+}
+
+extern "C" {
+
+// fused evaluation (ngp_evaluate)
 void hs_evaluate(void *h, int core, const int32_t *nodes, int n_layers, int bias, int schedule, int games, int max_frames, const float *genomes, int n,
                  const float *hof_genomes, const double *hof_fitness, int n_hof, const int32_t *hof_pick, uint64_t seed,
                  uint64_t generation, double *rewards, int32_t *frames)
 {
-    Sim *sim = (Sim *)h;
-    roll::RolloutParams p;
-    memset(&p, 0, sizeof(p));
-    p.tables = &sim->T; p.needed = sim->needed.data(); p.start = sim->start;
+    roll::RolloutParams p = rollout_params((Sim *)h, core, nodes, n_layers, bias, max_frames, seed, generation);
     p.genomes = genomes; p.hof_genomes = hof_genomes; p.hof_fitness = hof_fitness; p.hof_pick = hof_pick;
-    p.n = n; p.n_hof = n_hof; p.games = games; p.schedule = schedule; p.win_score = 3; p.timeout_thresh = 2000; p.max_frames = max_frames;
-    p.core = core; p.time_scaler = 100.0; p.paddle_height = 16.0; p.seed = seed; p.generation = generation;
-    p.shape.n_layers = n_layers; p.shape.bias = bias;
-    int G = 0;
-    for (int i = 0; i < n_layers; ++i) p.shape.nodes[i] = nodes[i];
-    for (int i = 0; i + 1 < n_layers; ++i) G += (nodes[i] + (bias ? 1 : 0)) * nodes[i + 1];
-    p.G = G;
+    p.n = n; p.n_hof = n_hof; p.games = games; p.schedule = schedule;
     p.rewards = rewards; p.frames = frames;
-    for (int players = 1; players <= 2; ++players)                 // as ngp_evaluate builds it (csrc/ngp_core.cu)
-        for (int la = 0; la < 3; ++la)
-            for (int ra = 0; ra < 3; ++ra) {
-                uint8_t a[16] = {0};
-                a[0] = 1; a[15] = 1;
-                a[4] = ra == pol::ACT_UP; a[5] = ra == pol::ACT_DOWN;
-                a[6] = la == pol::ACT_UP; a[7] = la == pol::ACT_DOWN;
-                p.input_table[players - 1][la * 3 + ra] = roll::action_to_input(a, players, kDefaultButtonMap);
-            }
-    a26::Ram ram{sim->ram_words};
-    for (int e = 0; e < n * games; ++e) {
-        roll::Episode ep;
-        a26::Chip s; a26::CpuRegs r;
-        roll::episode_begin(ep, p, e, s, r, ram);
-        double reward = 0.0;
-        if (core) { while (!roll::episode_frame<1>(ep, p, s, r, sim->T, ram, &reward)) {} }
-        else { while (!roll::episode_frame<0>(ep, p, s, r, sim->T, ram, &reward)) {} }
-        rewards[e] = reward; frames[e] = ep.frame;
-    }
+    play_lanes<false>((Sim *)h, p, roll::RecordArgs{});
+}
+
+int hs_validate_state(const ngp_game_state *st, uint64_t cart) { return gs::validate(st, cart); }
+
+// A match list: ngp_play_matches, ngp_record_matches and ngp_play_matches_states.  First the list check of match_check_kernel
+// (gs::match_entry_faults per match, gs::validate per start state): with any fault nothing is played or written and the
+// number of faults is returned.  Then every match plays as one lane.  With none of record, key, states, start and capture_at
+// the lanes mirror the flavours ngp_play_matches launches (REC = false); with any of them, the recording twins that
+// ngp_record_matches and ngp_play_matches_states launch (REC = true).  *frames_total (when given) = the frames played.
+long hs_play_list(void *h, int core, const int32_t *nodes, int n_layers, int bias, int max_frames, const float *genomes, int n_genomes,
+                  const int32_t *right, const int32_t *left, const double *mult, const int32_t *key, int n_matches,
+                  const ngp_game_state *states, int n_states, const int32_t *start, int fresh, const int32_t *capture_at,
+                  ngp_game_state *capture, int max_record, ngp_frame_record *record, uint64_t cart, uint64_t seed, uint64_t generation,
+                  double *rewards, int32_t *frames, int32_t *scores, uint64_t *frames_total)
+{
+    long faults = 0;
+    for (int m = 0; m < n_matches; ++m)
+        faults += gs::match_entry_faults(m, right, left, n_genomes, key, capture_at, start, states, n_states);
+    for (int k = 0; k < n_states; ++k) faults += gs::validate(states + k, cart) == 0;
+    if (faults) return faults;
+    roll::RolloutParams p = rollout_params((Sim *)h, core, nodes, n_layers, bias, max_frames, seed, generation);
+    p.genomes = genomes; p.n = n_matches; p.games = 1;
+    p.match_right = right; p.match_left = left; p.match_mult = mult;
+    p.rewards = rewards; p.frames = frames; p.scores = scores;
+    roll::RecordArgs rec = {};
+    rec.record = record; rec.key = key; rec.max_record = record ? max_record : 0;
+    rec.fresh = fresh; rec.states = states; rec.start = start; rec.capture_at = capture_at; rec.capture = capture; rec.cart = cart;
+    const bool twin = record || key || states || start || capture_at;
+    const uint64_t total = twin ? play_lanes<true>((Sim *)h, p, rec) : play_lanes<false>((Sim *)h, p, rec);
+    if (frames_total) *frames_total = total;
+    return 0;
 }
 
 // Self-test of the register mirror of the hot latches (csrc/a26_core.cuh: HotLatches, hot_write, hot_display_writes) against

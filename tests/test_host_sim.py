@@ -2,31 +2,19 @@
 an intrinsics shim and is compared with the oracle.  This is a debugging aid for the GPU-less build
 container; the binding parity evidence is tests/test_gpu_parity.py on a real B200."""
 import ctypes
-import os
-import subprocess
 
 import numpy as np
 import pytest
 
 import oracle
+from host_sim_lib import library
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-SRC = os.path.join(ROOT, "tests", "host_sim", "host_sim.cpp")
-LIB = os.path.join(ROOT, "tests", "host_sim", "libhost_sim.so")
 vp = ctypes.c_void_p
 
 
 @pytest.fixture(scope="module")
 def hs():
-    subprocess.check_call(["g++", "-O2", "-std=c++17", "-ffp-contract=off", "-fPIC", "-shared", "-Wno-unknown-pragmas", "-o", LIB, SRC])
-    L = ctypes.CDLL(LIB)
-    L.hs_create.restype = vp
-    L.hs_env_reset.argtypes = [vp, ctypes.c_int]
-    L.hs_env_power_on.argtypes = [vp]
-    L.hs_env_step.argtypes = [vp, ctypes.c_int] + [vp] * 7
-    L.hs_env_step_fast.argtypes = [vp, ctypes.c_int] + [vp] * 4
-    L.hs_evaluate.argtypes = [vp, ctypes.c_int, vp, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int, vp, ctypes.c_int, vp, vp,
-                              ctypes.c_int, vp, ctypes.c_uint64, ctypes.c_uint64, vp, vp]
+    L = library()
     return L, vp(L.hs_create(oracle.load_rom()))
 
 
@@ -100,13 +88,7 @@ def test_fused_mode_observation_matches_oracle(hs, core):
 
 
 def _build_variant(name, *flags):
-    lib = os.path.join(ROOT, "tests", "host_sim", f"libhost_sim_{name}.so")
-    srcs = [SRC] + ([os.path.join(ROOT, "tests", "host_sim", "host_sim_stats.cpp")] if "-DA26_STATS" in flags else [])
-    subprocess.check_call(["g++", "-O2", "-std=c++17", "-ffp-contract=off", "-fPIC", "-shared", "-Wno-unknown-pragmas", *flags, "-o", lib, *srcs])
-    L = ctypes.CDLL(lib)
-    L.hs_create.restype = vp
-    L.hs_env_reset.argtypes = [vp, ctypes.c_int]
-    L.hs_env_step_fast.argtypes = [vp, ctypes.c_int] + [vp] * 4
+    L = library(name, flags)
     return L, vp(L.hs_create(oracle.load_rom()))
 
 
@@ -132,7 +114,6 @@ def test_superblocks_are_taken():
     enters the main display loop's block and the score loop's block, and the dispatcher is left with < 100 trips per frame
     (188 without the blocks)."""
     L, sim = _build_variant("stats", "-DA26_STATS")
-    L.hs_stats.restype = ctypes.POINTER(ctypes.c_ulonglong * 16)
     st = L.hs_stats().contents
     frames = 200
     for i in range(16):
@@ -153,7 +134,6 @@ def test_hot_latch_mirror_equals_poke_quick_on_random_states(hs):
     hot_display_writes must give poke_quick()'s verdict and tia_apply()'s latch bytes for ANY latch state -- the cartridge's own
     traces never delay a player or unlock a missile, so those rules are exercised here on random states."""
     L, _ = hs
-    L.hs_hot_latch_selftest.argtypes = [ctypes.c_uint64, ctypes.c_int]
     assert L.hs_hot_latch_selftest(1, 200000) == 0
 
 
@@ -164,7 +144,6 @@ def test_display_loop_event_queue_early_replay():
     L, sim = _build_variant("smallqueue", "-DA26_SB_MAX_EVENTS=9")
     _run_fast_against_oracle(L, sim, 400, seed=5)
     # the every-pixel flavour through the same queue: frame buffer, RAM and CPU registers
-    L.hs_env_step.argtypes = [vp, ctypes.c_int] + [vp] * 7
     rng = np.random.RandomState(6)
     env = oracle.Atari(); env.reset_to_state(0); L.hs_env_reset(sim, 0)
     ram = np.zeros(128, np.uint8); fb = np.zeros((210, 160), np.uint8); loc = np.zeros(6); valid = np.zeros(3, np.uint8)

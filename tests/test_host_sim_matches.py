@@ -1,19 +1,15 @@
-"""CPU-side check of the match-list form of the fused rollout (ngp_play_matches): tests/host_sim/host_sim_matches.cpp runs
+"""CPU-side check of the match-list form of the fused rollout (ngp_play_matches): tests/host_sim runs
 csrc/rollout.cuh's plan_env with an explicit list, and every match must equal the oracle's perform_episode with the same
 opponent, start state, multiplier and random key (environment index = match index): reward, frame count and both scores.
 The list holds pairings neither built-in schedule can express."""
 import ctypes
-import os
-import subprocess
 
 import numpy as np
 import pytest
 
 import oracle
+from host_sim_lib import library
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-SRC = os.path.join(ROOT, "tests", "host_sim", "host_sim_matches.cpp")
-LIB = os.path.join(ROOT, "tests", "host_sim", "libhost_sim_matches.so")
 vp = ctypes.c_void_p
 
 OPP_HARDCODED, OPP_SCORE_HARDCODED, OPP_ROBOT = -1, -2, -3        # include/ngp.h NGP_OPP_*
@@ -37,11 +33,7 @@ MATCHES = [
 
 @pytest.fixture(scope="module")
 def hs():
-    subprocess.check_call(["g++", "-O2", "-std=c++17", "-ffp-contract=off", "-fPIC", "-shared", "-Wno-unknown-pragmas", "-o", LIB, SRC])
-    L = ctypes.CDLL(LIB)
-    L.hs_create.restype = vp
-    L.hs_play_matches.argtypes = [vp, ctypes.c_int, vp, ctypes.c_int, ctypes.c_int, ctypes.c_int, vp, vp, vp, vp, ctypes.c_int,
-                                  ctypes.c_uint64, ctypes.c_uint64, vp, vp, vp]
+    L = library()
     return L, vp(L.hs_create(oracle.load_rom()))
 
 
@@ -70,7 +62,8 @@ def test_match_list_matches_oracle(hs, core):
     n = len(MATCHES)
     rew = np.zeros(n); frm = np.zeros(n, np.int32); sc = np.zeros((n, 2), np.int32)
     seed, generation = 21, 3
-    L.hs_play_matches(sim, core, P(nodes), 3, 1, 0, P(genomes), P(right), P(left), P(mult), n, seed, generation, P(rew), P(frm), P(sc))
+    L.hs_play_list(sim, core, P(nodes), 3, 1, 0, P(genomes), len(genomes), P(right), P(left), P(mult), None, n, None, 0, None, 0, None,
+                   None, 0, None, 0, seed, generation, P(rew), P(frm), P(sc), None)
     shape = oracle.Shape.make([6, 2, 2])
     for m in range(n):
         res = oracle_match(shape, genomes, int(right[m]), int(left[m]), float(mult[m]), seed, generation, m)

@@ -1,20 +1,16 @@
-"""CPU-side check of the recording form of the fused rollout (ngp_record_matches): tests/host_sim/host_sim_record.cpp runs
+"""CPU-side check of the recording form of the fused rollout (ngp_record_matches): tests/host_sim runs
 csrc/rollout.cuh's episode_frame<.., REC = true> and record_frame over the irregular match list of test_host_sim_matches,
 and every recorded frame must equal the oracle's perform_episode trace: both decisions, both scores, the three valid bits,
 the timeout counter and the frame count.  With a key list, match m must equal the oracle run with env_id = key[m]."""
 import ctypes
-import os
-import subprocess
 
 import numpy as np
 import pytest
 
 import oracle
+from host_sim_lib import library
 from test_host_sim_matches import MATCHES, OPP_ROBOT, OPP_SCORE_HARDCODED
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-SRC = os.path.join(ROOT, "tests", "host_sim", "host_sim_record.cpp")
-LIB = os.path.join(ROOT, "tests", "host_sim", "libhost_sim_record.so")
 vp = ctypes.c_void_p
 MAX_RECORD = 12000
 # include/ngp.h ngp_frame_record
@@ -24,11 +20,7 @@ assert FRAME_RECORD.itemsize == 32
 
 @pytest.fixture(scope="module")
 def hs():
-    subprocess.check_call(["g++", "-O2", "-std=c++17", "-ffp-contract=off", "-fPIC", "-shared", "-Wno-unknown-pragmas", "-o", LIB, SRC])
-    L = ctypes.CDLL(LIB)
-    L.hs_create.restype = vp
-    L.hs_record_matches.argtypes = [vp, ctypes.c_int, vp, ctypes.c_int, ctypes.c_int, ctypes.c_int, vp, vp, vp, vp, vp, ctypes.c_int,
-                                    ctypes.c_uint64, ctypes.c_uint64, ctypes.c_int, vp, vp, vp, vp]
+    L = library()
     return L, vp(L.hs_create(oracle.load_rom()))
 
 
@@ -86,8 +78,8 @@ def test_record_matches_oracle_trace(hs, core, with_key):
     rec["timeout"] = -12345
     rew = np.zeros(n); frm = np.zeros(n, np.int32); sc = np.zeros((n, 2), np.int32)
     seed, generation = 21, 3
-    L.hs_record_matches(sim, core, P(nodes), 3, 1, 0, P(genomes), P(right), P(left), P(mult), P(keys) if with_key else None, n, seed,
-                        generation, MAX_RECORD, P(rec), P(rew), P(frm), P(sc))
+    L.hs_play_list(sim, core, P(nodes), 3, 1, 0, P(genomes), len(genomes), P(right), P(left), P(mult), P(keys) if with_key else None, n,
+                   None, 0, None, 0, None, None, MAX_RECORD, P(rec), 0, seed, generation, P(rew), P(frm), P(sc), None)
     check_against_oracle(rec, rew, frm, sc, genomes, right, left, mult, keys, seed, generation)
 
 
@@ -97,8 +89,6 @@ def test_key_drives_the_random_fall_back(hs, core):
     (self-play between visible paddles showed none), so the key decides the game.  Match m played with key[m] must equal
     the keyless game at list position key[m] bit for bit, and its decisions must be the oracle's Philox draws for key[m]."""
     L, _ = hs
-    L.hs_create_colours.restype = vp
-    L.hs_create_colours.argtypes = [ctypes.c_char_p, vp, vp, vp]
     colour = lambda c: np.array(c, np.uint8)                                                    # noqa: E731
     ball, blind, right_c = colour([236, 236, 236]), colour([1, 2, 3]), colour([92, 186, 92])
     sim = vp(L.hs_create_colours(oracle.load_rom(), P(ball), P(blind), P(right_c)))
@@ -110,8 +100,8 @@ def test_key_drives_the_random_fall_back(hs, core):
         n = len(right)
         rec = np.zeros((n, T), FRAME_RECORD)
         rew = np.zeros(n); frm = np.zeros(n, np.int32); sc = np.zeros((n, 2), np.int32)
-        L.hs_record_matches(sim, core, P(nodes), 3, 1, T, P(genomes), P(right), P(left), P(np.ones(n)), P(keys), n, seed, generation,
-                            T, P(rec), P(rew), P(frm), P(sc))
+        L.hs_play_list(sim, core, P(nodes), 3, 1, T, P(genomes), len(genomes), P(right), P(left), P(np.ones(n)), P(keys), n, None, 0, None,
+                       0, None, None, T, P(rec), 0, seed, generation, P(rew), P(frm), P(sc), None)
         return rec, rew, frm, sc
 
     right = np.array([0, 1, 2, 3, 0], np.int32)

@@ -1,22 +1,18 @@
-"""CPU-side check of save states (ngp_play_matches_states): tests/host_sim/host_sim_states.cpp runs csrc/rollout.cuh's frame
+"""CPU-side check of save states (ngp_play_matches_states): tests/host_sim runs csrc/rollout.cuh's frame
 code and csrc/game_state.cuh's pack / unpack / validate exactly as the recording twins of rollout_kernel call them, on both
 6507 cores.  A resumed capture must replay the rest of the uninterrupted game bit for bit; captures must not depend on the core;
 a fresh start from a capture must equal the oracle stepped to that frame and then playing a new episode; and no corrupted,
 foreign or mismatched state may get past the list check."""
 import ctypes
-import os
-import subprocess
 
 import numpy as np
 import pytest
 
 import oracle
+from host_sim_lib import library
 from test_host_sim_matches import MATCHES, OPP_ROBOT, OPP_SCORE_HARDCODED
 from test_host_sim_record import FRAME_RECORD
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-SRC = os.path.join(ROOT, "tests", "host_sim", "host_sim_states.cpp")
-LIB = os.path.join(ROOT, "tests", "host_sim", "libhost_sim_states.so")
 vp = ctypes.c_void_p
 STATE_BYTES = 512                     # include/ngp.h NGP_GAME_STATE_BYTES
 MAX_RECORD = 12000
@@ -44,14 +40,7 @@ def seal(state: np.ndarray) -> np.ndarray:
 
 @pytest.fixture(scope="module")
 def hs():
-    subprocess.check_call(["g++", "-O2", "-std=c++17", "-ffp-contract=off", "-fPIC", "-shared", "-Wno-unknown-pragmas", "-o", LIB, SRC])
-    L = ctypes.CDLL(LIB)
-    L.hs_create.restype = vp
-    L.hs_validate_state.argtypes = [vp, ctypes.c_uint64]
-    L.hs_play_states.restype = ctypes.c_long
-    L.hs_play_states.argtypes = [vp, ctypes.c_int, vp, ctypes.c_int, ctypes.c_int, ctypes.c_int, vp, ctypes.c_int, vp, vp, vp, vp,
-                                 ctypes.c_int, vp, ctypes.c_int, vp, ctypes.c_int, vp, vp, ctypes.c_int, vp, ctypes.c_uint64,
-                                 ctypes.c_uint64, ctypes.c_uint64, vp, vp, vp, vp]
+    L = library()
     rom = oracle.load_rom()
     return L, vp(L.hs_create(rom)), fnv1a64(rom)
 
@@ -62,7 +51,7 @@ def P(a):
 
 def play(hs, core, genomes, right, left, mult, key=None, states=None, start=None, fresh=0, capture_at=None, record=True,
          cart=None, capture=None):
-    """One hs_play_states call.  Returns (faults, dict of results); the record's timeout field starts at SENTINEL and the
+    """One hs_play_list call.  Returns (faults, dict of results); the record's timeout field starts at SENTINEL and the
     capture buffer at 0xAB (or `capture`)."""
     L, sim, cart0 = hs
     n = len(right)
@@ -76,10 +65,10 @@ def play(hs, core, genomes, right, left, mult, key=None, states=None, start=None
     if capture_at is not None:
         cap = np.full((n, STATE_BYTES), 0xAB, np.uint8) if capture is None else capture
     n_states = 0 if states is None else len(states)
-    faults = L.hs_play_states(sim, core, P(NODES), 3, 1, 0, P(genomes), len(genomes), P(right), P(left), P(mult), P(key), n,
-                              P(states), n_states, P(start), fresh, P(capture_at), P(cap), MAX_RECORD, P(rec),
-                              cart0 if cart is None else cart, SEED, GENERATION, P(out["rewards"]), P(out["frames"]),
-                              P(out["scores"]), ctypes.byref(out["total"]))
+    faults = L.hs_play_list(sim, core, P(NODES), 3, 1, 0, P(genomes), len(genomes), P(right), P(left), P(mult), P(key), n,
+                            P(states), n_states, P(start), fresh, P(capture_at), P(cap), MAX_RECORD, P(rec),
+                            cart0 if cart is None else cart, SEED, GENERATION, P(out["rewards"]), P(out["frames"]),
+                            P(out["scores"]), ctypes.byref(out["total"]))
     out["record"], out["capture"], out["total"] = rec, cap, out["total"].value
     return faults, out
 
