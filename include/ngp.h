@@ -170,7 +170,7 @@ enum { NGP_OPP_HARDCODED = -1,         /* dumb_ais.HardcodedAi: game 0 of main.e
  * A right[m] outside [0, n_genomes), a left[m] that is neither a row nor an NGP_OPP_* code, or n_matches < 1 return
  * NGP_ERR_INVALID and nothing is played: the lists are checked on the device and the count of bad entries is read back,
  * so the call synchronises its stream once before the rollout is launched.  Networks wider than the fused rollout
- * takes (any layer > 32 units) return NGP_ERR_UNSUPPORTED. */
+ * takes (any layer > 32 units) return NGP_ERR_UNSUPPORTED; ngp_play_matches_stepwise plays them. */
 int ngp_play_matches(ngp_handle *h, const float *genomes, int32_t n_genomes,
                      const int32_t *right, const int32_t *left, const double *mult, int32_t n_matches,
                      uint64_t seed, uint64_t generation,
@@ -201,7 +201,7 @@ typedef struct {
  * g has key g * games + k.
  * Refusals (NGP_ERR_INVALID, nothing written): those of ngp_play_matches, max_record < 1, a NULL or misaligned record, and
  * any key[m] < 0 (counted on the device with the list check, no further synchronisation).  Networks wider than 32 units
- * return NGP_ERR_UNSUPPORTED. */
+ * return NGP_ERR_UNSUPPORTED; ngp_play_matches_stepwise records them. */
 int ngp_record_matches(ngp_handle *h, const float *genomes, int32_t n_genomes,
                        const int32_t *right, const int32_t *left, const double *mult, const int32_t *key, int32_t n_matches,
                        uint64_t seed, uint64_t generation, int32_t max_record, ngp_frame_record *record,
@@ -242,8 +242,8 @@ int ngp_env_set_state(ngp_handle *h, const ngp_game_state *states, int32_t n_env
  * Refusals (NGP_ERR_INVALID, nothing written, one synchronisation as in ngp_play_matches): those of ngp_record_matches (with
  * a non-NULL record), start[m] outside [-1, n_states), a state that fails validation, a state whose players value disagrees
  * with left[m] (players 1 with NGP_OPP_ROBOT only), capture_at[m] < 0, capture_at without capture, misaligned state arrays.
- * Networks wider than 32 units return NGP_ERR_UNSUPPORTED.  With start, capture_at and record all NULL the results are
- * ngp_play_matches' bits. */
+ * Networks wider than 32 units return NGP_ERR_UNSUPPORTED (ngp_play_matches_stepwise below plays them).  With start,
+ * capture_at and record all NULL the results are ngp_play_matches' bits. */
 int ngp_play_matches_states(ngp_handle *h, const float *genomes, int32_t n_genomes,
                             const int32_t *right, const int32_t *left, const double *mult, const int32_t *key, int32_t n_matches,
                             const ngp_game_state *states, int32_t n_states, const int32_t *start, int32_t fresh,
@@ -251,6 +251,27 @@ int ngp_play_matches_states(ngp_handle *h, const float *genomes, int32_t n_genom
                             int32_t max_record, ngp_frame_record *record,
                             uint64_t seed, uint64_t generation, double *rewards, int32_t *frames, int32_t *scores,
                             uint64_t *frames_total, void *stream);
+
+/* ---- ngp_play_matches_states on the per-frame driver, for networks of any width.
+ * Takes ngp_play_matches_states' arguments in the same order and has its contract: the same outputs, the same record and
+ * capture semantics, the same refusals (NGP_ERR_INVALID, nothing written) with the same single read-back before anything is
+ * played.  Every match is played by the per-frame driver of wide ngp_evaluate: one launch per frame emulates every running
+ * match, the networks run between the frames, one more launch decides.
+ * Wide networks (any layer > 32 units): 6 inputs and at most 8 outputs as in ngp_evaluate, otherwise NGP_ERR_INVALID.  Every
+ *   MLP side of every match is one row per frame; the rows are grouped by genome into chunks of T rows (T = the smallest power
+ *   of two in [16, 128] not below the mean rows per genome that plays), and the chunks run through ngp_evaluate's wide MLP
+ *   kernels with each chunk's genome as the weight index.  The whole genome table is packed once per call as ngp_mlp_prepare
+ *   packs it (about 1.05 MB per genome for [6,512,512,2]).
+ * Networks the fused rollout takes: the decisions are its FP64 policies, so rewards, frames, scores, records, captures and
+ *   *frames_total are the fused entry points' bits on the same arguments.
+ * The call returns after every match has finished: like wide ngp_evaluate it synchronises its stream every 8 frames. */
+int ngp_play_matches_stepwise(ngp_handle *h, const float *genomes, int32_t n_genomes,
+                              const int32_t *right, const int32_t *left, const double *mult, const int32_t *key, int32_t n_matches,
+                              const ngp_game_state *states, int32_t n_states, const int32_t *start, int32_t fresh,
+                              const int32_t *capture_at, ngp_game_state *capture,
+                              int32_t max_record, ngp_frame_record *record,
+                              uint64_t seed, uint64_t generation, double *rewards, int32_t *frames, int32_t *scores,
+                              uint64_t *frames_total, void *stream);
 
 /* ---- K4: GA step.  Replaces toolbox.select / varAnd(mate, mutate) inside eaSimple
  * (ga.py:89-94, main.py:165-170; DEAP selTournament, cxBlend, mutGaussian).

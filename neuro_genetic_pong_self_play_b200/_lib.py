@@ -28,6 +28,7 @@ EXPORTS = [
     "ngp_config_size", "ngp_set_option", "ngp_select", "ngp_mate", "ngp_mutate", "ngp_hof_update", "ngp_exchange_bytes",
     "ngp_pack_elites", "ngp_unpack_elites", "ngp_mlp_prepare", "ngp_mlp_forward_prepared",
     "ngp_play_matches", "ngp_record_matches", "ngp_env_get_state", "ngp_env_set_state", "ngp_play_matches_states",
+    "ngp_play_matches_stepwise",
 ]
 
 
@@ -96,6 +97,7 @@ def load(build_if_missing: bool = True):
     L.ngp_env_set_state.argtypes = [vp, vp, i32, vp]
     L.ngp_play_matches_states.argtypes = [vp, vp, i32, vp, vp, vp, vp, i32, vp, i32, vp, i32, vp, vp, i32, vp, u64, u64, vp, vp, vp,
                                           ctypes.POINTER(u64), vp]
+    L.ngp_play_matches_stepwise.argtypes = L.ngp_play_matches_states.argtypes
     L.ngp_evaluate_host.argtypes = [vp, vp, i32, vp, vp, i32, u64, u64, vp, ctypes.POINTER(u64)]
     L.ngp_ga_step.argtypes = [vp, vp, vp, i32, u64, u64, ctypes.POINTER(NgpNoise), vp, vp, vp, vp, vp]
     L.ngp_init_population.argtypes = [vp, vp, i32, u64, vp]

@@ -150,7 +150,10 @@ __global__ void env_digest_kernel(const Snapshot *envs, int n, uint32_t *out)
     o[7] = s.dump_enabled;
 }
 
-int ngp_evaluate_stepwise(ngp_handle *h, const RolloutParams &p, cudaStream_t st);     // ngp_stepwise.cu
+// ngp_stepwise.cu
+int ngp_evaluate_stepwise(ngp_handle *h, const RolloutParams &p, cudaStream_t st);
+int ngp_list_layout_count(ngp_handle *h, const int32_t *right, const int32_t *left, int n_matches, int n_genomes, cudaStream_t st);
+int ngp_play_list_stepwise(ngp_handle *h, const RolloutParams &p, const roll::RecordArgs &rec, int n_genomes, bool wide, cudaStream_t st);
 
 // fitness[g] = sum(rewards[g][:]) / games, summed in game order (main.py:65)
 __global__ void fitness_reduce_kernel(const double *__restrict__ rewards, int n, int games, double *__restrict__ fitness)
@@ -260,9 +263,9 @@ extern "C" int ngp_create(const ngp_config *cfg, const uint8_t *rom, int32_t dev
     NGP_CUDA(h->d_palette.ensure(128));
     NGP_CUDA(cudaMemcpy(h->d_palette.p, ngp_host::ntsc_palette, sizeof(ngp_host::ntsc_palette), cudaMemcpyHostToDevice));
     NGP_CUDA(h->d_start.ensure(2));
-    NGP_CUDA(h->d_counters.ensure(8));
-    NGP_CUDA(cudaMemset(h->d_counters.p, 0, 8 * sizeof(unsigned long long)));
-    NGP_CUDA(h->h_counters.ensure(8));
+    NGP_CUDA(h->d_counters.ensure(16));
+    NGP_CUDA(cudaMemset(h->d_counters.p, 0, 16 * sizeof(unsigned long long)));
+    NGP_CUDA(h->h_counters.ensure(16));
     // The two start snapshots depend on the cartridge image only: built once per process by the CUDA core (a single warp,
     // tens of milliseconds) and kept as an immutable host copy for later handles.
     {
@@ -544,23 +547,29 @@ extern "C" int ngp_evaluate(ngp_handle *h, const float *genomes, int32_t n, cons
 }
 
 // ngp_play_matches; ngp_record_matches and ngp_play_matches_states when `rec` is set (its pointers' alignment and the record
-// length already checked; n_states = the length of rec->states)
+// length already checked; n_states = the length of rec->states).  stepwise (ngp_play_matches_stepwise): the per-frame driver
+// plays the list (ngp_stepwise.cu) instead of the fused rollout; everything up to the one read-back is shared.
 static int play_match_list(ngp_handle *h, const float *genomes, int32_t n_genomes, const int32_t *right, const int32_t *left,
                            const double *mult, int32_t n_matches, uint64_t seed, uint64_t generation, double *rewards, int32_t *frames,
                            int32_t *scores, uint64_t *frames_total, cudaStream_t st, const roll::RecordArgs *rec, int32_t n_states,
-                           const char *who)
+                           const char *who, bool stepwise = false)
 {
     if (!(h && genomes && right && left && rewards && n_genomes > 0 && n_matches > 0)) {
         ngp_set_error("%s: bad arguments", who);
         return NGP_ERR_INVALID;
     }
-    for (int i = 0; i < h->cfg.n_layers; ++i)
-        if (h->cfg.nodes[i] > pol::FUSED_MAX_WIDTH) {
-            // the stepwise driver batches the MLP by genome with a fixed number of rows per genome; a match list has none
-            ngp_set_error("%s: networks with a layer wider than %d units are not supported (the fused rollout only)", who,
-                          pol::FUSED_MAX_WIDTH);
-            return NGP_ERR_UNSUPPORTED;
-        }
+    bool wide = false;
+    for (int i = 0; i < h->cfg.n_layers; ++i) wide |= h->cfg.nodes[i] > pol::FUSED_MAX_WIDTH;
+    if (wide && !stepwise) {
+        // the fused rollout runs the MLP in a thread's registers; ngp_play_matches_stepwise takes any width
+        ngp_set_error("%s: networks with a layer wider than %d units are not supported (the fused rollout only)", who,
+                      pol::FUSED_MAX_WIDTH);
+        return NGP_ERR_UNSUPPORTED;
+    }
+    if (wide && !(h->cfg.nodes[0] == 6 && h->cfg.nodes[h->cfg.n_layers - 1] <= 8)) {
+        ngp_set_error("%s: wide networks need 6 inputs and at most 8 outputs", who);
+        return NGP_ERR_INVALID;
+    }
     if (h->cfg.core && !h->rom_translated) {
         ngp_set_error("%s: the statically translated core was generated from a different cartridge; use NGP_CORE_INTERPRETER", who);
         return NGP_ERR_UNSUPPORTED;
@@ -577,7 +586,13 @@ static int play_match_list(ngp_handle *h, const float *genomes, int32_t n_genome
                                                      h->cart_hash, h->d_counters.p + 3);
     h->launches++;
     NGP_CUDA(cudaGetLastError());
-    NGP_CUDA(cudaMemcpyAsync(h->h_counters.p + 3, h->d_counters.p + 3, sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+    // the stepwise driver's chunk counts of wide networks (d_counters[8, 14)) come back with the fault count
+    const bool layout = stepwise && wide;
+    if (layout) {
+        const int rc = ngp_list_layout_count(h, right, left, n_matches, n_genomes, st);
+        if (rc != NGP_OK) return rc;
+    }
+    NGP_CUDA(cudaMemcpyAsync(h->h_counters.p + 3, h->d_counters.p + 3, (layout ? 11 : 1) * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
     NGP_CUDA(cudaStreamSynchronize(st));
     if (h->h_counters.p[3]) {
         if (ra.start || ra.capture_at || n_states)
@@ -593,6 +608,16 @@ static int play_match_list(ngp_handle *h, const float *genomes, int32_t n_genome
     p.n = n_matches; p.games = 1;
     p.match_right = right; p.match_left = left; p.match_mult = mult;
     p.rewards = rewards; p.frames = frames ? frames : h->d_frames.p; p.scores = scores;
+    if (stepwise) {
+        const int rc = ngp_play_list_stepwise(h, p, ra, n_genomes, wide, st);
+        if (rc != NGP_OK) return rc;
+        if (frames_total) *frames_total = h->h_counters.p[1];
+        if (h->h_counters.p[2]) {
+            ngp_set_error("%s: %llu environments stopped on an emulator error", who, h->h_counters.p[2]);
+            return NGP_ERR_EMULATOR;
+        }
+        return NGP_OK;
+    }
     const int rc = launch_rollout(h, p, n_matches, st, who, rec);
     if (rc != NGP_OK) return rc;
     return frames_total ? read_rollout_counters(h, st, frames_total, who) : NGP_OK;
@@ -619,6 +644,28 @@ extern "C" int ngp_record_matches(ngp_handle *h, const float *genomes, int32_t n
                            frames_total, (cudaStream_t)stream, &rec, 0, "ngp_record_matches");
 }
 
+// ngp_play_matches_states and ngp_play_matches_stepwise (same arguments, same checks in the same order)
+static int play_matches_states(ngp_handle *h, const float *genomes, int32_t n_genomes, const int32_t *right, const int32_t *left,
+                               const double *mult, const int32_t *key, int32_t n_matches, const ngp_game_state *states, int32_t n_states,
+                               const int32_t *start, int32_t fresh, const int32_t *capture_at, ngp_game_state *capture, int32_t max_record,
+                               ngp_frame_record *record, uint64_t seed, uint64_t generation, double *rewards, int32_t *frames,
+                               int32_t *scores, uint64_t *frames_total, void *stream, const char *who, bool stepwise)
+{
+    const std::string w(who);
+    NGP_REQUIRE(h, (w + ": null handle").c_str());
+    NGP_REQUIRE(!record || max_record >= 1, (w + ": a record needs max_record >= 1").c_str());
+    NGP_REQUIRE(((uintptr_t)record & 15) == 0, (w + ": the record buffer must be 16-byte aligned").c_str());
+    NGP_REQUIRE(n_states >= 0 && (n_states == 0 || states), (w + ": n_states states needed").c_str());
+    NGP_REQUIRE(((uintptr_t)states & 15) == 0 && ((uintptr_t)capture & 15) == 0, (w + ": state arrays must be 16-byte aligned").c_str());
+    NGP_REQUIRE(!capture_at || capture, (w + ": capture_at needs a capture buffer").c_str());
+    roll::RecordArgs rec = {};
+    rec.record = record; rec.key = key; rec.max_record = record ? max_record : 0;
+    rec.fresh = fresh ? 1 : 0; rec.states = states; rec.start = start; rec.capture_at = capture_at; rec.capture = capture;
+    rec.cart = h->cart_hash;
+    return play_match_list(h, genomes, n_genomes, right, left, mult, n_matches, seed, generation, rewards, frames, scores,
+                           frames_total, (cudaStream_t)stream, &rec, n_states, who, stepwise);
+}
+
 extern "C" int ngp_play_matches_states(ngp_handle *h, const float *genomes, int32_t n_genomes, const int32_t *right, const int32_t *left,
                                        const double *mult, const int32_t *key, int32_t n_matches, const ngp_game_state *states,
                                        int32_t n_states, const int32_t *start, int32_t fresh, const int32_t *capture_at,
@@ -626,18 +673,21 @@ extern "C" int ngp_play_matches_states(ngp_handle *h, const float *genomes, int3
                                        uint64_t generation, double *rewards, int32_t *frames, int32_t *scores, uint64_t *frames_total,
                                        void *stream)
 {
-    NGP_REQUIRE(h, "ngp_play_matches_states: null handle");
-    NGP_REQUIRE(!record || max_record >= 1, "ngp_play_matches_states: a record needs max_record >= 1");
-    NGP_REQUIRE(((uintptr_t)record & 15) == 0, "ngp_play_matches_states: the record buffer must be 16-byte aligned");
-    NGP_REQUIRE(n_states >= 0 && (n_states == 0 || states), "ngp_play_matches_states: n_states states needed");
-    NGP_REQUIRE(((uintptr_t)states & 15) == 0 && ((uintptr_t)capture & 15) == 0, "ngp_play_matches_states: state arrays must be 16-byte aligned");
-    NGP_REQUIRE(!capture_at || capture, "ngp_play_matches_states: capture_at needs a capture buffer");
-    roll::RecordArgs rec = {};
-    rec.record = record; rec.key = key; rec.max_record = record ? max_record : 0;
-    rec.fresh = fresh ? 1 : 0; rec.states = states; rec.start = start; rec.capture_at = capture_at; rec.capture = capture;
-    rec.cart = h->cart_hash;
-    return play_match_list(h, genomes, n_genomes, right, left, mult, n_matches, seed, generation, rewards, frames, scores,
-                           frames_total, (cudaStream_t)stream, &rec, n_states, "ngp_play_matches_states");
+    return play_matches_states(h, genomes, n_genomes, right, left, mult, key, n_matches, states, n_states, start, fresh, capture_at,
+                               capture, max_record, record, seed, generation, rewards, frames, scores, frames_total, stream,
+                               "ngp_play_matches_states", false);
+}
+
+extern "C" int ngp_play_matches_stepwise(ngp_handle *h, const float *genomes, int32_t n_genomes, const int32_t *right, const int32_t *left,
+                                         const double *mult, const int32_t *key, int32_t n_matches, const ngp_game_state *states,
+                                         int32_t n_states, const int32_t *start, int32_t fresh, const int32_t *capture_at,
+                                         ngp_game_state *capture, int32_t max_record, ngp_frame_record *record, uint64_t seed,
+                                         uint64_t generation, double *rewards, int32_t *frames, int32_t *scores, uint64_t *frames_total,
+                                         void *stream)
+{
+    return play_matches_states(h, genomes, n_genomes, right, left, mult, key, n_matches, states, n_states, start, fresh, capture_at,
+                               capture, max_record, record, seed, generation, rewards, frames, scores, frames_total, stream,
+                               "ngp_play_matches_stepwise", true);
 }
 
 extern "C" int ngp_profile_enable(ngp_handle *h, int32_t on)

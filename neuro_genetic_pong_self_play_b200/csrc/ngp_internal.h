@@ -65,7 +65,8 @@ struct ngp_handle {
     // fused evaluation scratch
     Buffer<double> d_rewards;
     Buffer<int32_t> d_frames;
-    Buffer<unsigned long long> d_counters;    // [0] next env, [1] frames, [2] emulator errors
+    Buffer<unsigned long long> d_counters;    // [0] next env, [1] frames, [2] emulator errors, [3] bad list entries / finished
+                                              // environments, [8, 14) ngp_play_matches_stepwise's chunk counts
     // host staging (pinned) for the *_host entry points
     HostBuffer<float> h_genomes; HostBuffer<double> h_fitness; Buffer<float> d_genomes_stage; Buffer<double> d_fitness_stage;
     Buffer<float> d_hof_stage; Buffer<double> d_hof_fit_stage;
@@ -79,6 +80,8 @@ struct ngp_handle {
     // ngp_evaluate for nets wider than the fused rollout (ngp_stepwise.cu): per-environment state (bytes of StepEnv), MLP
     // input rows, actions, gathered hall-of-fame opponents
     Buffer<uint8_t> step_envs; Buffer<float> step_x; Buffer<uint8_t> step_act; Buffer<float> step_opp;
+    // ngp_play_matches_stepwise's chunk layout: per genome rows | chunks | first chunk, the genome of every chunk, CUB scan scratch
+    Buffer<int32_t> list_genome; Buffer<int32_t> list_chunk; Buffer<uint8_t> list_scan_tmp;
     // ngp_mlp_prepare: packed wide layers of the prepared genome set (ngp_mlp_tmem.cu)
     Buffer<float> prep_packed; size_t prep_per_genome; const float *prep_src; int prep_n; int tmem_attr_set;
     int fs_per_sm;                                                          // resident find_stuff CTAs per SM
@@ -99,6 +102,10 @@ struct ngp_handle {
 // The wide MLP layer kernels take the genome from grid.y or grid.z, which CUDA caps at 65 535: ngp_mlp_forward and
 // ngp_mlp_prepare run larger genome sets in slices of at most this many genomes.
 constexpr int MLP_GENOME_SLICE = 65535;
+
+// ngp_ops.cu: the wide MLP over x[n_chunks][T][6] with the prepared weights of genome chunk_genome[c] for chunk c
+int ngp_mlp_forward_chunks(ngp_handle *h, const float *genomes, const int32_t *chunk_genome, const float *x, int n_chunks, int T,
+                           uint8_t *act, cudaStream_t st);
 
 void ngp_set_error(const char *fmt, ...);
 #define NGP_CUDA(expr)                                                                           \

@@ -139,10 +139,12 @@ __global__ void __launch_bounds__(256) mlp_pack_layer_kernel(const float *__rest
     }
 }
 
-template <int TN>
+// GATHER <true> (ngp_mlp_forward_chunks): batch g is a chunk of match-list rows with the packed weights of genome chunk_genome[g];
+// the empty pack keeps ngp_mlp_forward_prepared's instantiations as they were
+template <int TN, bool... GATHER>
 __global__ void __launch_bounds__(threads(TN), 2)
 mlp_layer_tmem_kernel(const float *__restrict__ packed, size_t per_genome, size_t layer_off, const float *__restrict__ in, int envs, int ni, int no,
-                      float *__restrict__ out)
+                      float *__restrict__ out, const int32_t *__restrict__ chunk_genome = nullptr)
 {
     constexpr uint32_t LBO = lbo(TN), TILE_B = tile_b(TN), STAGE_B = stage_b(TN), IDESC = idesc(TN);
     constexpr int B_WARPS = b_warps(TN), B_THREADS = 32 * B_WARPS;
@@ -163,7 +165,8 @@ mlp_layer_tmem_kernel(const float *__restrict__ packed, size_t per_genome, size_
         asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_base_slot)), "r"(TMEM_COLS) : "memory");
         asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
     }
-    const float *tiles = packed + (size_t)g * per_genome + layer_off + (size_t)ob * NC * (KC * TM);       // this CTA's NC contiguous 8 KB tiles
+    const size_t wg = (false || ... || GATHER) ? (size_t)chunk_genome[g] : (size_t)g;      // the genome whose packed weights this CTA streams
+    const float *tiles = packed + wg * per_genome + layer_off + (size_t)ob * NC * (KC * TM);       // this CTA's NC contiguous 8 KB tiles
     constexpr int COPY_WARP = (A_THREADS + B_THREADS) / 32 + 1;
     if (warp == COPY_WARP && lane == 0) {
         // the copy thread sets the barriers up itself and has the first NA weight tiles under way while warp 0 allocates tensor
@@ -328,7 +331,7 @@ mlp_layer_tmem_kernel(const float *__restrict__ packed, size_t per_genome, size_
         asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
         const int quad = warp & 3, colh = warp >> 2;
         const int o = ob * TM + quad * 32 + lane;
-        const float b = packed[(size_t)g * per_genome + layer_off + (size_t)((no + TM - 1) / TM) * NC * (KC * TM) + o];
+        const float b = packed[wg * per_genome + layer_off + (size_t)((no + TM - 1) / TM) * NC * (KC * TM) + o];
 #pragma unroll 1
         for (int part = 0; part < TN / 64; ++part) {
             const int col0 = colh * (TN / 2) + part * 32;
@@ -418,9 +421,11 @@ extern "C" int ngp_mlp_prepare(ngp_handle *h, const float *genomes, int32_t n_ge
     return NGP_OK;
 }
 
-// one prepared wide hidden layer (called by ngp_mlp_forward_prepared) for the prepared genomes [g0, g0 + n_genomes);
+// one prepared wide hidden layer (called by ngp_mlp_forward_prepared) for the prepared genomes [g0, g0 + n_genomes), or with
+// chunk_genome (ngp_mlp_forward_chunks) for n_genomes chunks of envs rows with the weights of prepared genomes chunk_genome[..];
 // NGP_ERR_UNSUPPORTED -> the caller uses the unprepared path
-int ngp_mlp_layer_tmem(ngp_handle *h, int l, size_t g0, const float *in, int n_genomes, int envs, float *out, cudaStream_t st)
+int ngp_mlp_layer_tmem(ngp_handle *h, int l, size_t g0, const float *in, int n_genomes, int envs, float *out, cudaStream_t st,
+                       const int32_t *chunk_genome)
 {
     const pol::Shape &sh = h->shape;
     if (!layer_is_packed(sh, l) || envs < 16 || !h->prep_packed.p) return NGP_ERR_UNSUPPORTED;
@@ -428,18 +433,24 @@ int ngp_mlp_layer_tmem(ngp_handle *h, int l, size_t g0, const float *in, int n_g
     for (int i = 0; i < l; ++i)
         if (layer_is_packed(sh, i)) layer_off += tmm::packed_floats(sh.nodes[i], sh.nodes[i + 1]);
     const int ni = sh.nodes[l], no = sh.nodes[l + 1];
-    const float *packed = h->prep_packed.p + g0 * h->prep_per_genome;
+    const float *packed = h->prep_packed.p + (chunk_genome ? 0 : g0) * h->prep_per_genome;
     if (!h->tmem_attr_set) {
         NGP_CUDA(cudaFuncSetAttribute(tmm::mlp_layer_tmem_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tmm::smem_bytes(64)));
         NGP_CUDA(cudaFuncSetAttribute(tmm::mlp_layer_tmem_kernel<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tmm::smem_bytes(128)));
+        NGP_CUDA(cudaFuncSetAttribute(tmm::mlp_layer_tmem_kernel<64, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tmm::smem_bytes(64)));
+        NGP_CUDA(cudaFuncSetAttribute(tmm::mlp_layer_tmem_kernel<128, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tmm::smem_bytes(128)));
         h->tmem_attr_set = 1;
     }
+    const uint32_t s64 = tmm::smem_bytes(64), s128 = tmm::smem_bytes(128);
+    const int t64 = tmm::threads(64), t128 = tmm::threads(128);
     if (envs > 64) {
         dim3 grid((no + tmm::TM - 1) / tmm::TM, (envs + 127) / 128, n_genomes);
-        tmm::mlp_layer_tmem_kernel<128><<<grid, tmm::threads(128), tmm::smem_bytes(128), st>>>(packed, h->prep_per_genome, layer_off, in, envs, ni, no, out);
+        if (chunk_genome) tmm::mlp_layer_tmem_kernel<128, true><<<grid, t128, s128, st>>>(packed, h->prep_per_genome, layer_off, in, envs, ni, no, out, chunk_genome);
+        else tmm::mlp_layer_tmem_kernel<128><<<grid, t128, s128, st>>>(packed, h->prep_per_genome, layer_off, in, envs, ni, no, out);
     } else {
         dim3 grid((no + tmm::TM - 1) / tmm::TM, 1, n_genomes);
-        tmm::mlp_layer_tmem_kernel<64><<<grid, tmm::threads(64), tmm::smem_bytes(64), st>>>(packed, h->prep_per_genome, layer_off, in, envs, ni, no, out);
+        if (chunk_genome) tmm::mlp_layer_tmem_kernel<64, true><<<grid, t64, s64, st>>>(packed, h->prep_per_genome, layer_off, in, envs, ni, no, out, chunk_genome);
+        else tmm::mlp_layer_tmem_kernel<64><<<grid, t64, s64, st>>>(packed, h->prep_per_genome, layer_off, in, envs, ni, no, out);
     }
     h->launches++;
     NGP_CUDA(cudaGetLastError());

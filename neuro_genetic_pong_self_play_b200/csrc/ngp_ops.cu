@@ -239,15 +239,19 @@ __global__ void __launch_bounds__(128) mlp_small_kernel(const float *__restrict_
 
 // one layer: in[g][e][ni] (+ implicit bias 1) x W_g[no][ni+bias] -> out[g][e][no] (sigmoid), or for the
 // last layer FP64 pre-activations zout[g][e][no]
-template <bool LAST>
+// GATHER (here and in every wide-path kernel below; ngp_mlp_forward_chunks): <.., true> takes batch g as a chunk of rows whose
+// weights are genome chunk_genome[g]'s.  An empty pack (the instantiations ngp_mlp_forward runs) reads no chunk_genome, and
+// keeps those instantiations' names and code.
+template <bool LAST, bool... GATHER>
 __global__ void __launch_bounds__(256) mlp_layer_kernel(const float *__restrict__ genomes, size_t w_off, int G, const float *__restrict__ in,
-                                                        int envs, int ni, int no, int bias, float *__restrict__ outp, double *__restrict__ zout)
+                                                        int envs, int ni, int no, int bias, float *__restrict__ outp, double *__restrict__ zout,
+                                                        const int32_t *__restrict__ chunk_genome = nullptr)
 {
     constexpr int TE = 64, TO = 64, TK = 32;
     __shared__ float As[TK][TE + 1];     // activations, k-major
     __shared__ float Ws[TK][TO + 1];     // weights, k-major
     const int g = blockIdx.z, e0 = blockIdx.y * TE, o0 = blockIdx.x * TO;
-    const float *W = genomes + (size_t)g * G + w_off;
+    const float *W = genomes + (size_t)((false || ... || GATHER) ? chunk_genome[g] : g) * G + w_off;
     const float *A = in + (size_t)g * envs * ni;
     const int K = ni + bias;
     const int tx = threadIdx.x & 15, ty = threadIdx.x >> 4;     // 16 x 16 threads, 4x4 outputs each
@@ -300,9 +304,10 @@ __global__ void __launch_bounds__(256) mlp_layer_kernel(const float *__restrict_
 // Thread = one output unit with its weight row in registers, the genome's input rows in shared memory (broadcast
 // reads), stores coalesced along the outputs.  Same accumulation order as mlp_layer_kernel (k ascending, bias last).
 constexpr int NARROW_K = 8;
-template <int NI>        // NI = compile-time fan-in (6: the observation vector), or 0 = run-time fan-in up to NARROW_K - bias
+template <int NI, bool... GATHER>        // NI = compile-time fan-in (6: the observation vector), or 0 = run-time fan-in up to NARROW_K - bias
 __global__ void __launch_bounds__(128) mlp_narrow_in_kernel(const float *__restrict__ genomes, size_t w_off, int G, const float *__restrict__ in,
-                                                            int envs, int ni_rt, int no, int bias, float *__restrict__ outp)
+                                                            int envs, int ni_rt, int no, int bias, float *__restrict__ outp,
+                                                            const int32_t *__restrict__ chunk_genome = nullptr)
 {
     constexpr int TE = 64;
     __shared__ float xs[TE * NARROW_K];
@@ -312,7 +317,7 @@ __global__ void __launch_bounds__(128) mlp_narrow_in_kernel(const float *__restr
     const float *src = in + ((size_t)g * envs + e0) * ni;
     for (int i = threadIdx.x; i < ne * ni; i += 128) xs[i] = __ldg(&src[i]);
     float w[NARROW_K];
-    const float *W = genomes + (size_t)g * G + w_off + (size_t)min(o, no - 1) * K;
+    const float *W = genomes + (size_t)((false || ... || GATHER) ? chunk_genome[g] : g) * G + w_off + (size_t)min(o, no - 1) * K;
 #pragma unroll
     for (int k = 0; k < NARROW_K; ++k) w[k] = k < K ? __ldg(&W[k]) : 0.f;
     float wb = 0.f;
@@ -338,12 +343,14 @@ __global__ void __launch_bounds__(128) mlp_narrow_in_kernel(const float *__restr
 
 // last layer with few outputs (the action layer): one warp per (genome, env) row, lanes stride over k, FP64
 // accumulation, decision on the FP64 sigmoids (reference argmax incl. the saturation tie rule)
+template <bool... GATHER>
 __global__ void __launch_bounds__(256) mlp_last_small_kernel(const float *__restrict__ genomes, size_t w_off, int G, const float *__restrict__ in,
-                                                             int envs, int ni, int no, int bias, uint8_t *__restrict__ act, float *__restrict__ out)
+                                                             int envs, int ni, int no, int bias, uint8_t *__restrict__ act, float *__restrict__ out,
+                                                             const int32_t *__restrict__ chunk_genome = nullptr)
 {
     extern __shared__ float w_s[];                     // [no][ni + bias]
     const int g = blockIdx.y, K = ni + bias;
-    const float *W = genomes + (size_t)g * G + w_off;
+    const float *W = genomes + (size_t)((false || ... || GATHER) ? chunk_genome[g] : g) * G + w_off;
     for (int i = threadIdx.x; i < no * K; i += blockDim.x) w_s[i] = __ldg(&W[i]);
     __syncthreads();
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -379,12 +386,13 @@ __global__ void __launch_bounds__(256) mlp_last_small_kernel(const float *__rest
 // warp w owns environments w, w+8, ..  Each lane keeps its 16 k-positions of every weight row in FP64 registers (loaded once
 // per genome), streams the activation rows with 16-byte loads (two rows in flight) and accumulates in FP64; the decision
 // is taken on the FP64 sigmoids like mlp_last_small_kernel.
-template <int NO>
+template <int NO, bool... GATHER>
 __global__ void __launch_bounds__(256) mlp_last_wide_kernel(const float *__restrict__ genomes, size_t w_off, int G, const float *__restrict__ in,
-                                                            int envs, int ni, int bias, uint8_t *__restrict__ act, float *__restrict__ out)
+                                                            int envs, int ni, int bias, uint8_t *__restrict__ act, float *__restrict__ out,
+                                                            const int32_t *__restrict__ chunk_genome = nullptr)
 {
     const int g = blockIdx.x, K = ni + bias, kj = ni >> 7;
-    const float *W = genomes + (size_t)g * G + w_off;
+    const float *W = genomes + (size_t)((false || ... || GATHER) ? chunk_genome[g] : g) * G + w_off;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     double w[NO][16];
 #pragma unroll
@@ -465,12 +473,13 @@ __global__ void mlp_decide_kernel(const double *__restrict__ z, long long rows, 
 int ngp_mlp_layer_tf32(ngp_handle *h, const float *genomes, size_t w_off, const float *in, int n_genomes, int envs, int ni, int no, int bias,
                        float *out, cudaStream_t st);   // ngp_mlp_tf32.cu
 
-int ngp_mlp_layer_tmem(ngp_handle *h, int l, size_t g0, const float *in, int n_genomes, int envs, float *out, cudaStream_t st);  // ngp_mlp_tmem.cu
+int ngp_mlp_layer_tmem(ngp_handle *h, int l, size_t g0, const float *in, int n_genomes, int envs, float *out, cudaStream_t st,
+                       const int32_t *chunk_genome);  // ngp_mlp_tmem.cu
 
 static int mlp_forward_impl(ngp_handle *h, const float *genomes, const float *x, int32_t n_genomes, int32_t envs, uint8_t *act, float *out,
                             void *stream, bool prepared);
 static int mlp_forward_slice(ngp_handle *h, const float *genomes, const float *x, size_t g0, int n_genomes, int envs, uint8_t *act,
-                             float *out, cudaStream_t st, bool prepared);
+                             float *out, cudaStream_t st, bool prepared, const int32_t *chunk_genome);
 
 extern "C" int ngp_mlp_forward(ngp_handle *h, const float *genomes, const float *x, int32_t n_genomes, int32_t envs, uint8_t *act,
                                float *out, void *stream)
@@ -511,17 +520,46 @@ static int mlp_forward_impl(ngp_handle *h, const float *genomes, const float *x,
         const int gn = n_genomes - g0 < MLP_GENOME_SLICE ? n_genomes - g0 : MLP_GENOME_SLICE;
         const size_t r0 = (size_t)g0 * envs;
         const int rc = mlp_forward_slice(h, genomes + (size_t)g0 * h->gene_size, x + r0 * n_in, g0, gn, envs, act + r0,
-                                         out ? out + r0 * n_out : nullptr, st, prepared);
+                                         out ? out + r0 * n_out : nullptr, st, prepared, nullptr);
+        if (rc != NGP_OK) return rc;
+    }
+    return NGP_OK;
+}
+
+// The match-list rows of ngp_play_matches_stepwise (ngp_stepwise_lists.cu): x[n_chunks][T][6] -> act[n_chunks][T], chunk c with
+// the weights of genome chunk_genome[c] of `genomes`, the set last passed to ngp_mlp_prepare.  The layer dispatch of the wide
+// path with every kernel's weight index taken from chunk_genome (the <.., true> instantiations); hidden layers the packed tcgen05
+// path does not take run on FFMA (mlp_layer_kernel), not on the unprepared 3xTF32 kernel.  Slices of at most MLP_GENOME_SLICE
+// chunks.
+int ngp_mlp_forward_chunks(ngp_handle *h, const float *genomes, const int32_t *chunk_genome, const float *x, int n_chunks, int T,
+                           uint8_t *act, cudaStream_t st)
+{
+    NGP_REQUIRE(h && h->prep_src == genomes && chunk_genome && x && act && n_chunks > 0 && T > 0,
+                "ngp_mlp_forward_chunks: bad arguments or genomes not prepared");
+    const pol::Shape &sh = h->shape;
+    int widest = 0;
+    for (int i = 0; i < sh.n_layers; ++i) widest = sh.nodes[i] > widest ? sh.nodes[i] : widest;
+    const int n_in = sh.nodes[0], n_out = sh.nodes[sh.n_layers - 1];
+    const size_t slice_rows = (size_t)(n_chunks < MLP_GENOME_SLICE ? n_chunks : MLP_GENOME_SLICE) * T;
+    NGP_CUDA(h->mlp_a.ensure(slice_rows * widest));
+    NGP_CUDA(h->mlp_b.ensure(slice_rows * widest));
+    NGP_CUDA(h->mlp_z.ensure(slice_rows * n_out));
+    for (int c0 = 0; c0 < n_chunks; c0 += MLP_GENOME_SLICE) {
+        const int cn = n_chunks - c0 < MLP_GENOME_SLICE ? n_chunks - c0 : MLP_GENOME_SLICE;
+        const size_t r0 = (size_t)c0 * T;
+        const int rc = mlp_forward_slice(h, genomes, x + r0 * n_in, 0, cn, T, act + r0, nullptr, st, true, chunk_genome + c0);
         if (rc != NGP_OK) return rc;
     }
     return NGP_OK;
 }
 
 // the layers of the wide path for genomes [g0, g0 + n_genomes) of the call (pointers already offset to g0; g0 locates the
-// genomes in the prepared packed copy)
+// genomes in the prepared packed copy); with chunk_genome: n_genomes chunks of `envs` rows with the weights of genomes
+// chunk_genome[..] (genomes not offset, g0 unused)
 static int mlp_forward_slice(ngp_handle *h, const float *genomes, const float *x, size_t g0, int n_genomes, int envs, uint8_t *act,
-                             float *out, cudaStream_t st, bool prepared)
+                             float *out, cudaStream_t st, bool prepared, const int32_t *chunk_genome)
 {
+    const bool gather = chunk_genome != nullptr;
     const pol::Shape &sh = h->shape;
     const long long rows = (long long)n_genomes * envs;
     const float *in = x;
@@ -535,21 +573,29 @@ static int mlp_forward_slice(ngp_handle *h, const float *genomes, const float *x
         if (l == L - 1 && no <= 8 && (size_t)no * (ni + bias) * 4 <= 48 * 1024) {
             // action layer: warp-per-row dot products, decision fused (no intermediate buffer)
             if (no <= 2 && ni % 128 == 0 && ni <= 512 && l > 0) {      // on top of a wide hidden layer (our own 16-byte aligned scratch)
-                if (no == 2) mlp_last_wide_kernel<2><<<n_genomes, 256, 0, st>>>(genomes, w_off, h->gene_size, in, envs, ni, bias, act, out);
+                if (gather) {
+                    if (no == 2) mlp_last_wide_kernel<2, true><<<n_genomes, 256, 0, st>>>(genomes, w_off, h->gene_size, in, envs, ni, bias, act, out, chunk_genome);
+                    else mlp_last_wide_kernel<1, true><<<n_genomes, 256, 0, st>>>(genomes, w_off, h->gene_size, in, envs, ni, bias, act, out, chunk_genome);
+                } else if (no == 2) mlp_last_wide_kernel<2><<<n_genomes, 256, 0, st>>>(genomes, w_off, h->gene_size, in, envs, ni, bias, act, out);
                 else mlp_last_wide_kernel<1><<<n_genomes, 256, 0, st>>>(genomes, w_off, h->gene_size, in, envs, ni, bias, act, out);
                 h->launches++;
                 NGP_CUDA(cudaGetLastError());
                 return NGP_OK;
             }
             dim3 g2((envs + 7) / 8, n_genomes);
-            mlp_last_small_kernel<<<g2, 256, (size_t)no * (ni + bias) * 4, st>>>(genomes, w_off, h->gene_size, in, envs, ni, no, bias, act, out);
+            const size_t smem = (size_t)no * (ni + bias) * 4;
+            if (gather) mlp_last_small_kernel<true><<<g2, 256, smem, st>>>(genomes, w_off, h->gene_size, in, envs, ni, no, bias, act, out, chunk_genome);
+            else mlp_last_small_kernel<><<<g2, 256, smem, st>>>(genomes, w_off, h->gene_size, in, envs, ni, no, bias, act, out);
             h->launches++;
             NGP_CUDA(cudaGetLastError());
             return NGP_OK;
         }
         if (l != L - 1 && ni + bias <= NARROW_K) {
             dim3 g3((no + 127) / 128, (envs + 63) / 64, n_genomes);
-            if (ni == 6) mlp_narrow_in_kernel<6><<<g3, 128, 0, st>>>(genomes, w_off, h->gene_size, in, envs, ni, no, bias, bufs[l & 1]);
+            if (gather) {
+                if (ni == 6) mlp_narrow_in_kernel<6, true><<<g3, 128, 0, st>>>(genomes, w_off, h->gene_size, in, envs, ni, no, bias, bufs[l & 1], chunk_genome);
+                else mlp_narrow_in_kernel<0, true><<<g3, 128, 0, st>>>(genomes, w_off, h->gene_size, in, envs, ni, no, bias, bufs[l & 1], chunk_genome);
+            } else if (ni == 6) mlp_narrow_in_kernel<6><<<g3, 128, 0, st>>>(genomes, w_off, h->gene_size, in, envs, ni, no, bias, bufs[l & 1]);
             else mlp_narrow_in_kernel<0><<<g3, 128, 0, st>>>(genomes, w_off, h->gene_size, in, envs, ni, no, bias, bufs[l & 1]);
             h->launches++;
             NGP_CUDA(cudaGetLastError());
@@ -557,18 +603,23 @@ static int mlp_forward_slice(ngp_handle *h, const float *genomes, const float *x
         }
         if (!launched && prepared && l != L - 1 && !h->opt_mlp_no_tf32) {
             // prepared genome set: weights stream from HBM straight into tensor memory (ngp_mlp_tmem.cu)
-            const int rc = ngp_mlp_layer_tmem(h, l, g0, in, n_genomes, envs, bufs[l & 1], st);
+            const int rc = ngp_mlp_layer_tmem(h, l, g0, in, n_genomes, envs, bufs[l & 1], st, chunk_genome);
             if (rc == NGP_OK) launched = true;
             else if (rc != NGP_ERR_UNSUPPORTED) return rc;
         }
-        if (!launched && l != L - 1 && !h->opt_mlp_no_tf32) {
+        if (!gather && !launched && l != L - 1 && !h->opt_mlp_no_tf32) {
             // wide hidden layer with enough environments per genome: tensor cores (3xTF32, tcgen05 + TMEM)
             const int rc = ngp_mlp_layer_tf32(h, genomes, w_off, in, n_genomes, envs, ni, no, bias, bufs[l & 1], st);
             if (rc == NGP_OK) launched = true;
             else if (rc != NGP_ERR_UNSUPPORTED) return rc;
         }
         if (!launched) {
-            if (l == L - 1) mlp_layer_kernel<true><<<grid, 256, 0, st>>>(genomes, w_off, h->gene_size, in, envs, ni, no, bias, nullptr, h->mlp_z.p);
+            if (gather) {
+                if (l == L - 1)
+                    mlp_layer_kernel<true, true><<<grid, 256, 0, st>>>(genomes, w_off, h->gene_size, in, envs, ni, no, bias, nullptr, h->mlp_z.p, chunk_genome);
+                else mlp_layer_kernel<false, true><<<grid, 256, 0, st>>>(genomes, w_off, h->gene_size, in, envs, ni, no, bias, bufs[l & 1], nullptr,
+                                                                        chunk_genome);
+            } else if (l == L - 1) mlp_layer_kernel<true><<<grid, 256, 0, st>>>(genomes, w_off, h->gene_size, in, envs, ni, no, bias, nullptr, h->mlp_z.p);
             else mlp_layer_kernel<false><<<grid, 256, 0, st>>>(genomes, w_off, h->gene_size, in, envs, ni, no, bias, bufs[l & 1], nullptr);
             h->launches++;
             NGP_CUDA(cudaGetLastError());

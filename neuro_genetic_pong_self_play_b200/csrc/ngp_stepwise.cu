@@ -13,31 +13,17 @@
 //   step_decide_kernel  get_actions' fall-backs, bots, bounds clamp, calculate_timeout_and_frames, termination, reward
 //                       (main.py:84-107, 128-154; utils.py:71-77, 104-109)
 //
-// Per-environment state (console snapshot + perform_episode's locals) lives in HBM between the kernels.  The host loop
-// launches frames without synchronising and reads the count of finished environments back every CHECK_EVERY frames.
+// Per-environment state (console snapshot + perform_episode's locals, stepwise.cuh) lives in HBM between the kernels.  The host
+// loop launches frames without synchronising and reads the count of finished environments back every CHECK_EVERY frames.
+// ngp_play_matches_stepwise (ngp_stepwise_lists.cu) runs match lists through the same frame kernel (ngp_step_frame).
 #include "ngp_internal.h"
 #include "rollout.cuh"
+#include "stepwise.cuh"
 
 using a26::Chip; using a26::CpuRegs; using a26::Ram; using a26::Snapshot; using a26::Tables;
 using roll::RolloutParams;
 
 namespace {
-
-constexpr int CHECK_EVERY = 8;
-
-struct StepEnv {
-    Snapshot snap;
-    // perform_episode's locals (main.py:70-75)
-    int32_t done, frame, timeout, total_frames, last_s1, last_s2;
-    uint8_t have_last_score, have_last_ball, left_act, right_act;
-    double last_ball[2];
-    // what the frame kernel saw (consumed by the decide kernel)
-    double loc[3][2];
-    uint8_t valid[3], s1, s2, emu_error, pad_[2];
-    // plan (main.py:33-58 / round-robin)
-    int32_t state, left_kind, left_row, right_row;      // rows of the batched MLP input / action arrays (-1: no MLP on the left)
-    double mult;
-};
 
 __device__ __forceinline__ void load_tables_cta(Tables &dst, const Tables *__restrict__ src)
 {
@@ -187,6 +173,17 @@ __global__ void step_decide_kernel(RolloutParams p, StepEnv *envs, int total, co
 }
 
 }  // namespace
+
+// one frame of every running environment (step_frame_kernel): the frame kernel of ngp_play_matches_stepwise's loop
+int ngp_step_frame(ngp_handle *h, const RolloutParams &p, void *envs, int total, float *x, float *x_hof, cudaStream_t st)
+{
+    StepEnv *e = static_cast<StepEnv *>(envs);
+    if (p.core) step_frame_kernel<1><<<(total + 31) / 32, 32, 0, st>>>(p, e, total, x, x_hof);
+    else step_frame_kernel<0><<<(total + 31) / 32, 32, 0, st>>>(p, e, total, x, x_hof);
+    h->launches++;
+    NGP_CUDA(cudaGetLastError());
+    return NGP_OK;
+}
 
 // called by ngp_evaluate (ngp_core.cu) with the rollout parameters filled in; synchronises the stream
 int ngp_evaluate_stepwise(ngp_handle *h, const RolloutParams &p, cudaStream_t st)

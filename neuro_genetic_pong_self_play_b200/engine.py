@@ -196,6 +196,17 @@ class Engine:
                                         ctypes.byref(total) if sync else None, _stream(self.device)), "ngp_evaluate")
         return {"fitness": fitness, "rewards": rewards, "frames": frames, "frames_total": int(total.value) if sync else None}
 
+    @property
+    def fused_fits(self) -> bool:
+        """True when every layer of the network fits the fused rollout (<= 32 units): the match-list methods then play in one
+        fused launch by default; wider networks are played by the per-frame driver (ngp_play_matches_stepwise)."""
+        return max(self.config.NETWORK_SHAPE) <= 32
+
+    def _stepwise(self, driver: str | None) -> bool:
+        if driver not in (None, "fused", "stepwise"):
+            raise ValueError(f"driver must be None, 'fused' or 'stepwise', not {driver!r}")
+        return driver == "stepwise" or (driver is None and not self.fused_fits)
+
     def _match_list(self, genomes, right, left, **per_match):
         """The argument check and the outputs the match-list methods share: genomes f32[N, gene_size], right and left i32[M],
         and per_match name=(tensor or None, dtype) of shape [M].  Returns dict(rewards f64[M], frames i32[M], scores i32[M, 2])."""
@@ -214,12 +225,19 @@ class Engine:
                 "scores": torch.empty((m, 2), dtype=torch.int32, device=self.device)}
 
     def play_matches(self, genomes: torch.Tensor, right: torch.Tensor, left: torch.Tensor, mult: torch.Tensor | None = None,
-                     seed: int = 0, generation: int = 0, sync: bool = True):
+                     seed: int = 0, generation: int = 0, sync: bool = True, driver: str | None = None):
         """An explicit match list in one fused launch (ngp_play_matches): match m puts genome row right[m] on the right against
         genome row left[m] (x-mirrored, as in self-play) or an OPP_* code; mult[m] is the hall-of-fame multiplier of the right
         player's score bonus (None = 1.0).  Returns dict(rewards f64[M] of the right player, frames i32[M], scores i32[M, 2]
         = (left, right) points, frames_total).  The lists are checked on the device; a bad entry raises NgpError and nothing
-        is played."""
+        is played.
+        driver: None = the fused launch when the network fits it (fused_fits), the per-frame driver (ngp_play_matches_stepwise,
+        any width, the call waits for the last match) otherwise; "fused" or "stepwise" forces one ("fused" raises NgpError on
+        wide networks).  Networks the fused rollout takes give the same bits on both drivers."""
+        if self._stepwise(driver):
+            out = self.play_matches_states(genomes, right, left, mult, seed=seed, generation=generation, sync=sync, driver="stepwise")
+            del out["left"]
+            return out
         out = self._match_list(genomes, right, left, mult=(mult, torch.float64))
         total = ctypes.c_uint64(0)
         _lib.check(self._L.ngp_play_matches(self._h, _p(genomes), genomes.shape[0], _p(right), _p(left), _p(mult), right.shape[0], seed,
@@ -229,13 +247,19 @@ class Engine:
         return out
 
     def record_matches(self, genomes: torch.Tensor, right: torch.Tensor, left: torch.Tensor, mult: torch.Tensor | None = None,
-                       key: torch.Tensor | None = None, max_record: int = 2048, seed: int = 0, generation: int = 0, sync: bool = True):
+                       key: torch.Tensor | None = None, max_record: int = 2048, seed: int = 0, generation: int = 0, sync: bool = True,
+                       driver: str | None = None):
         """play_matches with a per-frame trace of every match, recorded in the same fused launch (ngp_record_matches).
         key[m] (None = m) is the environment index of the random fall-back key, so that one match can reproduce one game of
         an evaluate call (round-robin game k of genome g: key g * games + k).  Returns play_matches' dict plus `left` (kept
         for rendering) and `record`: named views over one u8[M, T, 32] buffer (T = max_record; frame t of match m is valid
         for t < min(frames[m], T)): loc f32[M, T, 3, 2], valid u8[M, T] (bit 0 ball, 1 left, 2 right), score u8[M, T, 2],
-        act u8[M, T] (left | right << 2, after the bounds clamp) and timeout i32[M, T]."""
+        act u8[M, T] (left | right << 2, after the bounds clamp) and timeout i32[M, T].  driver: as in play_matches."""
+        if self._stepwise(driver):
+            if int(max_record) < 1:
+                raise _lib.NgpError("record_matches: max_record must be >= 1")
+            return self.play_matches_states(genomes, right, left, mult, key=key, max_record=max_record, seed=seed, generation=generation,
+                                            sync=sync, driver="stepwise")
         out = self._match_list(genomes, right, left, mult=(mult, torch.float64), key=(key, torch.int32))
         m = right.shape[0]
         raw = torch.empty((m, max(int(max_record), 0), _lib.NGP_FRAME_RECORD_BYTES), dtype=torch.uint8, device=self.device)
@@ -250,14 +274,17 @@ class Engine:
     def play_matches_states(self, genomes: torch.Tensor, right: torch.Tensor, left: torch.Tensor, mult: torch.Tensor | None = None,
                             key: torch.Tensor | None = None, states: torch.Tensor | None = None, start: torch.Tensor | None = None,
                             fresh: bool = False, capture_at: torch.Tensor | None = None, max_record: int = 0, seed: int = 0,
-                            generation: int = 0, sync: bool = True):
+                            generation: int = 0, sync: bool = True, driver: str | None = None):
         """record_matches whose matches may start from save states and capture their own (ngp_play_matches_states).
         states: u8[S, NGP_GAME_STATE_BYTES]; start[m] (None = all -1) picks match m's start state, -1 = the built-in one.  A
         state with an episode resumes it unless `fresh`; a fresh start plays a new episode from the state's console.
         capture_at[m]: after that many env.steps from the episode's start the state of match m is captured (left as zeros
         when the game ended before).  max_record > 0 records every frame as record_matches does.  Returns play_matches'
         dict plus `left`, plus `capture` u8[M, NGP_GAME_STATE_BYTES] when capture_at is given and `record` views when
-        max_record > 0.  Bad entries or states raise NgpError and nothing is played."""
+        max_record > 0.  Bad entries or states raise NgpError and nothing is played.  driver: as in play_matches (the per-frame
+        driver is ngp_play_matches_stepwise, with this method's arguments)."""
+        fn, who = ((self._L.ngp_play_matches_stepwise, "ngp_play_matches_stepwise") if self._stepwise(driver)
+                   else (self._L.ngp_play_matches_states, "ngp_play_matches_states"))
         out = self._match_list(genomes, right, left, mult=(mult, torch.float64), key=(key, torch.int32), start=(start, torch.int32),
                                capture_at=(capture_at, torch.int32))
         m = right.shape[0]
@@ -270,11 +297,10 @@ class Engine:
         raw = (torch.empty((m, int(max_record), _lib.NGP_FRAME_RECORD_BYTES), dtype=torch.uint8, device=self.device)
                if max_record > 0 else None)
         total = ctypes.c_uint64(0)
-        _lib.check(self._L.ngp_play_matches_states(
+        _lib.check(fn(
             self._h, _p(genomes), genomes.shape[0], _p(right), _p(left), _p(mult), _p(key), m, _p(states) if n_states else None,
             n_states, _p(start), 1 if fresh else 0, _p(capture_at), _p(capture), int(max_record), _p(raw), seed, generation,
-            _p(out["rewards"]), _p(out["frames"]), _p(out["scores"]), ctypes.byref(total) if sync else None, _stream(self.device)),
-            "ngp_play_matches_states")
+            _p(out["rewards"]), _p(out["frames"]), _p(out["scores"]), ctypes.byref(total) if sync else None, _stream(self.device)), who)
         out.update(frames_total=int(total.value) if sync else None, left=left)
         if capture is not None:
             out["capture"] = capture

@@ -10,7 +10,7 @@ Names and argument meaning follow the reference so its call sites read the same:
   save_checkpoint / load_latest_population                     utils.py:116-125, ga.py:13-53
   replay(individual) / repeat_upsample                         pickle_inspector.py:1-12, main.py:115-125, utils.py:156-168
   cross_play(toolbox, a, b)                                    no counterpart: main.evaluate's schedule as any match list
-  render_recorded / replay_selfplay                            main.evaluate(render=True) for recorded fused games
+  render_recorded / replay_selfplay                            main.evaluate(render=True) for recorded games
 Every call lands in libngp.so's CUDA kernels through Engine; nothing here computes on the CPU except argument
 marshalling (individuals are rows of device tensors instead of Python lists)."""
 from __future__ import annotations
@@ -193,8 +193,9 @@ class Toolbox:
 
 
 def cross_play(toolbox: Toolbox, a: torch.Tensor, b: torch.Tensor):
-    """Every row of `a` on the right against every row of `b` on the left, one fused launch (ngp_play_matches over
-    cat([a, b]), the toolbox's seed and generation): a cross table such as this generation's champions against earlier
+    """Every row of `a` on the right against every row of `b` on the left, as one match list (Engine.play_matches over
+    cat([a, b]), the toolbox's seed and generation): one fused launch when the network fits the fused rollout, the per-frame
+    driver (ngp_play_matches_stepwise) for wider networks.  A cross table such as this generation's champions against earlier
     generations' champions.  Returns dict(reward f64[A][B] of the right player, score i32[A][B][2] = (left, right) points,
     frames i32[A][B]); match (i, j) is list entry i * B + j."""
     eng = toolbox.engine
@@ -426,7 +427,8 @@ def branch(toolbox: Toolbox, genomes: torch.Tensor, right, left, m: int, t: int,
     """A counterfactual branch of list match m (right[m] vs left[m], a genome row or OPP_* code; lists as play_matches takes
     them): the game is played to env.step t and captured there (Engine.play_matches_states), then continued from that exact
     position with new_right / new_left (None = the same players; a robot match stays a robot match) under the same fall-back
-    key (key = None: m, the match's index in the list) and the toolbox's seed and generation.  The first resumed env.step
+    key (key = None: m, the match's index in the list) and the toolbox's seed and generation.  Both calls run on the driver
+    Engine.play_matches_states picks (the fused rollout, or the per-frame driver for wide networks).  The first resumed env.step
     still uses the decisions the old players took on frame t.  Returns record_matches' dict for the one branched match:
     rewards, frames, scores (the whole episode's), frames_total (the frames emulated after t), left, record (entries below
     t are the original game's) -- plus `capture`, the state at t, and `start_states` = (capture, t) for render_recorded.
@@ -459,8 +461,8 @@ def branch(toolbox: Toolbox, genomes: torch.Tensor, right, left, m: int, t: int,
 
 def replay_selfplay(toolbox: Toolbox, genomes: torch.Tensor, g: int, k: int, upsample=(4, 4)):
     """Round-robin game k of genome g, played and rendered exactly as Engine.evaluate plays it under SCHEDULE_ROUND_ROBIN
-    with the toolbox's seed and generation: one record_matches call (right = g, left = (g + k + 1) % n, key = g * games + k),
-    then render_recorded.  Returns replay's dict: frames u8[T, 210*k, 160*l, 3], reward, steps, score = (left, right)."""
+    with the toolbox's seed and generation: one record_matches call (right = g, left = (g + k + 1) % n, key = g * games + k;
+    the fused rollout, or the per-frame driver for wide networks), then render_recorded.  Returns replay's dict: frames u8[T, 210*k, 160*l, 3], reward, steps, score = (left, right)."""
     eng, cfg = toolbox.engine, toolbox.config
     dev = eng.device
     n, games = genomes.shape[0], cfg.GAMES_TO_PLAY
