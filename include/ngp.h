@@ -273,6 +273,61 @@ int ngp_play_matches_stepwise(ngp_handle *h, const float *genomes, int32_t n_gen
                               uint64_t seed, uint64_t generation, double *rewards, int32_t *frames, int32_t *scores,
                               uint64_t *frames_total, void *stream);
 
+/* ---- match sessions: a match list that the caller advances one env.step at a time, with seats whose decisions the caller
+ * supplies.  The reference's perform_episode (main.py:69-112) takes any object with .run(vec6) -> [up, down] as a player
+ * (a NeuralNetwork, a dumb_ais bot, human_control.HumanInput: SURVEY.md section 8b); NGP_PLAYER_EXTERNAL is such a player
+ * outside the library -- a policy of another framework, a person, any controller.
+ *
+ * NGP_PLAYER_EXTERNAL, as right[m] or left[m] of a session's list, is a model in perform_episode's sense: its decision is
+ * consumed only on the frames on which get_actions calls the models (ball and both paddles found); on other frames the
+ * fall-back random or none action is played with the usual Philox key; the bounds clamp applies to it; timeout, termination,
+ * reward, scores, records and captures are what ngp_play_matches_stepwise computes.  An external right seat may face a genome
+ * row, an NGP_OPP_* code or NGP_OPP_ROBOT; an external left seat a genome row or an external right seat.  Only the session
+ * entry points accept the code: every other match-list entry point refuses it. */
+enum { NGP_PLAYER_EXTERNAL = -4 };
+/* bits of a session's per-match flags */
+enum { NGP_SESSION_NEED = 1,            /* the next step consumes this match's external decisions */
+       NGP_SESSION_DONE = 2,            /* the match has ended (for good: the bit stays set) */
+       NGP_SESSION_EMULATOR_ERROR = 4 };/* it ended on an emulator error */
+
+typedef struct ngp_session ngp_session;
+
+/* Begins a session over a match list and plays its env.step 0.
+ * genomes .. generation, rewards, frames and scores mean what they mean in ngp_play_matches_stepwise (networks of any width;
+ * genomes may be NULL with n_genomes == 0 when no seat names a row).  The refusals are that call's (NGP_ERR_INVALID, nothing
+ * written, no session created), with NGP_PLAYER_EXTERNAL allowed as above, after the same single read-back of the list check.
+ * obs: device f32[n_matches][2][6] and flags: device u8[n_matches], written by begin and by every step:
+ *   flags[m]: NGP_SESSION_* bits.  On a step that sets NEED, obs[m][0] (left seat) and obs[m][1] (right seat) of an external seat
+ *   hold utils.inference's vector (utils.py:139-153) exactly as a genome in that seat would get it, the left seat's x-mirrored as
+ *   in self-play; the rows of the other seats are unspecified.
+ * scores (may be NULL) holds the (left, right) points of the last decided frame after every step, the final points at the end.
+ * The session owns its per-match state, MLP rows and counters: other calls on the handle between two steps (ngp_evaluate,
+ * ngp_play_matches*, another session) do not disturb it.  Wide networks share the handle's packed weight copy
+ * (ngp_mlp_prepare): a step re-packs the session's genome table when another call replaced it.
+ * Every device array passed to begin is read or written by later steps and must stay valid and unchanged (genomes, lists, mult,
+ * key, states) until ngp_session_end.  *out receives the session. */
+int ngp_session_begin(ngp_handle *h, const float *genomes, int32_t n_genomes,
+                      const int32_t *right, const int32_t *left, const double *mult, const int32_t *key, int32_t n_matches,
+                      const ngp_game_state *states, int32_t n_states, const int32_t *start, int32_t fresh,
+                      int32_t max_record, ngp_frame_record *record, uint64_t seed, uint64_t generation,
+                      double *rewards, int32_t *frames, int32_t *scores, float *obs, uint8_t *flags,
+                      void *stream, ngp_session **out);
+/* One env.step of every running match: (1) the decisions of the frame just observed, the external seats' from actions (device
+ * u8[n_matches][2], (left, right) NGP_ACT_*; entries of other seats are ignored, a consumed value outside 0..2 is played as
+ * NGP_ACT_NONE and counted), (2) the record entry, the scores and, for a match that ends, its reward and frame count,
+ * (3) with capture (device ngp_game_state[n_matches], 16-byte aligned, or NULL) the state of every match still running --
+ * the state ngp_play_matches_states writes with capture_at[m] = its frame count at that point, (4) the env.step, (5) the wide
+ * MLP rows of the next decisions.  Neither synchronises, allocates nor reads back (a wide step after another call replaced the
+ * packed weights re-packs them first), so the caller's policy can run on the same stream between steps, and steps can be
+ * captured into a CUDA graph.  A step after every match has ended changes no output. */
+int ngp_session_step(ngp_session *s, const uint8_t *actions, float *obs, uint8_t *flags, ngp_game_state *capture, void *stream);
+/* Synchronises the stream.  *running (may be NULL) = the matches still running, *frames_total (may be NULL) = the env.steps
+ * emulated so far (ngp_play_matches_stepwise's *frames_total once every match has ended).  Returns NGP_ERR_EMULATOR if a
+ * match stopped on an emulator error, NGP_ERR_INVALID if out-of-range actions were consumed (the message has the count). */
+int ngp_session_status(ngp_session *s, int32_t *running, uint64_t *frames_total, void *stream);
+/* Frees the session (waits for its work first).  ngp_destroy ends every session still open on the handle. */
+int ngp_session_end(ngp_session *s);
+
 /* ---- K4: GA step.  Replaces toolbox.select / varAnd(mate, mutate) inside eaSimple
  * (ga.py:89-94, main.py:165-170; DEAP selTournament, cxBlend, mutGaussian).
  * Injected noise (all device, all optional = NULL -> Philox(seed, generation)). */

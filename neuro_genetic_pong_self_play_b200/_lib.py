@@ -14,6 +14,10 @@ SCHEDULE_REFERENCE, SCHEDULE_ROUND_ROBIN = 0, 1
 CORE_INTERPRETER, CORE_TRANSLATED = 0, 1
 # left-player codes of ngp_play_matches that are not genome rows (include/ngp.h NGP_OPP_*)
 OPP_HARDCODED, OPP_SCORE_HARDCODED, OPP_ROBOT = -1, -2, -3
+# a seat of a match session whose decisions the caller supplies (include/ngp.h NGP_PLAYER_EXTERNAL)
+PLAYER_EXTERNAL = -4
+# bits of a match session's per-match flags (include/ngp.h NGP_SESSION_*)
+SESSION_NEED, SESSION_DONE, SESSION_EMULATOR_ERROR = 1, 2, 4
 # sizeof(ngp_frame_record) (include/ngp.h): one recorded frame of ngp_record_matches
 NGP_FRAME_RECORD_BYTES = 32
 # sizeof(ngp_game_state) (include/ngp.h): one save state of a game
@@ -28,7 +32,7 @@ EXPORTS = [
     "ngp_config_size", "ngp_set_option", "ngp_select", "ngp_mate", "ngp_mutate", "ngp_hof_update", "ngp_exchange_bytes",
     "ngp_pack_elites", "ngp_unpack_elites", "ngp_mlp_prepare", "ngp_mlp_forward_prepared",
     "ngp_play_matches", "ngp_record_matches", "ngp_env_get_state", "ngp_env_set_state", "ngp_play_matches_states",
-    "ngp_play_matches_stepwise",
+    "ngp_play_matches_stepwise", "ngp_session_begin", "ngp_session_step", "ngp_session_status", "ngp_session_end",
 ]
 
 
@@ -98,6 +102,11 @@ def load(build_if_missing: bool = True):
     L.ngp_play_matches_states.argtypes = [vp, vp, i32, vp, vp, vp, vp, i32, vp, i32, vp, i32, vp, vp, i32, vp, u64, u64, vp, vp, vp,
                                           ctypes.POINTER(u64), vp]
     L.ngp_play_matches_stepwise.argtypes = L.ngp_play_matches_states.argtypes
+    L.ngp_session_begin.argtypes = [vp, vp, i32, vp, vp, vp, vp, i32, vp, i32, vp, i32, i32, vp, u64, u64, vp, vp, vp, vp, vp, vp,
+                                    ctypes.POINTER(vp)]
+    L.ngp_session_step.argtypes = [vp, vp, vp, vp, vp, vp]
+    L.ngp_session_status.argtypes = [vp, ctypes.POINTER(i32), ctypes.POINTER(u64), vp]
+    L.ngp_session_end.argtypes = [vp]
     L.ngp_evaluate_host.argtypes = [vp, vp, i32, vp, vp, i32, u64, u64, vp, ctypes.POINTER(u64)]
     L.ngp_ga_step.argtypes = [vp, vp, vp, i32, u64, u64, ctypes.POINTER(NgpNoise), vp, vp, vp, vp, vp]
     L.ngp_init_population.argtypes = [vp, vp, i32, u64, vp]

@@ -209,13 +209,16 @@ __host__ __device__ __forceinline__ int validate(const ngp_game_state *st, uint6
 // The argument check of the match-list entry points for match m (match_check_kernel, ngp_core.cu): the number of faults of
 // entry m -- a right row outside [0, n_genomes), a left entry that is neither a row nor an NGP_OPP_* code, a negative key, a
 // negative capture frame, a start index outside [-1, n_states), a start state whose players value disagrees with left[m].
-// Start states themselves are validated once each by the caller.
+// Start states themselves are validated once each by the caller.  external (match sessions only): NGP_PLAYER_EXTERNAL is a
+// valid entry on either side.
 __host__ __device__ __forceinline__ int match_entry_faults(int m, const int32_t *right, const int32_t *left, int n_genomes,
                                                            const int32_t *key, const int32_t *capture_at, const int32_t *start,
-                                                           const ngp_game_state *states, int n_states)
+                                                           const ngp_game_state *states, int n_states, bool external = false)
 {
     const int r = right[m], l = left[m];
-    int c = (r < 0 || r >= n_genomes) + (l < NGP_OPP_ROBOT || l >= n_genomes) + (key && key[m] < 0) + (capture_at && capture_at[m] < 0);
+    const bool xr = external && r == NGP_PLAYER_EXTERNAL, xl = external && l == NGP_PLAYER_EXTERNAL;
+    int c = (!xr && (r < 0 || r >= n_genomes)) + (!xl && (l < NGP_OPP_ROBOT || l >= n_genomes)) + (key && key[m] < 0) +
+            (capture_at && capture_at[m] < 0);
     if (start) {
         const int k = start[m];
         if (k < -1 || k >= n_states) ++c;

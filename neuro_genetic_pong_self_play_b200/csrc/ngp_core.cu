@@ -154,6 +154,9 @@ __global__ void env_digest_kernel(const Snapshot *envs, int n, uint32_t *out)
 int ngp_evaluate_stepwise(ngp_handle *h, const RolloutParams &p, cudaStream_t st);
 int ngp_list_layout_count(ngp_handle *h, const int32_t *right, const int32_t *left, int n_matches, int n_genomes, cudaStream_t st);
 int ngp_play_list_stepwise(ngp_handle *h, const RolloutParams &p, const roll::RecordArgs &rec, int n_genomes, bool wide, cudaStream_t st);
+// ngp_session.cu
+int ngp_session_start(ngp_handle *h, const RolloutParams &p, const roll::RecordArgs &rec, int n_genomes, bool wide, float *obs,
+                      uint8_t *flags, cudaStream_t st, ngp_session **out);
 
 // fitness[g] = sum(rewards[g][:]) / games, summed in game order (main.py:65)
 __global__ void fitness_reduce_kernel(const double *__restrict__ rewards, int n, int games, double *__restrict__ fitness)
@@ -166,14 +169,14 @@ __global__ void fitness_reduce_kernel(const double *__restrict__ rewards, int n,
 }
 
 // the argument check of the match-list entry points: counts the faults of every match entry (gs::match_entry_faults) and the
-// start states that fail validation
+// start states that fail validation; external: a match session's list (NGP_PLAYER_EXTERNAL allowed)
 __global__ void match_check_kernel(const int32_t *__restrict__ right, const int32_t *__restrict__ left, const int32_t *__restrict__ key,
                                    int n, int n_genomes, const int32_t *__restrict__ capture_at, const int32_t *__restrict__ start,
-                                   const ngp_game_state *__restrict__ states, int n_states, uint64_t cart, unsigned long long *bad)
+                                   const ngp_game_state *__restrict__ states, int n_states, uint64_t cart, int external, unsigned long long *bad)
 {
     unsigned long long c = 0;
     for (int m = blockIdx.x * blockDim.x + threadIdx.x; m < n; m += gridDim.x * blockDim.x)
-        c += gs::match_entry_faults(m, right, left, n_genomes, key, capture_at, start, states, n_states);
+        c += gs::match_entry_faults(m, right, left, n_genomes, key, capture_at, start, states, n_states, external != 0);
     for (int k = blockIdx.x * blockDim.x + threadIdx.x; k < n_states; k += gridDim.x * blockDim.x) c += gs::validate(states + k, cart) == 0;
     if (c) atomicAdd(bad, c);
 }
@@ -292,6 +295,7 @@ extern "C" int ngp_destroy(ngp_handle *h)
 {
     if (!h) return NGP_OK;
     cudaSetDevice(h->device);
+    while (!h->sessions.empty()) ngp_session_end(h->sessions.back());
     delete h;
     return NGP_OK;
 }
@@ -548,13 +552,17 @@ extern "C" int ngp_evaluate(ngp_handle *h, const float *genomes, int32_t n, cons
 
 // ngp_play_matches; ngp_record_matches and ngp_play_matches_states when `rec` is set (its pointers' alignment and the record
 // length already checked; n_states = the length of rec->states).  stepwise (ngp_play_matches_stepwise): the per-frame driver
-// plays the list (ngp_stepwise.cu) instead of the fused rollout; everything up to the one read-back is shared.
+// plays the list (ngp_stepwise.cu) instead of the fused rollout; everything up to the one read-back is shared.  session
+// (ngp_session_begin, stepwise): the list may name NGP_PLAYER_EXTERNAL and no genome at all; after the check a match session
+// begins (ngp_session.cu) with obs and flags.
 static int play_match_list(ngp_handle *h, const float *genomes, int32_t n_genomes, const int32_t *right, const int32_t *left,
                            const double *mult, int32_t n_matches, uint64_t seed, uint64_t generation, double *rewards, int32_t *frames,
                            int32_t *scores, uint64_t *frames_total, cudaStream_t st, const roll::RecordArgs *rec, int32_t n_states,
-                           const char *who, bool stepwise = false)
+                           const char *who, bool stepwise = false, ngp_session **session = nullptr, float *obs = nullptr,
+                           uint8_t *flags = nullptr)
 {
-    if (!(h && genomes && right && left && rewards && n_genomes > 0 && n_matches > 0)) {
+    const bool table = session && !genomes && n_genomes == 0 ? true : genomes && n_genomes > 0;       // a session may have no genome table
+    if (!(h && table && right && left && rewards && n_matches > 0)) {
         ngp_set_error("%s: bad arguments", who);
         return NGP_ERR_INVALID;
     }
@@ -577,17 +585,17 @@ static int play_match_list(ngp_handle *h, const float *genomes, int32_t n_genome
     const roll::RecordArgs none = {};
     const roll::RecordArgs &ra = rec ? *rec : none;
     NGP_CUDA(cudaSetDevice(h->device));
-    if (!frames) NGP_CUDA(h->d_frames.ensure(n_matches));
+    if (!frames && !session) NGP_CUDA(h->d_frames.ensure(n_matches));
     NGP_CUDA(cudaMemsetAsync(h->d_counters.p, 0, 8 * sizeof(unsigned long long), st));
     // the lists and states live on the device: count their bad entries there and refuse before anything is played
     const long long check_items = std::max<long long>(n_matches, n_states);
     const int check_blocks = (int)std::min<long long>((check_items + 255) / 256, 4ll * h->sm_count);
     match_check_kernel<<<check_blocks, 256, 0, st>>>(right, left, ra.key, n_matches, n_genomes, ra.capture_at, ra.start, ra.states, n_states,
-                                                     h->cart_hash, h->d_counters.p + 3);
+                                                     h->cart_hash, session ? 1 : 0, h->d_counters.p + 3);
     h->launches++;
     NGP_CUDA(cudaGetLastError());
     // the stepwise driver's chunk counts of wide networks (d_counters[8, 14)) come back with the fault count
-    const bool layout = stepwise && wide;
+    const bool layout = stepwise && wide && n_genomes > 0;
     if (layout) {
         const int rc = ngp_list_layout_count(h, right, left, n_matches, n_genomes, st);
         if (rc != NGP_OK) return rc;
@@ -607,7 +615,8 @@ static int play_match_list(ngp_handle *h, const float *genomes, int32_t n_genome
     RolloutParams p = rollout_params(h, genomes, seed, generation);
     p.n = n_matches; p.games = 1;
     p.match_right = right; p.match_left = left; p.match_mult = mult;
-    p.rewards = rewards; p.frames = frames ? frames : h->d_frames.p; p.scores = scores;
+    p.rewards = rewards; p.frames = frames ? frames : session ? nullptr : h->d_frames.p; p.scores = scores;     // a session owns its own
+    if (session) return ngp_session_start(h, p, ra, n_genomes, wide, obs, flags, st, session);
     if (stepwise) {
         const int rc = ngp_play_list_stepwise(h, p, ra, n_genomes, wide, st);
         if (rc != NGP_OK) return rc;
@@ -688,6 +697,27 @@ extern "C" int ngp_play_matches_stepwise(ngp_handle *h, const float *genomes, in
     return play_matches_states(h, genomes, n_genomes, right, left, mult, key, n_matches, states, n_states, start, fresh, capture_at,
                                capture, max_record, record, seed, generation, rewards, frames, scores, frames_total, stream,
                                "ngp_play_matches_stepwise", true);
+}
+
+extern "C" int ngp_session_begin(ngp_handle *h, const float *genomes, int32_t n_genomes, const int32_t *right, const int32_t *left,
+                                 const double *mult, const int32_t *key, int32_t n_matches, const ngp_game_state *states, int32_t n_states,
+                                 const int32_t *start, int32_t fresh, int32_t max_record, ngp_frame_record *record, uint64_t seed,
+                                 uint64_t generation, double *rewards, int32_t *frames, int32_t *scores, float *obs, uint8_t *flags,
+                                 void *stream, ngp_session **out)
+{
+    NGP_REQUIRE(h && out && obs && flags, "ngp_session_begin: bad arguments (handle, obs, flags and out are required)");
+    *out = nullptr;
+    NGP_REQUIRE(!record || max_record >= 1, "ngp_session_begin: a record needs max_record >= 1");
+    NGP_REQUIRE(((uintptr_t)record & 15) == 0, "ngp_session_begin: the record buffer must be 16-byte aligned");
+    NGP_REQUIRE(n_states >= 0 && (n_states == 0 || states), "ngp_session_begin: n_states states needed");
+    NGP_REQUIRE(((uintptr_t)states & 15) == 0, "ngp_session_begin: state arrays must be 16-byte aligned");
+    NGP_REQUIRE(((uintptr_t)obs & 3) == 0, "ngp_session_begin: obs must be 4-byte aligned");
+    roll::RecordArgs rec = {};
+    rec.record = record; rec.key = key; rec.max_record = record ? max_record : 0;
+    rec.fresh = fresh ? 1 : 0; rec.states = states; rec.start = start;
+    rec.cart = h->cart_hash;
+    return play_match_list(h, genomes, n_genomes, right, left, mult, n_matches, seed, generation, rewards, frames, scores, nullptr,
+                           (cudaStream_t)stream, &rec, n_states, "ngp_session_begin", true, out, obs, flags);
 }
 
 extern "C" int ngp_profile_enable(ngp_handle *h, int32_t on)

@@ -92,6 +92,8 @@ struct ngp_handle {
     int profile_on;
     std::vector<std::pair<cudaEvent_t, cudaEvent_t>> prof_events;
     int prof_used;
+    // match sessions open on this handle (ngp_session.cu); ngp_destroy ends them
+    std::vector<ngp_session *> sessions;
 
     ~ngp_handle()
     {

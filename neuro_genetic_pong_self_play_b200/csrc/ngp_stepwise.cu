@@ -25,14 +25,6 @@ using roll::RolloutParams;
 
 namespace {
 
-__device__ __forceinline__ void load_tables_cta(Tables &dst, const Tables *__restrict__ src)
-{
-    const uint32_t *s = reinterpret_cast<const uint32_t *>(src);
-    uint32_t *d = reinterpret_cast<uint32_t *>(&dst);
-    for (unsigned i = threadIdx.x; i < sizeof(Tables) / 4; i += blockDim.x) d[i] = s[i];
-    __syncthreads();
-}
-
 // rows of the MLP batch: round-robin -> x[n][2*games][6]: genome g's row k = its game k as the right player, row games+k = the
 // game it plays on the left (environment ((g-k-1) mod n, k)); reference schedule -> right rows x[n][games][6], hall-of-fame
 // opponents one row each in a second batch x_hof[3n][1][6] over the gathered opponent genomes.
@@ -67,14 +59,6 @@ __global__ void step_gather_opponents_kernel(RolloutParams p, float *__restrict_
     for (int i = threadIdx.x; i < p.G; i += blockDim.x) dst[i] = src ? src[i] : 0.f;
 }
 
-__device__ __forceinline__ void write_inference_row(float *__restrict__ x, const double ball[2], const double last[2], double me_row, double enemy_row)
-{
-    // utils.inference (utils.py:139-153): ball x, ball y, last x, last y, my row, enemy row, all divided by 160
-    x[0] = (float)__ddiv_rn(ball[1], 160.0); x[1] = (float)__ddiv_rn(ball[0], 160.0);
-    x[2] = (float)__ddiv_rn(last[1], 160.0); x[3] = (float)__ddiv_rn(last[0], 160.0);
-    x[4] = (float)__ddiv_rn(me_row, 160.0);  x[5] = (float)__ddiv_rn(enemy_row, 160.0);
-}
-
 template <int CORE>
 __global__ void __launch_bounds__(32) step_frame_kernel(RolloutParams p, StepEnv *envs, int total, float *__restrict__ x, float *__restrict__ x_hof)
 {
@@ -85,6 +69,8 @@ __global__ void __launch_bounds__(32) step_frame_kernel(RolloutParams p, StepEnv
     if (e >= total) return;
     StepEnv &v = envs[e];
     if (v.done) return;
+    // the body of step_env_frame (stepwise.cuh), kept inline here: through the helper the compiler inlines the frame differently
+    // (168 registers instead of 128 for the translated core), and this kernel stays as the wide ngp_evaluate has measured it
     Ram ram{&ram_smem[threadIdx.x]};
     Chip s; CpuRegs r;
     roll::load_snapshot(&v.snap, s, r, ram);

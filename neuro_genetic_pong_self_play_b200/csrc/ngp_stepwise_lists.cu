@@ -1,5 +1,5 @@
 // ngp_stepwise_lists.cu -- ngp_play_matches_stepwise: a match list (ngp_play_matches_states' arguments) on the per-frame driver of
-// wide ngp_evaluate (ngp_stepwise.cu), for networks of any width.  Environment m is match m, planned from the lists by
+// wide ngp_evaluate (ngp_stepwise.cu), for networks of any width.  Match sessions (ngp_session.cu) play lists on the same pieces.  Environment m is match m, planned from the lists by
 // roll::plan_env, started from a save state when asked (list_begin_kernel), stepped by ngp_evaluate's frame kernel
 // (ngp_step_frame), decided, recorded and captured by list_decide_kernel.  Wide networks' MLP rows are grouped by genome into
 // chunks of T rows (the layout kernels below) and run by ngp_mlp_forward_chunks.  A translation unit of its own, so that wide
@@ -39,9 +39,10 @@ static __device__ __noinline__ void capture_env(const RecordArgs &rec, StepEnv &
 // as rollout_kernel does after episode_begin.  With `base`, each MLP side takes the next free row of its genome's chunks
 // (genome g's rows are base[g] * T ..; cursor[g] counts the rows handed out): the ranks depend on the atomics' order, the
 // results do not, since every row is computed on its own.  Without, no MLP batch runs: match e writes its rows 2e, 2e + 1
-// (which nothing reads), so that wide ngp_evaluate's frame kernel serves both drivers unchanged.
+// (which nothing reads), so that wide ngp_evaluate's frame kernel serves both drivers unchanged.  ext (a match session): the
+// EXT_* bits of match e; an external seat takes no MLP row.
 __global__ void list_begin_kernel(RolloutParams p, RecordArgs rec, StepEnv *envs, int total, const int32_t *__restrict__ base,
-                                  int32_t *__restrict__ cursor, int T)
+                                  int32_t *__restrict__ cursor, int T, const uint8_t *__restrict__ ext)
 {
     const int e = blockIdx.x * blockDim.x + threadIdx.x;
     if (e >= total) return;
@@ -60,10 +61,11 @@ __global__ void list_begin_kernel(RolloutParams p, RecordArgs rec, StepEnv *envs
     v.left_act = (uint8_t)ep.left_act; v.right_act = (uint8_t)ep.right_act;
     v.last_ball[0] = ep.last_ball[0]; v.last_ball[1] = ep.last_ball[1];
     v.state = pl.state; v.left_kind = pl.left_kind; v.mult = pl.mult;
+    v.ext = ext ? ext[e] : 0;
     if (base) {
         const int r = p.match_right[e], l = p.match_left[e];
-        v.right_row = base[r] * T + atomicAdd(&cursor[r], 1);
-        v.left_row = l >= 0 ? base[l] * T + atomicAdd(&cursor[l], 1) : -1;
+        v.right_row = v.ext & EXT_RIGHT ? -1 : base[r] * T + atomicAdd(&cursor[r], 1);
+        v.left_row = l >= 0 && !(v.ext & EXT_LEFT) ? base[l] * T + atomicAdd(&cursor[l], 1) : -1;
     } else {
         v.right_row = 2 * e; v.left_row = 2 * e + 1;
     }
@@ -72,12 +74,16 @@ __global__ void list_begin_kernel(RolloutParams p, RecordArgs rec, StepEnv *envs
 
 // step_decide_kernel (ngp_stepwise.cu) for a match list: the fall-back key is rec.key[e] (or e), rec.record gets entry
 // frame - 1 after the clamp and the timeout update (the fields of roll::record_frame), a running episode is captured when its
-// frame reaches rec.capture_at[e], and p.scores gets the last scores.  Left MLP rows are in `act` too.  act == NULL: networks the fused rollout takes, run here in FP64 by
-// roll::run_policy as the fused rollout runs them.
-__global__ void list_decide_kernel(RolloutParams p, RecordArgs rec, StepEnv *envs, int total, const uint8_t *__restrict__ act)
+// frame reaches rec.capture_at[e], and p.scores gets the last scores.  Left MLP rows are in `act` too.  act == NULL: networks the
+// fused rollout takes, run here in FP64 by roll::run_policy as the fused rollout runs them.
+// A match session's step (ss.actions set): an external seat (v.ext) plays ss.actions[e][0] (left) or [1] (right) on the frames on
+// which a model is called, a value outside 0..2 as NGP_ACT_NONE, counted in p.counters[4]; p.scores gets every frame's scores;
+// with ss.capture_all every match still running is captured.
+__global__ void list_decide_kernel(RolloutParams p, RecordArgs rec, StepEnv *envs, int total, const uint8_t *__restrict__ act, SessionStep ss)
 {
     const int e = blockIdx.x * blockDim.x + threadIdx.x;
     bool stepped = false, finished = false;
+    int bad = 0;
     if (e < total && !envs[e].done) {
         StepEnv &v = envs[e];
         stepped = true;
@@ -86,20 +92,21 @@ __global__ void list_decide_kernel(RolloutParams p, RecordArgs rec, StepEnv *env
         // ---- get_actions (main.py:138-154) ----
         int left_act = pol::ACT_NONE, right_act = pol::ACT_NONE;
         if (vb) {
-            if (!act && vl && vr) {
-                const roll::EnvPlan pl = roll::plan_env(p, e);
+            if (vl && vr) {
                 const double lb[2] = {v.have_last_ball ? v.last_ball[0] : v.loc[0][0], v.have_last_ball ? v.last_ball[1] : v.loc[0][1]};
                 const double fball[2] = {v.loc[0][0], __dsub_rn(160.0, v.loc[0][1])}, flast[2] = {lb[0], __dsub_rn(160.0, lb[1])};
-                left_act = roll::run_policy(p.shape, v.left_kind, pl.left_genome, fball, flast, v.loc[1][0], v.loc[2][0], s1, s2);
-                right_act = roll::run_policy(p.shape, pol::KIND_MLP, pl.right_genome, v.loc[0], lb, v.loc[2][0], v.loc[1][0], s1, s2);
-            } else if (vl && vr) {
-                right_act = act[v.right_row];
-                if (v.left_kind == pol::KIND_MLP) left_act = act[v.left_row];
-                else {
-                    const double lb[2] = {v.have_last_ball ? v.last_ball[0] : v.loc[0][0], v.have_last_ball ? v.last_ball[1] : v.loc[0][1]};
-                    const double fball[2] = {v.loc[0][0], __dsub_rn(160.0, v.loc[0][1])}, flast[2] = {lb[0], __dsub_rn(160.0, lb[1])};
-                    left_act = roll::run_policy(p.shape, v.left_kind, nullptr, fball, flast, v.loc[1][0], v.loc[2][0], s1, s2);
-                }
+                const float *lg = nullptr, *rg = nullptr;
+                if (!act) { const roll::EnvPlan pl = roll::plan_env(p, e); lg = pl.left_genome; rg = pl.right_genome; }
+                if (v.ext & EXT_LEFT) {
+                    left_act = ss.actions[2 * e];
+                    if (left_act > pol::ACT_DOWN) { left_act = pol::ACT_NONE; ++bad; }
+                } else if (act && v.left_kind == pol::KIND_MLP) left_act = act[v.left_row];
+                else left_act = roll::run_policy(p.shape, v.left_kind, lg, fball, flast, v.loc[1][0], v.loc[2][0], s1, s2);
+                if (v.ext & EXT_RIGHT) {
+                    right_act = ss.actions[2 * e + 1];
+                    if (right_act > pol::ACT_DOWN) { right_act = pol::ACT_NONE; ++bad; }
+                } else if (act) right_act = act[v.right_row];
+                else right_act = roll::run_policy(p.shape, pol::KIND_MLP, rg, v.loc[0], lb, v.loc[2][0], v.loc[1][0], s1, s2);
             } else {            // same deviation as the fused path: the reference raises TypeError here; the random action is kept
                 const uint32_t key = rec.key ? (uint32_t)rec.key[e] : (uint32_t)e;
                 left_act = pol::random_action_bit(p.seed, p.generation, key, (uint32_t)v.frame, 0) ? pol::ACT_DOWN : pol::ACT_UP;
@@ -141,14 +148,17 @@ __global__ void list_decide_kernel(RolloutParams p, RecordArgs rec, StepEnv *env
             roll::record_store(rec, e, v.frame - 1, 1, w[4], w[5],
                                vbits | (uint32_t)s1 << 8 | (uint32_t)s2 << 16 | (uint32_t)(v.left_act | v.right_act << 2) << 24, (uint32_t)v.timeout);
         }
-        if (finished) {
-            if (p.scores) { p.scores[2 * e] = s1; p.scores[2 * e + 1] = s2; }
-        } else if (rec.capture_at && v.frame == rec.capture_at[e]) capture_env(rec, v, e);
+        if (p.scores && (finished || ss.actions)) { p.scores[2 * e] = s1; p.scores[2 * e + 1] = s2; }
+        if (!finished && (ss.capture_all || (rec.capture_at && v.frame == rec.capture_at[e]))) capture_env(rec, v, e);
     }
     const unsigned m_step = __ballot_sync(0xFFFFFFFFu, stepped), m_fin = __ballot_sync(0xFFFFFFFFu, finished);
     if ((threadIdx.x & 31) == 0) {
         if (m_step) atomicAdd(&p.counters[1], (unsigned long long)__popc(m_step));
         if (m_fin) atomicAdd(&p.counters[3], (unsigned long long)__popc(m_fin));
+    }
+    if (ss.actions) {
+        bad = __reduce_add_sync(0xFFFFFFFFu, bad);
+        if ((threadIdx.x & 31) == 0 && bad) atomicAdd(&p.counters[4], (unsigned long long)bad);
     }
 }
 
@@ -218,19 +228,16 @@ int ngp_list_layout_count(ngp_handle *h, const int32_t *right, const int32_t *le
     return NGP_OK;
 }
 
-// ngp_play_matches_stepwise after the list check: p and rec are filled in (p.n = matches, p.games = 1).  Wide networks use the
-// counts ngp_list_layout_count left in h_counters[8 .. 14).  Synchronises the stream every CHECK_EVERY frames and at the end;
-// h_counters[1], [2] then hold the frames and the emulator errors.
-int ngp_play_list_stepwise(ngp_handle *h, const RolloutParams &p, const RecordArgs &rec, int n_genomes, bool wide, cudaStream_t st)
+int ngp_list_begin(ngp_handle *h, const RolloutParams &p, const RecordArgs &rec, int n_genomes, bool wide, const uint8_t *ext,
+                   Buffer<uint8_t> &envs_buf, Buffer<float> &x_buf, Buffer<uint8_t> &act_buf, Buffer<int32_t> &chunk, int *T_out,
+                   long long *C_out, cudaStream_t st)
 {
     const int total = p.n;
-    NGP_CUDA(h->step_envs.ensure((size_t)total * sizeof(StepEnv)));
-    StepEnv *envs = reinterpret_cast<StepEnv *>(h->step_envs.p);
-    float *x = nullptr;
-    uint8_t *act = nullptr;
+    NGP_CUDA(envs_buf.ensure((size_t)total * sizeof(StepEnv)));
+    StepEnv *envs = reinterpret_cast<StepEnv *>(envs_buf.p);
     int T = 0;
     long long C = 0;
-    if (wide) {
+    if (wide && n_genomes > 0) {
         // T: the smallest power of two in [16, 128] not below the mean rows per genome with rows (a heuristic, not measured)
         const unsigned long long *stats = h->h_counters.p + 8, rows = stats[1], used = stats[0];
         int ti = 1;
@@ -241,13 +248,15 @@ int ngp_play_list_stepwise(ngp_handle *h, const RolloutParams &p, const RecordAr
             ngp_set_error("ngp_play_matches_stepwise: %lld chunks of %d rows are too many", C, T);
             return NGP_ERR_UNSUPPORTED;
         }
+    }
+    *T_out = T; *C_out = C;
+    if (C > 0) {
         int32_t *count = h->list_genome.p, *nchunk = count + n_genomes, *base = nchunk + n_genomes;
-        NGP_CUDA(h->list_chunk.ensure((size_t)C));
-        NGP_CUDA(h->step_x.ensure((size_t)C * T * 6));
-        NGP_CUDA(h->step_act.ensure((size_t)C * T));
-        x = h->step_x.p; act = h->step_act.p;
-        NGP_CUDA(cudaMemsetAsync(x, 0, (size_t)C * T * 6 * sizeof(float), st));     // padding rows are computed, never read: keep them finite
-        NGP_CUDA(cudaMemsetAsync(act, 0, (size_t)C * T, st));
+        NGP_CUDA(chunk.ensure((size_t)C));
+        NGP_CUDA(x_buf.ensure((size_t)C * T * 6));
+        NGP_CUDA(act_buf.ensure((size_t)C * T));
+        NGP_CUDA(cudaMemsetAsync(x_buf.p, 0, (size_t)C * T * 6 * sizeof(float), st));     // padding rows are computed, never read: keep them finite
+        NGP_CUDA(cudaMemsetAsync(act_buf.p, 0, (size_t)C * T, st));
         const int gb = (n_genomes + 255) / 256;
         list_chunks_kernel<<<gb, 256, 0, st>>>(count, n_genomes, T, nchunk);
         h->launches++;
@@ -257,31 +266,54 @@ int ngp_play_list_stepwise(ngp_handle *h, const RolloutParams &p, const RecordAr
         NGP_CUDA(h->list_scan_tmp.ensure(tmp_bytes));
         NGP_CUDA(cub::DeviceScan::ExclusiveSum(h->list_scan_tmp.p, tmp_bytes, nchunk, base, n_genomes, st));
         h->launches++;
-        list_fill_kernel<<<gb, 256, 0, st>>>(count, nchunk, base, n_genomes, h->list_chunk.p);
+        list_fill_kernel<<<gb, 256, 0, st>>>(count, nchunk, base, n_genomes, chunk.p);
         h->launches++;
         NGP_CUDA(cudaGetLastError());
-        list_begin_kernel<<<(total + 127) / 128, 128, 0, st>>>(p, rec, envs, total, base, count, T);
+        list_begin_kernel<<<(total + 127) / 128, 128, 0, st>>>(p, rec, envs, total, base, count, T, ext);
     } else {
-        NGP_CUDA(h->step_x.ensure((size_t)total * 2 * 6));
-        x = h->step_x.p;
-        list_begin_kernel<<<(total + 127) / 128, 128, 0, st>>>(p, rec, envs, total, nullptr, nullptr, 0);
+        list_begin_kernel<<<(total + 127) / 128, 128, 0, st>>>(p, rec, envs, total, nullptr, nullptr, 0, ext);
     }
     h->launches++;
     NGP_CUDA(cudaGetLastError());
+    return NGP_OK;
+}
+
+int ngp_list_decide(ngp_handle *h, const RolloutParams &p, const RecordArgs &rec, void *envs, int total, const uint8_t *act,
+                    const SessionStep &ss, cudaStream_t st)
+{
+    list_decide_kernel<<<(total + 127) / 128, 128, 0, st>>>(p, rec, static_cast<StepEnv *>(envs), total, act, ss);
+    h->launches++;
+    NGP_CUDA(cudaGetLastError());
+    return NGP_OK;
+}
+
+// ngp_play_matches_stepwise after the list check: p and rec are filled in (p.n = matches, p.games = 1).  Wide networks use the
+// counts ngp_list_layout_count left in h_counters[8 .. 14).  Synchronises the stream every CHECK_EVERY frames and at the end;
+// h_counters[1], [2] then hold the frames and the emulator errors.
+int ngp_play_list_stepwise(ngp_handle *h, const RolloutParams &p, const RecordArgs &rec, int n_genomes, bool wide, cudaStream_t st)
+{
+    const int total = p.n;
+    int T = 0;
+    long long C = 0;
+    int rc = ngp_list_begin(h, p, rec, n_genomes, wide, nullptr, h->step_envs, h->step_x, h->step_act, h->list_chunk, &T, &C, st);
+    if (rc != NGP_OK) return rc;
+    StepEnv *envs = reinterpret_cast<StepEnv *>(h->step_envs.p);
+    if (!wide) NGP_CUDA(h->step_x.ensure((size_t)total * 2 * 6));      // the rows 2e, 2e + 1 ngp_step_frame writes and nothing reads
+    float *x = h->step_x.p;
+    uint8_t *act = wide ? h->step_act.p : nullptr;
     if (wide) {     // the table's networks are built once per call and run every frame
-        const int rc = ngp_mlp_prepare(h, p.genomes, n_genomes, st);
+        rc = ngp_mlp_prepare(h, p.genomes, n_genomes, st);
         if (rc != NGP_OK) return rc;
     }
     for (long long frame = 1;; ++frame) {
-        int rc = ngp_step_frame(h, p, envs, total, x, x, st);
+        rc = ngp_step_frame(h, p, envs, total, x, x, st);
         if (rc != NGP_OK) return rc;
         if (wide) {
             rc = ngp_mlp_forward_chunks(h, p.genomes, h->list_chunk.p, x, (int)C, T, act, st);
             if (rc != NGP_OK) return rc;
         }
-        list_decide_kernel<<<(total + 127) / 128, 128, 0, st>>>(p, rec, envs, total, act);
-        h->launches++;
-        NGP_CUDA(cudaGetLastError());
+        rc = ngp_list_decide(h, p, rec, envs, total, act, SessionStep{}, st);
+        if (rc != NGP_OK) return rc;
         if (frame % CHECK_EVERY == 0) {
             NGP_CUDA(cudaMemcpyAsync(h->h_counters.p, h->d_counters.p, 4 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
             NGP_CUDA(cudaStreamSynchronize(st));
@@ -290,4 +322,3 @@ int ngp_play_list_stepwise(ngp_handle *h, const RolloutParams &p, const RecordAr
     }
     return NGP_OK;
 }
-

@@ -4,6 +4,7 @@ from __future__ import annotations
 
 import ctypes
 import os
+import weakref
 from typing import Optional
 
 import numpy as np
@@ -59,9 +60,12 @@ class Engine:
         self._h = h
         self.gene_size = int(self._L.ngp_gene_size(self._h))
         self._n_envs = 0
+        self._sessions = weakref.WeakSet()
 
     def close(self):
         if getattr(self, "_h", None):
+            for s in list(self._sessions):        # ngp_destroy ends them; their Python objects must not end them again
+                s._s = None
             self._L.ngp_destroy(self._h)
             self._h = None
 
@@ -308,6 +312,40 @@ class Engine:
             out["record"] = record_views(raw)
         return out
 
+    def session(self, genomes: torch.Tensor | None, right: torch.Tensor, left: torch.Tensor, mult: torch.Tensor | None = None,
+                key: torch.Tensor | None = None, states: torch.Tensor | None = None, start: torch.Tensor | None = None, fresh: bool = False,
+                max_record: int = 0, seed: int = 0, generation: int = 0) -> "MatchSession":
+        """A match session (ngp_session_begin): the list of play_matches_states (networks of any width, the per-frame driver),
+        advanced one env.step at a time by MatchSession.step.  right[m] / left[m] may be PLAYER_EXTERNAL: that seat's decisions
+        come from the caller on every step (a policy of another framework, a person, any controller), on the frames on which
+        perform_episode would call a model; everything else is play_matches_states' game.  genomes may be None when no seat
+        names a row.  Bad entries or states raise NgpError and no session is created.  The session plays env.step 0 here."""
+        if genomes is None:
+            genomes = torch.empty((0, self.gene_size), dtype=torch.float32, device=self.device)
+        out = self._match_list(genomes, right, left, mult=(mult, torch.float64), key=(key, torch.int32), start=(start, torch.int32))
+        m = right.shape[0]
+        n_states = 0
+        if states is not None:
+            self._check_tensor(states, torch.uint8, "states")
+            assert states.dim() == 2 and states.shape[1] == _lib.NGP_GAME_STATE_BYTES
+            n_states = states.shape[0]
+        raw = (torch.empty((m, int(max_record), _lib.NGP_FRAME_RECORD_BYTES), dtype=torch.uint8, device=self.device)
+               if max_record > 0 else None)
+        obs = torch.zeros((m, 2, 6), dtype=torch.float32, device=self.device)
+        flags = torch.zeros(m, dtype=torch.uint8, device=self.device)
+        out["scores"].zero_()
+        h = ctypes.c_void_p()
+        n_genomes = genomes.shape[0]
+        _lib.check(self._L.ngp_session_begin(
+            self._h, _p(genomes) if n_genomes else None, n_genomes, _p(right), _p(left), _p(mult), _p(key), m,
+            _p(states) if n_states else None, n_states, _p(start), 1 if fresh else 0, int(max_record), _p(raw), seed, generation,
+            _p(out["rewards"]), _p(out["frames"]), _p(out["scores"]), _p(obs), _p(flags), _stream(self.device), ctypes.byref(h)),
+            "ngp_session_begin")
+        sess = MatchSession(self, h, out, obs, flags, raw, left,
+                            keep=(genomes, right, left, mult, key, states, start))
+        self._sessions.add(sess)
+        return sess
+
     def evaluate_host(self, genomes: np.ndarray, hof_genomes: np.ndarray | None = None, hof_fitness: np.ndarray | None = None,
                       seed: int = 0, generation: int = 0):
         """Same, through host buffers (H2D of genomes and D2H of fitness inside the call)."""
@@ -414,3 +452,91 @@ class Engine:
         _lib.check(self._L.ngp_unpack_elites(self._h, _p(gathered), world, n_max, k_max, _p(fit), _p(eg), _p(ef), _stream(self.device)),
                    "ngp_unpack_elites")
         return fit, eg, ef
+
+
+class MatchSession:
+    """A match list advanced one env.step at a time (Engine.session; include/ngp.h ngp_session_*).  The tensors below are
+    persistent and rewritten in place by every step, so that steps can be captured into a CUDA graph:
+      obs f32[M, 2, 6]: on a step that sets NEED, the (left, right) seat rows of every external seat hold utils.inference's vector
+        (the left seat's x-mirrored); other rows are unspecified
+      flags u8[M]: SESSION_NEED | SESSION_DONE | SESSION_EMULATOR_ERROR; `need` and `done` are bool views of the first two bits
+        computed on demand
+      scores i32[M, 2] (left, right points of the last decided frame), rewards f64[M] and frames i32[M] (written when a match ends)
+    The session keeps a reference to every tensor passed to Engine.session: they must not change while it is open."""
+
+    def __init__(self, engine: Engine, handle: ctypes.c_void_p, out: dict, obs: torch.Tensor, flags: torch.Tensor,
+                 raw: torch.Tensor | None, left: torch.Tensor, keep: tuple):
+        self.engine = engine
+        self._s = handle
+        self.obs, self.flags = obs, flags
+        self.scores, self.rewards, self.frames = out["scores"], out["rewards"], out["frames"]
+        self.n = obs.shape[0]
+        self._raw, self._left, self._keep = raw, left, keep
+        self._capture = None
+
+    @property
+    def need(self) -> torch.Tensor:
+        return (self.flags & _lib.SESSION_NEED) != 0
+
+    @property
+    def done(self) -> torch.Tensor:
+        return (self.flags & _lib.SESSION_DONE) != 0
+
+    def _live(self):
+        if not self._s:
+            raise _lib.NgpError("the match session is closed")
+        return self._s
+
+    def step(self, actions: torch.Tensor, capture: bool = False) -> torch.Tensor | None:
+        """One env.step of every running match.  actions: u8[M, 2] (left, right) NGP_ACT_* of the external seats, consumed on
+        the matches whose NEED is set (other entries are ignored).  Does not synchronise.  With capture, returns the state of
+        every match still running after this step's decisions, u8[M, NGP_GAME_STATE_BYTES] (one buffer, rewritten by the next
+        capturing step)."""
+        self.engine._check_tensor(actions, torch.uint8, "actions")
+        assert tuple(actions.shape) == (self.n, 2)
+        cap = None
+        if capture:
+            if self._capture is None:
+                self._capture = torch.zeros((self.n, _lib.NGP_GAME_STATE_BYTES), dtype=torch.uint8, device=self.engine.device)
+            cap = self._capture
+        _lib.check(self.engine._L.ngp_session_step(self._live(), _p(actions), _p(self.obs), _p(self.flags), _p(cap),
+                                                   _stream(self.engine.device)), "ngp_session_step")
+        return cap
+
+    def _status(self):
+        running, total = ctypes.c_int32(0), ctypes.c_uint64(0)
+        rc = self.engine._L.ngp_session_status(self._live(), ctypes.byref(running), ctypes.byref(total), _stream(self.engine.device))
+        return rc, int(running.value), int(total.value)
+
+    def running(self) -> int:
+        """The matches still running (synchronises)."""
+        return self._status()[1]
+
+    def result(self) -> dict:
+        """Synchronises; play_matches_states' dict (rewards, frames, scores, frames_total, left, and record views when the
+        session records).  Raises NgpError on an emulator error, on consumed actions outside 0..2, or while a match runs."""
+        rc, running, total = self._status()
+        _lib.check(rc, "ngp_session_status")
+        if running:
+            raise _lib.NgpError(f"the match session has {running} matches still running")
+        out = {"rewards": self.rewards, "frames": self.frames, "scores": self.scores, "frames_total": total, "left": self._left}
+        if self._raw is not None:
+            out["record"] = record_views(self._raw)
+        return out
+
+    def close(self):
+        if getattr(self, "_s", None):
+            self.engine._L.ngp_session_end(self._s)
+            self._s = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()

@@ -11,6 +11,8 @@ Names and argument meaning follow the reference so its call sites read the same:
   replay(individual) / repeat_upsample                         pickle_inspector.py:1-12, main.py:115-125, utils.py:156-168
   cross_play(toolbox, a, b)                                    no counterpart: main.evaluate's schedule as any match list
   render_recorded / replay_selfplay                            main.evaluate(render=True) for recorded games
+  play_policy / model_policy                                   perform_episode with any model object (main.py:69-112,
+                                                               play_against_human.py): outside policies in a match list
 Every call lands in libngp.so's CUDA kernels through Engine; nothing here computes on the CPU except argument
 marshalling (individuals are rows of device tensors instead of Python lists)."""
 from __future__ import annotations
@@ -457,6 +459,54 @@ def branch(toolbox: Toolbox, genomes: torch.Tensor, right, left, m: int, t: int,
     out["capture"] = orig["capture"]
     out["start_states"] = (orig["capture"], int(t))
     return out
+
+
+def model_policy(model):
+    """A policy for play_policy from a reference-style model object -- anything with .run(vec6) -> [up, down], as
+    perform_episode takes it (main.py:69-112): numpy_nn.NeuralNetwork, a dumb_ais bot, a keyboard reader.  Each observation row
+    is passed to model.run as a list of six floats; [1, 0] is NGP_ACT_UP, [0, 1] NGP_ACT_DOWN, anything else NGP_ACT_NONE
+    (both buttons held cancel, FILTERED, main.py:23,55)."""
+    def policy(obs: torch.Tensor) -> torch.Tensor:
+        acts = []
+        for vec in obs.detach().cpu().double().numpy():
+            up, down = (bool(v) for v in model.run([float(v) for v in vec])[:2])
+            acts.append(_lib.ACT_UP if up and not down else _lib.ACT_DOWN if down and not up else _lib.ACT_NONE)
+        return torch.tensor(acts, dtype=torch.uint8, device=obs.device)
+    return policy
+
+
+def play_policy(toolbox: Toolbox, genomes: torch.Tensor | None, right, left, policy, mult=None, key=None, states=None, start=None,
+                fresh: bool = False, max_record: int | None = None, check_every: int = 8):
+    """Plays a match list in which every seat named PLAYER_EXTERNAL is driven by `policy` (play_against_human.py /
+    main.run_against_human with any controller): policy(obs f32[K, 6]) -> K NGP_ACT_* decisions (a tensor or a sequence), called
+    once per step on the external seats whose match needs a decision (Engine.session's NEED; utils.inference's vector, the left
+    seat's x-mirrored), not called on a step without one.  right / left: lists as Engine.session takes them (sequences or int32
+    tensors); genomes may be None when no seat names a row.  Runs on the toolbox's seed and generation and records every frame
+    (max_record None = the longest possible game of the config), so that render_recorded re-renders any game of the result.
+    check_every: steps between two reads of the running count (each read synchronises).  Returns MatchSession.result()."""
+    eng, cfg = toolbox.engine, toolbox.config
+    dev = eng.device
+
+    def dev_i32(v):
+        return (v if torch.is_tensor(v) else torch.tensor(list(v), dtype=torch.int32)).to(dev, torch.int32).contiguous()
+
+    r, l = dev_i32(right), dev_i32(left)
+    bound = max_record or (cfg.MAX_FRAMES if cfg.MAX_FRAMES > 0 else 2 * cfg.WIN_SCORE * (cfg.TIMEOUT_THRESH + 2))
+    if genomes is not None:
+        genomes = genomes.to(dev, torch.float32).contiguous()
+    with eng.session(genomes, r, l, mult=mult, key=key, states=states, start=start, fresh=fresh, max_record=bound, seed=toolbox.seed,
+                     generation=toolbox.generation) as s:
+        external = torch.stack([l == _lib.PLAYER_EXTERNAL, r == _lib.PLAYER_EXTERNAL], dim=1)          # [M, 2] (left, right)
+        actions = torch.zeros((r.shape[0], 2), dtype=torch.uint8, device=dev)
+        step = 0
+        while step % check_every or s.running():
+            rows = external & s.need[:, None]
+            if bool(rows.any()):
+                act = policy(s.obs[rows])
+                actions[rows] = torch.as_tensor(act, device=dev).to(torch.uint8)
+            s.step(actions)
+            step += 1
+        return s.result()
 
 
 def replay_selfplay(toolbox: Toolbox, genomes: torch.Tensor, g: int, k: int, upsample=(4, 4)):
